@@ -5,6 +5,7 @@ BASELINE.json workload, one JSON line on stdout.
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C2] [--scale 1.0] [--catalogue full]
     python bench.py --impl reference ...      # CPU arm: the UNMODIFIED reference scripts on the host cores
     torchrun ... bench.py --gpus N [--scaling strong]
+    python bench.py --dump-outputs DIR ...    # also write what the last timed step computed as DIR/<name>.npy
 
 A "step" is one pass of the hot path over one batch of synthetic GAF (one file of the named config per
 GPU): counters reset -> filter chain (probe, scan, exact kernels) -> counters of all ranks summed (inside
@@ -40,12 +41,21 @@ METRIC = "gaf_alignments_filtered_assigned_per_sec"
 UNIT = "alignments/s"
 REF_DIR = os.path.join(ROOT, "baseline", "_ref")          # the three unmodified scripts, copied by __graft_entry__.build()
 REF_SCRIPTS = ("filter-alignments.py", "predict-genotype.py")
+DUMP_BYTES = 60_000_000   # --dump-outputs: the arrays of all files together; with the .npy headers below 64 MB
+DUMP_SEED = 20240601      # rows kept where an output is larger than its share
+
+
+def at_least_one(text):
+    n = int(text)
+    if n < 1:
+        raise argparse.ArgumentTypeError(f"must be at least 1, got {n}")
+    return n
 
 
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=at_least_one, default=100, help="timed steps of the hot path")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="C2", choices=["C2", "C3", "C4", "C5"])
@@ -62,7 +72,30 @@ def parse_args():
     ap.add_argument("--tile-lines", type=int, default=0, help="developer: lines a tile of the scan kernel should hold")
     ap.add_argument("--collective", default="p2p", choices=["p2p", "nccl"],
                     help="N > 1: counters summed inside the genotype kernel over NVLink peer memory (p2p), or ncclAllReduce")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="one GPU: write the counters, hit tuples and genotype arrays of the last timed step to DIR/<name>.npy "
+                         "(float64, at most 64 MB in all: a larger array is cut to the same seeded sample of rows every run)")
     return ap.parse_args()
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array of ``arrays`` (name -> numpy array, rows first) as ``out_dir/<name>.npy`` in float64, which
+    holds every integer the path computes exactly.  Each array gets an equal share of DUMP_BYTES; one with more rows
+    than fit keeps a sorted sample drawn with DUMP_SEED, so arrays of equal length keep the same rows and two builds
+    that compute the same thing write the same files.  Returns name -> (rows written, rows computed)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // max(1, len(arrays))
+    kept = {}
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        n_max = share // (8 * max(1, int(np.prod(a.shape[1:]))))
+        if len(a) > n_max:
+            rows = np.random.default_rng(DUMP_SEED).choice(len(a), size=n_max, replace=False)
+            a = a[np.sort(rows)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+        kept[name] = (len(a), len(arrays[name]))
+    return kept
 
 
 def workload(args, stream):
@@ -420,6 +453,8 @@ def main():
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a GPU (there is no CPU fallback); use --impl reference for the CPU arm")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the outputs of one GPU: run it without torchrun")
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     if world > 1:
@@ -627,6 +662,22 @@ def main():
     st = filt.read_stats()
     if xchg and xchg.timed_out():
         raise SystemExit(f"rank {rank}: a wait in the fused counter exchange timed out")
+    dumped = None
+    if args.dump_outputs:
+        # the last timed step's results, read before the measurements below launch on the same buffers
+        nh = st["n_hits"]
+        if st["status"] or nh > filt.hit_cap:
+            raise SystemExit(f"--dump-outputs: the last timed step did not complete: {st}")
+        sv2 = filt.hit_sv2[:nh].cpu().numpy().view(np.uint32)
+        off = filt.hit_off[:nh].cpu().numpy().view(np.uint32)
+        ln = filt.hit_len[:nh].cpu().numpy().view(np.uint32)
+        order = np.lexsort((ln, sv2, off))               # the kernels append hits in any order: sorted into file order
+        dumped = dump_outputs(args.dump_outputs, {
+            "counts": filt.counts[:tables.num_sv].cpu().numpy().view(np.uint32),
+            "hit_sv2": sv2[order], "hit_off": off[order], "hit_len": ln[order],
+            "genotype_gt": d_gt[:n_loc].cpu().numpy(), "genotype_flags": d_fl[:n_loc].cpu().numpy(),
+            "genotype_ad2": d_ad[:n_loc].cpu().numpy().view(np.uint32), "genotype_pl": d_pl[:n_loc].cpu().numpy(),
+        })
 
     # the dominant kernel on its own: the library records CUDA events around its scan kernel on this stream
     def timed_scan(n_iter):
@@ -781,6 +832,8 @@ def main():
         "gpu_launches": 5 * K,   # reset + probe + scan + exact + genotype
         "clocks": clocks,
     }
+    if dumped is not None:
+        line["dumped_outputs"] = {name: {"rows": n, "of": total} for name, (n, total) in dumped.items()}
     print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
