@@ -10,7 +10,8 @@
 //   probe       one block: line length at the head of the shard -> bytes per tile, so that a tile
 //               holds about one line per lane of the warp that parses it; zeroes the list cursors.
 //   scan        every WARP is an independent worker with its own shared-memory window
-//               (no block barrier).  It walks tiles of the byte buffer; a tile plus 1 KiB of
+//               (no block barrier).  It takes tiles of the byte buffer from a queue (one atomic
+//               cursor: a warp that drew node-dense tiles takes fewer); a tile plus 1 KiB of
 //               look-ahead is staged by one TMA bulk copy (the warp's next tile is prefetched into L2).
 //               A  byte-parallel: every lane classifies 32 bytes with SWAR compares into four
 //                  classes (newline, tab, '<'/'>', non-digit); the newlines go straight into the
@@ -36,6 +37,8 @@
 //               window gets the fast rules applied where it lies (giant_line()).
 // The GAF bytes are read from DRAM once (scan); only the exact route reads them again.
 // A line belongs to the tile its first byte is in.
+// scan and exact are launched with programmatic stream serialization (launch_pdl): each is scheduled while
+// the kernel in front of it finishes, sets up what needs no data of it, then waits for it.
 #include <cooperative_groups.h>
 #include <cuda_runtime.h>
 
@@ -92,7 +95,7 @@ constexpr uint32_t COMMA_PATH = 0xFFFFFFFFu;
 
 // device scratch of one svjg_filter_device() call
 struct Scratch {
-    uint32_t *cnt;        // [2] exact-route lines, [4] bytes per tile, [5] pool cursor
+    uint32_t *cnt;        // [2] exact-route lines, [4] bytes per tile, [5] pool cursor, [6] tile queue
     uint32_t *exact;      // line start offsets
     uint4 *slab;          // per warp of the scan kernel: nodes of a long line (long_line())
     uint4 *pool;          // exact kernel: bitmaps and nodes of giant lines, bump-allocated (cnt[5])
@@ -1105,6 +1108,7 @@ template <class G>
 __global__ void __launch_bounds__(THREADS, G::MB) scan_kernel(const __grid_constant__ FilterArgs a) {
     extern __shared__ __align__(128) uint8_t smem_all[];
     __shared__ __align__(8) uint64_t mbars[WARPS];
+    __shared__ uint32_t next_tile[WARPS];                                  // the tile each warp takes next
 
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const uint32_t lt_mask = (1u << lane) - 1u;
@@ -1127,11 +1131,15 @@ __global__ void __launch_bounds__(THREADS, G::MB) scan_kernel(const __grid_const
     const uint32_t one = a.one;
     const uint32_t n_workers = gridDim.x * WARPS;
 
+    cudaGridDependencySynchronize();                               // probe_kernel: the tile size, zeroed cursors
+    cudaTriggerProgrammaticLaunchCompletion();                     // exact_kernel may be scheduled as blocks retire
     const uint32_t tile_bytes = a.sc.cnt[4];                       // chosen by probe_kernel: a multiple of 32, at most G::TILE_MAX
     const uint32_t n_tiles = uint32_t((a.n + tile_bytes - 1) / tile_bytes);
     const uint32_t win_bytes = HEAD + tile_bytes + LOOKAHEAD, n_pairs = win_bytes / 32u;
 
-    for (uint32_t tile = blockIdx.x * WARPS + warp; tile < n_tiles; tile += n_workers) {
+    // The first tile of every warp is fixed, the rest come from the queue cnt[6] (tiles n_workers, n_workers + 1, ...):
+    // a warp that drew slow tiles takes fewer, and the SMs run out of work together.
+    for (uint32_t tile = blockIdx.x * WARPS + warp; tile < n_tiles; tile = next_tile[warp], __syncwarp()) {
         const uint64_t tile_start = uint64_t(tile) * tile_bytes;
         const uint64_t g0 = tile_start ? tile_start - HEAD : 0;
         const uint32_t dst0 = tile_start ? 0 : HEAD;
@@ -1143,12 +1151,16 @@ __global__ void __launch_bounds__(THREADS, G::MB) scan_kernel(const __grid_const
         const uint32_t valid_end = dst0 + nbytes;
         const uint32_t wbase = uint32_t(tile_start) - HEAD;            // shard offset = wbase + window offset
 
-        if (lane == 0 && bulk) {
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            mbar_expect_tx(mbar, bulk);
-            bulk_g2s(win + dst0, a.gaf + g0, bulk, mbar);
-            // the tile this warp takes next: on its way into L2 while this one is parsed
-            const uint64_t nx = tile_start + uint64_t(n_workers) * tile_bytes;
+        if (lane == 0) {
+            if (bulk) {
+                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                mbar_expect_tx(mbar, bulk);
+                bulk_g2s(win + dst0, a.gaf + g0, bulk, mbar);
+            }
+            // the tile this warp takes next, drawn while the copy is in flight: on its way into L2 while this one is parsed
+            const uint32_t next = n_workers + atomicAdd(a.sc.cnt + 6, 1u);
+            next_tile[warp] = next;                                // read behind the tile's last __syncwarp()
+            const uint64_t nx = uint64_t(next) * tile_bytes;
             if (nx + tile_bytes + LOOKAHEAD <= a.n) l2_prefetch(a.gaf + nx - HEAD, win_bytes);
         }
         if (bulk != nbytes || dst0 || valid_end < win_bytes) {                       // the first and the last tiles of the shard
@@ -1479,7 +1491,10 @@ __device__ __noinline__ bool giant_line(const FilterArgs &a, uint32_t ps, uint32
 }
 
 __global__ void __launch_bounds__(FLAT_THREADS) exact_kernel(const __grid_constant__ FilterArgs a) {
+    cudaGridDependencySynchronize();                               // scan_kernel: the list and its length
+    cudaTriggerProgrammaticLaunchCompletion();
     const uint32_t n = min(a.sc.cnt[2], a.sc.cap_exact);
+    if (n == 0) return;                                            // the rule on regular input: nothing to set up
     Local loc;
     // Lines differ wildly in the work they need (general() is quadratic in the path nodes), and lanes
     // of a warp that run different lines execute one after the other.  While there are few lines,
@@ -1516,11 +1531,13 @@ __global__ void __launch_bounds__(FLAT_THREADS) exact_kernel(const __grid_consta
 
 // ===========================================================================
 // probe: average line length of the head of the shard -> bytes per tile, so that a tile holds about
-// one line per lane of the warp that parses it
+// one line per lane of the warp that parses it.  Launched plainly (it zeroes scratch the kernels in front of it
+// may have used); the scan kernel is scheduled while it runs and waits for its result.
 // ===========================================================================
 constexpr int PROBE_THREADS = 1024, PROBE_BYTES = 64 << 10;
 
 __global__ void __launch_bounds__(PROBE_THREADS) probe_kernel(const __grid_constant__ FilterArgs a) {
+    cudaTriggerProgrammaticLaunchCompletion();
     __shared__ uint32_t total;
     if (threadIdx.x == 0) total = 0;
     if (threadIdx.x < 16 && threadIdx.x != 4) a.sc.cnt[threadIdx.x] = 0;      // the lists' cursors
@@ -1563,6 +1580,25 @@ __global__ void reset_kernel(uint32_t *counts, uint64_t n, unsigned long long *s
     uint64_t stride = uint64_t(gridDim.x) * blockDim.x;
     for (uint64_t k = i; k < n; k += stride) counts[k] = 0;
     if (i < 8) stats[i] = (i == 5) ? ~0ull : 0ull;
+}
+
+// Launch with programmatic stream serialization: when the work in front of it on the stream is a kernel, this one
+// may be scheduled while that kernel still runs (from the point where every block of it has called
+// cudaTriggerProgrammaticLaunchCompletion() or exited).  Every thread of a kernel launched so calls
+// cudaGridDependencySynchronize() before it reads or writes memory the kernels in front of it use.
+template <typename... P, typename... A>
+cudaError_t launch_pdl(void (*kernel)(P...), unsigned grid, unsigned block, size_t smem, cudaStream_t st, A &&...args) {
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(grid);
+    cfg.blockDim = dim3(block);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = st;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    return cudaLaunchKernelEx(&cfg, kernel, static_cast<A &&>(args)...);
 }
 
 // ---- launch configuration, fixed per device the first time a shard is filtered there
@@ -1743,14 +1779,16 @@ int svjg::filter_device_abs(const svjg_tables *t, const uint8_t *d_gaf, uint64_t
 
     const uint32_t max_tiles = uint32_t((n_bytes + TILE_MIN - 1) / TILE_MIN);
     const int scan_grid = int(std::min<uint32_t>((max_tiles + WARPS - 1) / WARPS, uint32_t(cfg->grid_cap)));
+    // with profiling on, the events between the kernels keep them apart: the scan kernel's time is its own
     probe_kernel<<<1, PROBE_THREADS, 0, st>>>(a);
-    if (g_profile) cudaEventRecord(cfg->ev0, st);
-    if (cfg->min_blocks == 8) scan_kernel<Geo8><<<scan_grid, THREADS, cfg->smem, st>>>(a);
-    else scan_kernel<Geo6><<<scan_grid, THREADS, cfg->smem, st>>>(a);
-    if (g_profile) cudaEventRecord(cfg->ev1, st), cfg->timed = true;
-    if (!(a.flags & FLAG_STOP_AFTER_SCAN))
-        exact_kernel<<<cfg->sms * 2, FLAT_THREADS, 0, st>>>(a);     // a few lines as a rule: a small grid starts faster
     cudaError_t le = cudaGetLastError();
+    if (g_profile) cudaEventRecord(cfg->ev0, st);
+    if (le == cudaSuccess)
+        le = launch_pdl(cfg->min_blocks == 8 ? scan_kernel<Geo8> : scan_kernel<Geo6>, scan_grid, THREADS, cfg->smem, st, a);
+    if (g_profile) cudaEventRecord(cfg->ev1, st), cfg->timed = true;
+    if (le == cudaSuccess && !(a.flags & FLAG_STOP_AFTER_SCAN))
+        le = launch_pdl(exact_kernel, cfg->sms * 2, FLAT_THREADS, 0, st, a);     // a few lines as a rule: a small grid starts faster
+    if (le == cudaSuccess) le = cudaGetLastError();
     cudaError_t fe = cudaFreeAsync(ws, st);
     SVJG_CUDA(le);
     SVJG_CUDA(fe);
