@@ -233,6 +233,32 @@ int svjg_genotype_host(const uint32_t *counts, uint32_t num_counts, const uint32
                        const double *lut, uint32_t lut_nmax, const double *k_override, int64_t *pl, uint8_t *gt,
                        uint32_t *ad2, uint8_t *flags);
 
+/* ---- cohorts: one catalogue genotyped in many samples -------------------------
+ * The reference genotypes one sample per run; a cohort of S samples keeps the counters of every sample on the
+ * device at once, so the tables are loaded and the context created once.  The counter matrix is [S][num_sv][2]
+ * u32 (sample-major: each sample's slice is the counter array of svjg_filter_host).
+ *   svjg_cohort_create      a zeroed counter matrix on the device of `t` (t must stay alive and on its device)
+ *   svjg_cohort_filter      svjg_filter_host into sample `sample`'s counters, from host bytes: ACCUMULATED (several
+ *                           files of one sample are counted together, as the reference counts the GAFs it appends
+ *                           into one file); no hit list.  Synchronous.  SVJG_E_INPUT with stats->status and
+ *                           stats->err_offset (offset within `gaf`) where the reference would raise
+ *   svjg_cohort_read_counts / svjg_cohort_load_counts   host copy [num_sv][2] of one sample's counters, out / in
+ *   svjg_cohort_genotype    svjg_genotype_host for n records in every sample (no k_override: cells whose rounded
+ *                           counts exceed lut_nmax get SVJG_GT_NEED_K; the caller recomputes those cells from their
+ *                           counters, e.g. with svjg_genotype_host).  Outputs are host arrays [n][S]: pl [n][S][3],
+ *                           gt, flags [n][S], ad2 [n][S][2].  The LUT and the block buffers are cached in the handle.
+ *                           Synchronous. */
+typedef struct svjg_cohort svjg_cohort;
+int svjg_cohort_create(svjg_tables *t, uint32_t n_samples, svjg_cohort **out);
+void svjg_cohort_free(svjg_cohort *c);
+int svjg_cohort_filter(svjg_cohort *c, uint32_t sample, const uint8_t *gaf, uint64_t n_bytes, int64_t d_over,
+                       svjg_filter_stats *stats);
+int svjg_cohort_read_counts(svjg_cohort *c, uint32_t sample, uint32_t *counts);
+int svjg_cohort_load_counts(svjg_cohort *c, uint32_t sample, const uint32_t *counts);
+int svjg_cohort_genotype(svjg_cohort *c, const uint32_t *sv_index, const uint8_t *svtype, uint32_t n, int64_t min_support,
+                         double log10_1me, double log10_e, double log10_half, const double *lut, uint32_t lut_nmax,
+                         int64_t *pl, uint8_t *gt, uint32_t *ad2, uint8_t *flags);
+
 /* Page-locked host memory (cudaHostAlloc) for file buffers and results: copies to and from it run
  * at PCIe speed.  For callers that do not want a tensor library just to pin memory. */
 int svjg_host_alloc(uint64_t bytes, void **out);
@@ -324,6 +350,15 @@ int svjg_vcf_index_tables(const svjg_vcf *v, const svjg_tables *t, uint32_t *sv_
 int svjg_vcf_index_counts(const svjg_vcf *v, const svjg_aln_counts *c, uint32_t *sv_index, uint8_t *svtype);
 int svjg_vcf_format(const svjg_vcf *v, const uint8_t *gt, const uint8_t *flags, const uint32_t *ad2,
                     const int64_t *pl, char **out, uint64_t *out_len, uint64_t *n_genotyped);
+/* svjg_vcf_format_cohort: the text of records [lo, hi) of a multi-sample VCF (svjg_cohort_genotype's arrays of those
+ * records, [hi - lo][n_samples]); the pieces of consecutive ranges joined are the whole file.  Every line is the
+ * single-sample line with one column per sample, and the column header names the samples: `names` is the names
+ * joined by '\t' (names_len bytes).  A range holds the header lines in front of its records and, when hi is the
+ * number of records, the ones behind the last.  n_genotyped[s] is ADDED to.  svjg_vcf_format is this with one
+ * sample named "SAMPLE". */
+int svjg_vcf_format_cohort(const svjg_vcf *v, uint32_t lo, uint32_t hi, uint32_t n_samples, const char *names,
+                           uint64_t names_len, const uint8_t *gt, const uint8_t *flags, const uint32_t *ad2,
+                           const int64_t *pl, char **out, uint64_t *out_len, uint64_t *n_genotyped);
 void svjg_buffer_free(char *p);
 
 /* ---- output (host) ------------------------------------------------------------

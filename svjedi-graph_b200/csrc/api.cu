@@ -186,144 +186,6 @@ extern "C" void svjg_tables_free(svjg_tables *t) {
 // ---------------------------------------------------------------------------
 // host-buffer filter
 // ---------------------------------------------------------------------------
-extern "C" int svjg_filter_host(svjg_tables *t, const uint8_t *gaf, uint64_t n_bytes, int64_t d_over, uint32_t *counts,
-                                uint32_t *hit_sv2, uint64_t *hit_off, uint32_t *hit_len, uint64_t hit_cap,
-                                svjg_filter_stats *stats) {
-    if (!t || t->device < 0) return set_error(SVJG_E_ARG, "svjg_filter_host: tables are not on a device");
-    if (!counts || !stats || (n_bytes && !gaf)) return set_error(SVJG_E_ARG, "svjg_filter_host: NULL argument");
-    if (hit_cap && (!hit_sv2 || !hit_off || !hit_len)) return set_error(SVJG_E_ARG, "svjg_filter_host: NULL hit buffer");
-    SVJG_CUDA(cudaSetDevice(t->device));
-    const uint32_t num_sv = uint32_t(t->sv_ids.size());
-
-    // chunk plan: cut at line ends, each chunk < 4 GiB
-    std::vector<uint64_t> cut{0};
-    while (cut.back() < n_bytes) {
-        uint64_t b = cut.back(), e = std::min(n_bytes, b + HostWs::CHUNK);
-        if (e < n_bytes) {
-            const void *nl = memrchr(gaf + b, '\n', size_t(e - b));
-            if (nl) {
-                e = uint64_t(static_cast<const uint8_t *>(nl) - gaf) + 1;
-            } else {
-                const void *fw = memchr(gaf + e, '\n', size_t(n_bytes - e));
-                e = fw ? uint64_t(static_cast<const uint8_t *>(fw) - gaf) + 1 : n_bytes;
-            }
-        }
-        if (e - b >= 0xFFFF0000ull) return set_error(SVJG_E_ARG, "a single GAF line exceeds 4 GiB");
-        cut.push_back(e);
-    }
-    const size_t n_chunks = cut.size() - 1;
-    uint64_t max_chunk = 0;
-    for (size_t k = 0; k < n_chunks; ++k) max_chunk = std::max(max_chunk, cut[k + 1] - cut[k]);
-
-    if (!t->ws) {
-        t->ws = new HostWs();
-        HostWs *w = t->ws;
-        SVJG_CUDA(cudaStreamCreateWithFlags(&w->s_copy, cudaStreamNonBlocking));
-        SVJG_CUDA(cudaStreamCreateWithFlags(&w->s_comp, cudaStreamNonBlocking));
-        for (int i = 0; i < 2; ++i) {
-            SVJG_CUDA(cudaEventCreateWithFlags(&w->copied[i], cudaEventDisableTiming));
-            SVJG_CUDA(cudaEventCreateWithFlags(&w->freed[i], cudaEventDisableTiming));
-        }
-        SVJG_CUDA(cudaMalloc(&w->d_counts, std::max<size_t>(16, size_t(num_sv) * 8)));
-        SVJG_CUDA(cudaMalloc(&w->d_stats, sizeof(svjg_filter_stats)));
-    }
-    HostWs *w = t->ws;
-    if (w->buf_cap < max_chunk) {
-        for (int i = 0; i < 2; ++i) {
-            if (w->d_buf[i]) SVJG_CUDA(cudaFree(w->d_buf[i]));
-            w->d_buf[i] = nullptr;
-        }
-        w->buf_cap = 0;
-        uint64_t cap = (max_chunk + 255) & ~255ull;
-        for (int i = 0; i < (n_chunks > 1 ? 2 : 1); ++i) SVJG_CUDA(cudaMalloc(&w->d_buf[i], cap));
-        w->buf_cap = cap;
-    } else if (n_chunks > 1 && !w->d_buf[1]) {
-        SVJG_CUDA(cudaMalloc(&w->d_buf[1], w->buf_cap));
-    }
-    if (w->hit_cap < hit_cap) {
-        for (int i = 0; i < 3; ++i) {
-            if (w->d_hit[i]) SVJG_CUDA(cudaFree(w->d_hit[i]));
-            w->d_hit[i] = nullptr;
-        }
-        w->hit_cap = 0;
-        for (int i = 0; i < 3; ++i) SVJG_CUDA(cudaMalloc(&w->d_hit[i], hit_cap * 4));
-        if (w->d_off64) SVJG_CUDA(cudaFree(w->d_off64));
-        w->d_off64 = nullptr;
-        SVJG_CUDA(cudaMalloc(&w->d_off64, hit_cap * 8));
-        w->hit_cap = hit_cap;
-    }
-    // Result arrays in page-locked host memory are written by the kernels themselves (the device can
-    // address them): the hits cross PCIe while later chunks are still coming in, and no copy is left
-    // for the end.  Pageable arrays get the hits by a copy from device buffers.
-    auto device_view = [](void *p) -> void * {
-        cudaPointerAttributes at;
-        if (!p || cudaPointerGetAttributes(&at, p) != cudaSuccess) {
-            cudaGetLastError();
-            return nullptr;
-        }
-        return at.type == cudaMemoryTypeHost ? at.devicePointer : nullptr;
-    };
-    uint32_t *k_sv2 = w->d_hit[0], *k_len = w->d_hit[2];
-    uint64_t *k_off = w->d_off64;
-    bool direct = false;
-    // Up to 64 MB of hit tuples; beyond that the copy engines take them at the end.  (Measured: 0.5 GB
-    // of tuples per GPU written by the kernels is fine on one GPU -- 5 ms, hidden behind the upload --
-    // but took 1.3 s when eight GPUs of a node did it at once.)
-    if (hit_cap && hit_cap * 16 <= (64ull << 20)) {
-        void *v0 = device_view(hit_sv2), *v1 = device_view(hit_off), *v2 = device_view(hit_len);
-        if (v0 && v1 && v2) {
-            k_sv2 = static_cast<uint32_t *>(v0);
-            k_off = static_cast<uint64_t *>(v1);
-            k_len = static_cast<uint32_t *>(v2);
-            direct = true;
-        }
-    }
-
-    int rc = svjg_filter_reset(w->d_counts, num_sv, w->d_stats, w->s_comp);
-    if (rc) return rc;
-    for (size_t k = 0; k < n_chunks; ++k) {
-        int b = int(k & 1);
-        uint64_t len = cut[k + 1] - cut[k];
-        if (k >= 2) SVJG_CUDA(cudaStreamWaitEvent(w->s_copy, w->freed[b], 0));
-        SVJG_CUDA(cudaMemcpyAsync(w->d_buf[b], gaf + cut[k], len, cudaMemcpyHostToDevice, w->s_copy));
-        SVJG_CUDA(cudaEventRecord(w->copied[b], w->s_copy));
-        SVJG_CUDA(cudaStreamWaitEvent(w->s_comp, w->copied[b], 0));
-        rc = filter_device_abs(t, w->d_buf[b], len, cut[k], d_over, w->d_counts, k_sv2, nullptr, k_off, k_len, hit_cap,
-                               w->d_stats, w->s_comp);
-        if (rc) {
-            // copies out of the caller's buffer and kernels may still be in flight: not behind the caller's back
-            cudaStreamSynchronize(w->s_copy);
-            cudaStreamSynchronize(w->s_comp);
-            return rc;
-        }
-        SVJG_CUDA(cudaEventRecord(w->freed[b], w->s_comp));
-    }
-    SVJG_CUDA(cudaMemcpyAsync(stats, w->d_stats, sizeof(svjg_filter_stats), cudaMemcpyDeviceToHost, w->s_comp));
-    SVJG_CUDA(cudaMemcpyAsync(counts, w->d_counts, size_t(num_sv) * 8, cudaMemcpyDeviceToHost, w->s_comp));
-    SVJG_CUDA(cudaStreamSynchronize(w->s_comp));
-    if (n_bytes == 0) memset(stats, 0, sizeof *stats), stats->err_offset = ~0ull;
-    if (stats->status) {
-        char msg[160];
-        snprintf(msg, sizeof msg, "GAF line at byte %llu: the reference raises here (reason %llu)",
-                 (unsigned long long)stats->err_offset, (unsigned long long)stats->status);
-        return set_error(SVJG_E_INPUT, msg);
-    }
-    if (hit_cap == 0) return SVJG_OK;
-    if (stats->n_hits > hit_cap) return set_error(SVJG_E_HITS_OVERFLOW, "hit buffers too small");
-    const uint64_t nh = stats->n_hits;
-    if (nh && !direct) {
-        // pageable result arrays: staged by the driver
-        SVJG_CUDA(cudaMemcpyAsync(hit_sv2, w->d_hit[0], nh * 4, cudaMemcpyDeviceToHost, w->s_comp));
-        SVJG_CUDA(cudaMemcpyAsync(hit_off, w->d_off64, nh * 8, cudaMemcpyDeviceToHost, w->s_comp));
-        SVJG_CUDA(cudaMemcpyAsync(hit_len, w->d_hit[2], nh * 4, cudaMemcpyDeviceToHost, w->s_comp));
-        SVJG_CUDA(cudaStreamSynchronize(w->s_comp));
-    }
-    return SVJG_OK;
-}
-
-// ---------------------------------------------------------------------------
-// host-buffer filter with the informative_aln.json text rendered on the device
-// ---------------------------------------------------------------------------
 static int ensure_ws(svjg_tables *t, uint32_t num_sv) {
     if (t->ws) return SVJG_OK;
     t->ws = new HostWs();
@@ -354,6 +216,214 @@ static int ensure_hit_arrays(HostWs *w, uint64_t hit_cap) {
     return SVJG_OK;
 }
 
+// Host bytes through the filter chain into d_counts and w->d_stats (neither is reset here), on w->s_comp: chunks cut
+// at line ends, each copied on w->s_copy into one of two device buffers while the kernels work on the other.
+// Returns once every chunk is enqueued.
+static int filter_chunks(svjg_tables *t, const uint8_t *gaf, uint64_t n_bytes, int64_t d_over, uint32_t *d_counts,
+                         uint32_t *k_sv2, uint64_t *k_off, uint32_t *k_len, uint64_t hit_cap) {
+    HostWs *w = t->ws;
+    // chunk plan: cut at line ends, each chunk < 4 GiB
+    std::vector<uint64_t> cut{0};
+    while (cut.back() < n_bytes) {
+        uint64_t b = cut.back(), e = std::min(n_bytes, b + HostWs::CHUNK);
+        if (e < n_bytes) {
+            const void *nl = memrchr(gaf + b, '\n', size_t(e - b));
+            if (nl) {
+                e = uint64_t(static_cast<const uint8_t *>(nl) - gaf) + 1;
+            } else {
+                const void *fw = memchr(gaf + e, '\n', size_t(n_bytes - e));
+                e = fw ? uint64_t(static_cast<const uint8_t *>(fw) - gaf) + 1 : n_bytes;
+            }
+        }
+        if (e - b >= 0xFFFF0000ull) return set_error(SVJG_E_ARG, "a single GAF line exceeds 4 GiB");
+        cut.push_back(e);
+    }
+    const size_t n_chunks = cut.size() - 1;
+    uint64_t max_chunk = 0;
+    for (size_t k = 0; k < n_chunks; ++k) max_chunk = std::max(max_chunk, cut[k + 1] - cut[k]);
+
+    if (w->buf_cap < max_chunk) {
+        for (int i = 0; i < 2; ++i) {
+            if (w->d_buf[i]) SVJG_CUDA(cudaFree(w->d_buf[i]));
+            w->d_buf[i] = nullptr;
+        }
+        w->buf_cap = 0;
+        uint64_t cap = (max_chunk + 255) & ~255ull;
+        for (int i = 0; i < (n_chunks > 1 ? 2 : 1); ++i) SVJG_CUDA(cudaMalloc(&w->d_buf[i], cap));
+        w->buf_cap = cap;
+    } else if (n_chunks > 1 && !w->d_buf[1]) {
+        SVJG_CUDA(cudaMalloc(&w->d_buf[1], w->buf_cap));
+    }
+    for (size_t k = 0; k < n_chunks; ++k) {
+        int b = int(k & 1);
+        uint64_t len = cut[k + 1] - cut[k];
+        if (k >= 2) SVJG_CUDA(cudaStreamWaitEvent(w->s_copy, w->freed[b], 0));
+        SVJG_CUDA(cudaMemcpyAsync(w->d_buf[b], gaf + cut[k], len, cudaMemcpyHostToDevice, w->s_copy));
+        SVJG_CUDA(cudaEventRecord(w->copied[b], w->s_copy));
+        SVJG_CUDA(cudaStreamWaitEvent(w->s_comp, w->copied[b], 0));
+        int rc = filter_device_abs(t, w->d_buf[b], len, cut[k], d_over, d_counts, k_sv2, nullptr, k_off, k_len, hit_cap,
+                                   w->d_stats, w->s_comp);
+        if (rc) {
+            // copies out of the caller's buffer and kernels may still be in flight: not behind the caller's back
+            cudaStreamSynchronize(w->s_copy);
+            cudaStreamSynchronize(w->s_comp);
+            return rc;
+        }
+        SVJG_CUDA(cudaEventRecord(w->freed[b], w->s_comp));
+    }
+    return SVJG_OK;
+}
+
+// the stats of a finished filter call: SVJG_E_INPUT where the reference would raise
+static int input_status(svjg_filter_stats *stats, uint64_t n_bytes) {
+    if (n_bytes == 0) memset(stats, 0, sizeof *stats), stats->err_offset = ~0ull;
+    if (stats->status) {
+        char msg[160];
+        snprintf(msg, sizeof msg, "GAF line at byte %llu: the reference raises here (reason %llu)",
+                 (unsigned long long)stats->err_offset, (unsigned long long)stats->status);
+        return set_error(SVJG_E_INPUT, msg);
+    }
+    return SVJG_OK;
+}
+
+extern "C" int svjg_filter_host(svjg_tables *t, const uint8_t *gaf, uint64_t n_bytes, int64_t d_over, uint32_t *counts,
+                                uint32_t *hit_sv2, uint64_t *hit_off, uint32_t *hit_len, uint64_t hit_cap,
+                                svjg_filter_stats *stats) {
+    if (!t || t->device < 0) return set_error(SVJG_E_ARG, "svjg_filter_host: tables are not on a device");
+    if (!counts || !stats || (n_bytes && !gaf)) return set_error(SVJG_E_ARG, "svjg_filter_host: NULL argument");
+    if (hit_cap && (!hit_sv2 || !hit_off || !hit_len)) return set_error(SVJG_E_ARG, "svjg_filter_host: NULL hit buffer");
+    SVJG_CUDA(cudaSetDevice(t->device));
+    const uint32_t num_sv = uint32_t(t->sv_ids.size());
+
+    int rc = ensure_ws(t, num_sv);
+    if (rc) return rc;
+    HostWs *w = t->ws;
+    rc = ensure_hit_arrays(w, hit_cap);
+    if (rc) return rc;
+    // Result arrays in page-locked host memory are written by the kernels themselves (the device can
+    // address them): the hits cross PCIe while later chunks are still coming in, and no copy is left
+    // for the end.  Pageable arrays get the hits by a copy from device buffers.
+    auto device_view = [](void *p) -> void * {
+        cudaPointerAttributes at;
+        if (!p || cudaPointerGetAttributes(&at, p) != cudaSuccess) {
+            cudaGetLastError();
+            return nullptr;
+        }
+        return at.type == cudaMemoryTypeHost ? at.devicePointer : nullptr;
+    };
+    uint32_t *k_sv2 = w->d_hit[0], *k_len = w->d_hit[2];
+    uint64_t *k_off = w->d_off64;
+    bool direct = false;
+    // Up to 64 MB of hit tuples; beyond that the copy engines take them at the end.  (Measured: 0.5 GB
+    // of tuples per GPU written by the kernels is fine on one GPU -- 5 ms, hidden behind the upload --
+    // but took 1.3 s when eight GPUs of a node did it at once.)
+    if (hit_cap && hit_cap * 16 <= (64ull << 20)) {
+        void *v0 = device_view(hit_sv2), *v1 = device_view(hit_off), *v2 = device_view(hit_len);
+        if (v0 && v1 && v2) {
+            k_sv2 = static_cast<uint32_t *>(v0);
+            k_off = static_cast<uint64_t *>(v1);
+            k_len = static_cast<uint32_t *>(v2);
+            direct = true;
+        }
+    }
+
+    rc = svjg_filter_reset(w->d_counts, num_sv, w->d_stats, w->s_comp);
+    if (rc) return rc;
+    rc = filter_chunks(t, gaf, n_bytes, d_over, w->d_counts, k_sv2, k_off, k_len, hit_cap);
+    if (rc) return rc;
+    SVJG_CUDA(cudaMemcpyAsync(stats, w->d_stats, sizeof(svjg_filter_stats), cudaMemcpyDeviceToHost, w->s_comp));
+    SVJG_CUDA(cudaMemcpyAsync(counts, w->d_counts, size_t(num_sv) * 8, cudaMemcpyDeviceToHost, w->s_comp));
+    SVJG_CUDA(cudaStreamSynchronize(w->s_comp));
+    rc = input_status(stats, n_bytes);
+    if (rc) return rc;
+    if (hit_cap == 0) return SVJG_OK;
+    if (stats->n_hits > hit_cap) return set_error(SVJG_E_HITS_OVERFLOW, "hit buffers too small");
+    const uint64_t nh = stats->n_hits;
+    if (nh && !direct) {
+        // pageable result arrays: staged by the driver
+        SVJG_CUDA(cudaMemcpyAsync(hit_sv2, w->d_hit[0], nh * 4, cudaMemcpyDeviceToHost, w->s_comp));
+        SVJG_CUDA(cudaMemcpyAsync(hit_off, w->d_off64, nh * 8, cudaMemcpyDeviceToHost, w->s_comp));
+        SVJG_CUDA(cudaMemcpyAsync(hit_len, w->d_hit[2], nh * 4, cudaMemcpyDeviceToHost, w->s_comp));
+        SVJG_CUDA(cudaStreamSynchronize(w->s_comp));
+    }
+    return SVJG_OK;
+}
+
+// ---------------------------------------------------------------------------
+// cohort counters: one slice per sample, filled by the same chunk loop
+// ---------------------------------------------------------------------------
+extern "C" int svjg_cohort_create(svjg_tables *t, uint32_t n_samples, svjg_cohort **out) {
+    if (!t || t->device < 0) return set_error(SVJG_E_ARG, "svjg_cohort_create: tables are not on a device");
+    if (!out || n_samples == 0) return set_error(SVJG_E_ARG, "svjg_cohort_create: bad argument");
+    SVJG_CUDA(cudaSetDevice(t->device));
+    svjg_cohort *c = new svjg_cohort();
+    c->t = t;
+    c->n_samples = n_samples;
+    c->num_sv = uint32_t(t->sv_ids.size());
+    const size_t bytes = std::max<size_t>(16, size_t(n_samples) * c->num_sv * 8);
+    cudaError_t e = cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking);
+    if (e == cudaSuccess) e = cudaMalloc(&c->d_counts, bytes);
+    if (e == cudaSuccess) e = cudaMemset(c->d_counts, 0, bytes);
+    if (e != cudaSuccess) {
+        svjg_cohort_free(c);
+        return cuda_fail(int(e), "svjg_cohort_create");
+    }
+    *out = c;
+    return SVJG_OK;
+}
+
+extern "C" void svjg_cohort_free(svjg_cohort *c) {
+    if (!c) return;
+    cudaSetDevice(c->t->device);
+    if (c->d_counts) cudaFree(c->d_counts);
+    if (c->d_lut) cudaFree(c->d_lut);
+    if (c->d_blk) cudaFree(c->d_blk);
+    if (c->stream) cudaStreamDestroy(c->stream);
+    delete c;
+}
+
+extern "C" int svjg_cohort_filter(svjg_cohort *c, uint32_t sample, const uint8_t *gaf, uint64_t n_bytes, int64_t d_over,
+                                  svjg_filter_stats *stats) {
+    if (!c || !stats || (n_bytes && !gaf)) return set_error(SVJG_E_ARG, "svjg_cohort_filter: NULL argument");
+    if (sample >= c->n_samples) return set_error(SVJG_E_ARG, "svjg_cohort_filter: sample out of range");
+    svjg_tables *t = c->t;
+    SVJG_CUDA(cudaSetDevice(t->device));
+    int rc = ensure_ws(t, c->num_sv);
+    if (rc) return rc;
+    HostWs *w = t->ws;
+    uint32_t *d_counts = c->d_counts + size_t(sample) * c->num_sv * 2;
+    rc = svjg_filter_reset(d_counts, 0, w->d_stats, w->s_comp);          // the stats only: the counters accumulate
+    if (rc) return rc;
+    rc = filter_chunks(t, gaf, n_bytes, d_over, d_counts, nullptr, nullptr, nullptr, 0);
+    if (rc) return rc;
+    SVJG_CUDA(cudaMemcpyAsync(stats, w->d_stats, sizeof(svjg_filter_stats), cudaMemcpyDeviceToHost, w->s_comp));
+    SVJG_CUDA(cudaStreamSynchronize(w->s_comp));
+    return input_status(stats, n_bytes);
+}
+
+extern "C" int svjg_cohort_read_counts(svjg_cohort *c, uint32_t sample, uint32_t *counts) {
+    if (!c || (!counts && c->num_sv)) return set_error(SVJG_E_ARG, "svjg_cohort_read_counts: NULL argument");
+    if (sample >= c->n_samples) return set_error(SVJG_E_ARG, "svjg_cohort_read_counts: sample out of range");
+    SVJG_CUDA(cudaSetDevice(c->t->device));
+    SVJG_CUDA(cudaMemcpyAsync(counts, c->d_counts + size_t(sample) * c->num_sv * 2, size_t(c->num_sv) * 8,
+                              cudaMemcpyDeviceToHost, c->stream));
+    SVJG_CUDA(cudaStreamSynchronize(c->stream));
+    return SVJG_OK;
+}
+
+extern "C" int svjg_cohort_load_counts(svjg_cohort *c, uint32_t sample, const uint32_t *counts) {
+    if (!c || (!counts && c->num_sv)) return set_error(SVJG_E_ARG, "svjg_cohort_load_counts: NULL argument");
+    if (sample >= c->n_samples) return set_error(SVJG_E_ARG, "svjg_cohort_load_counts: sample out of range");
+    SVJG_CUDA(cudaSetDevice(c->t->device));
+    SVJG_CUDA(cudaMemcpyAsync(c->d_counts + size_t(sample) * c->num_sv * 2, counts, size_t(c->num_sv) * 8,
+                              cudaMemcpyHostToDevice, c->stream));
+    SVJG_CUDA(cudaStreamSynchronize(c->stream));
+    return SVJG_OK;
+}
+
+// ---------------------------------------------------------------------------
+// host-buffer filter with the informative_aln.json text rendered on the device
+// ---------------------------------------------------------------------------
 extern "C" int svjg_filter_json_begin(svjg_tables *t, const uint8_t *gaf, uint64_t n_bytes, int64_t d_over, uint32_t *counts,
                                       svjg_filter_stats *stats) {
     return svjg_filter_json_begin_at(t, gaf, n_bytes, 0, d_over, counts, stats);

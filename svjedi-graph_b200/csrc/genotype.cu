@@ -95,6 +95,83 @@ __device__ int64_t pl_of(const F192 &x) {
     return neg ? int64_t(q) : -int64_t(q);
 }
 
+// The genotype of one SV of one sample from its two counters: the gate of predict-genotype.py:216,
+// allele_normalization, the likelihoods, the unique argmax, -ms, the rounded counts, log10 C(n, k) and PL.
+// Results go to gt[o], flags[o], ad2[2o..], pl[3o..]; k_override[o] is read when k_override is given.
+__device__ __forceinline__ void genotype_one(uint32_t n0, uint32_t n1, uint32_t idx, uint32_t ty, int64_t min_support,
+                                             double la, double lb, double lh, const double *lut, uint32_t lut_nmax,
+                                             const double *k_override, size_t o, int64_t *pl, uint8_t *gt,
+                                             uint32_t *ad2, uint8_t *flags) {
+    // predict-genotype.py:216 — a key is "in the dict" once it has at least one hit
+    bool gate = (ty & 0x3F) <= 3 && !(ty & 0x80) && ty != 255 && idx != 0xFFFFFFFFu && ((n0 | n1) != 0 || (ty & 0x40));
+    if (!gate) {
+        gt[o] = 3;
+        flags[o] = 0;
+        ad2[2 * o] = 0;
+        ad2[2 * o + 1] = 0;
+        pl[3 * o] = pl[3 * o + 1] = pl[3 * o + 2] = 0;
+        return;
+    }
+    ty &= 0x3F;
+    // allele_normalization (:327-338): counts in half units
+    uint64_t t1 = 2ull * n0, t2 = 2ull * n1;
+    uint32_t fl = SVJG_GT_GENOTYPED;
+    if (ty == 0 && n0 > 0) {
+        t1 = n0;
+        fl |= SVJG_GT_HALVED_0;
+    } else if (ty == 1 && n1 > 0) {
+        t2 = n1;
+        fl |= SVJG_GT_HALVED_1;
+    }
+    double c1 = double(t1) * 0.5, c2 = double(t2) * 0.5, cs = double(t1 + t2) * 0.5;   // exact
+    bool ok = true;
+    // :295-297 — each product is the double the reference computes
+    F192 l0 = f_add(f_from_double(__dmul_rn(c1, la), ok), f_from_double(__dmul_rn(c2, lb), ok));
+    F192 l1 = f_from_double(__dmul_rn(cs, lh), ok);
+    F192 l2 = f_add(f_from_double(__dmul_rn(c2, la), ok), f_from_double(__dmul_rn(c1, lb), ok));
+    // unique argmax (:301-307)
+    int c01 = f_cmp(l0, l1), c02 = f_cmp(l0, l2), c12 = f_cmp(l1, l2);
+    uint32_t g = 3;
+    if (c01 > 0 && c02 > 0) g = 0;
+    else if (c01 < 0 && c12 > 0) g = 1;
+    else if (c02 < 0 && c12 < 0) g = 2;
+    if (int64_t(t1 + t2) < 2 * min_support) g = 3;                                       // :310
+    // rc = int(round(c, 0)), half to even (:291-292)
+    uint64_t r1 = (t1 >> 1) + ((t1 & 1) ? ((t1 >> 1) & 1) : 0);
+    uint64_t r2 = (t2 >> 1) + ((t2 & 1) ? ((t2 >> 1) & 1) : 0);
+    uint64_t nn = r1 + r2;
+    double kval;
+    bool have_k = false;
+    if (k_override) {
+        double ko = k_override[o];
+        if (ko == ko) {
+            kval = ko;
+            have_k = true;
+        }
+    }
+    if (!have_k && nn <= lut_nmax) {
+        kval = lut[nn * (nn + 1) / 2 + r1];
+        have_k = true;
+    }
+    int64_t p0 = 0, p1 = 0, p2 = 0;
+    if (have_k) {
+        F192 k = f_from_double(kval, ok);                                                // :313
+        p0 = pl_of(f_add(l0, k));
+        p1 = pl_of(f_add(l1, k));
+        p2 = pl_of(f_add(l2, k));
+    } else {
+        fl |= SVJG_GT_NEED_K;
+    }
+    if (!ok) fl |= SVJG_GT_NEED_K;   // out-of-format value: never produce a wrong PL silently
+    gt[o] = uint8_t(g);
+    flags[o] = uint8_t(fl);
+    ad2[2 * o] = uint32_t(t1);
+    ad2[2 * o + 1] = uint32_t(t2);
+    pl[3 * o] = p0;
+    pl[3 * o + 1] = p1;
+    pl[3 * o + 2] = p2;
+}
+
 // Counters of all ranks, read where they lie: every rank's exchange region is mapped into this
 // process (CUDA IPC, NVLink peer access).  The kernel first waits until every rank has signalled
 // that its filter is done for this step, then every thread sums the per-rank counters of its SV --
@@ -154,74 +231,28 @@ __global__ void genotype_kernel(const uint32_t *__restrict__ counts, const __gri
             n1 = c.y;
         }
     }
-    // predict-genotype.py:216 — a key is "in the dict" once it has at least one hit
-    bool gate = (ty & 0x3F) <= 3 && !(ty & 0x80) && ty != 255 && idx != 0xFFFFFFFFu && ((n0 | n1) != 0 || (ty & 0x40));
-    if (!gate) {
-        gt[i] = 3;
-        flags[i] = 0;
-        ad2[2 * size_t(i)] = 0;
-        ad2[2 * size_t(i) + 1] = 0;
-        pl[3 * size_t(i)] = pl[3 * size_t(i) + 1] = pl[3 * size_t(i) + 2] = 0;
-        return;
+    genotype_one(n0, n1, idx, ty, min_support, la, lb, lh, lut, lut_nmax, k_override, i, pl, gt, ad2, flags);
+}
+
+// One thread per cell (record i, sample s) of a block of records.  The counters are the cohort's sample-major
+// matrix ([S][num_sv][2], as the filter writes a sample's counters); the results are record-major ([n][S], the
+// order of the VCF text).
+__global__ void genotype_cohort_kernel(const uint32_t *__restrict__ counts, uint32_t num_sv, uint32_t n_samples,
+                                       const uint32_t *__restrict__ sv_index, const uint8_t *__restrict__ svtype,
+                                       uint32_t n_cells, int64_t min_support, double la, double lb, double lh,
+                                       const double *__restrict__ lut, uint32_t lut_nmax, int64_t *__restrict__ pl,
+                                       uint8_t *__restrict__ gt, uint32_t *__restrict__ ad2, uint8_t *__restrict__ flags) {
+    const uint32_t c = blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= n_cells) return;
+    const uint32_t i = c / n_samples, s = c - i * n_samples;
+    const uint32_t idx = sv_index[i];
+    uint32_t n0 = 0, n1 = 0;
+    if (idx != 0xFFFFFFFFu) {
+        const uint2 v = *reinterpret_cast<const uint2 *>(counts + (size_t(s) * num_sv + idx) * 2);
+        n0 = v.x;
+        n1 = v.y;
     }
-    ty &= 0x3F;
-    // allele_normalization (:327-338): counts in half units
-    uint64_t t1 = 2ull * n0, t2 = 2ull * n1;
-    uint32_t fl = SVJG_GT_GENOTYPED;
-    if (ty == 0 && n0 > 0) {
-        t1 = n0;
-        fl |= SVJG_GT_HALVED_0;
-    } else if (ty == 1 && n1 > 0) {
-        t2 = n1;
-        fl |= SVJG_GT_HALVED_1;
-    }
-    double c1 = double(t1) * 0.5, c2 = double(t2) * 0.5, cs = double(t1 + t2) * 0.5;   // exact
-    bool ok = true;
-    // :295-297 — each product is the double the reference computes
-    F192 l0 = f_add(f_from_double(__dmul_rn(c1, la), ok), f_from_double(__dmul_rn(c2, lb), ok));
-    F192 l1 = f_from_double(__dmul_rn(cs, lh), ok);
-    F192 l2 = f_add(f_from_double(__dmul_rn(c2, la), ok), f_from_double(__dmul_rn(c1, lb), ok));
-    // unique argmax (:301-307)
-    int c01 = f_cmp(l0, l1), c02 = f_cmp(l0, l2), c12 = f_cmp(l1, l2);
-    uint32_t g = 3;
-    if (c01 > 0 && c02 > 0) g = 0;
-    else if (c01 < 0 && c12 > 0) g = 1;
-    else if (c02 < 0 && c12 < 0) g = 2;
-    if (int64_t(t1 + t2) < 2 * min_support) g = 3;                                       // :310
-    // rc = int(round(c, 0)), half to even (:291-292)
-    uint64_t r1 = (t1 >> 1) + ((t1 & 1) ? ((t1 >> 1) & 1) : 0);
-    uint64_t r2 = (t2 >> 1) + ((t2 & 1) ? ((t2 >> 1) & 1) : 0);
-    uint64_t nn = r1 + r2;
-    double kval;
-    bool have_k = false;
-    if (k_override) {
-        double ko = k_override[i];
-        if (ko == ko) {
-            kval = ko;
-            have_k = true;
-        }
-    }
-    if (!have_k && nn <= lut_nmax) {
-        kval = lut[nn * (nn + 1) / 2 + r1];
-        have_k = true;
-    }
-    int64_t p0 = 0, p1 = 0, p2 = 0;
-    if (have_k) {
-        F192 k = f_from_double(kval, ok);                                                // :313
-        p0 = pl_of(f_add(l0, k));
-        p1 = pl_of(f_add(l1, k));
-        p2 = pl_of(f_add(l2, k));
-    } else {
-        fl |= SVJG_GT_NEED_K;
-    }
-    if (!ok) fl |= SVJG_GT_NEED_K;   // out-of-format value: never produce a wrong PL silently
-    gt[i] = uint8_t(g);
-    flags[i] = uint8_t(fl);
-    ad2[2 * size_t(i)] = uint32_t(t1);
-    ad2[2 * size_t(i) + 1] = uint32_t(t2);
-    pl[3 * size_t(i)] = p0;
-    pl[3 * size_t(i) + 1] = p1;
-    pl[3 * size_t(i) + 2] = p2;
+    genotype_one(n0, n1, idx, svtype[i], min_support, la, lb, lh, lut, lut_nmax, nullptr, c, pl, gt, ad2, flags);
 }
 
 }  // namespace
@@ -299,6 +330,65 @@ extern "C" int svjg_genotype_host(const uint32_t *counts, uint32_t num_counts, c
     cudaStreamDestroy(st);
     if (e != cudaSuccess) return svjg::cuda_fail(int(e), "svjg_genotype_host");
     return rc;
+}
+
+// ---------------------------------------------------------------------------
+// cohort: one block of records genotyped in every sample
+// ---------------------------------------------------------------------------
+extern "C" int svjg_cohort_genotype(svjg_cohort *c, const uint32_t *sv_index, const uint8_t *svtype, uint32_t n,
+                                    int64_t min_support, double log10_1me, double log10_e, double log10_half,
+                                    const double *lut, uint32_t lut_nmax, int64_t *pl, uint8_t *gt, uint32_t *ad2,
+                                    uint8_t *flags) {
+    if (!c) return svjg::set_error(SVJG_E_ARG, "svjg_cohort_genotype: NULL cohort");
+    if (n == 0) return SVJG_OK;
+    if (!sv_index || !svtype || !lut || !pl || !gt || !ad2 || !flags)
+        return svjg::set_error(SVJG_E_ARG, "svjg_cohort_genotype: NULL argument");
+    if (!(log10_1me == log10_1me) || !(log10_e == log10_e) || !(log10_half == log10_half))
+        return svjg::set_error(SVJG_E_ARG, "svjg_cohort_genotype: NaN constant");
+    const uint64_t cells = uint64_t(n) * c->n_samples;
+    if (cells >= 0xFFFFFFFFull) return svjg::set_error(SVJG_E_ARG, "svjg_cohort_genotype: block of more than 2^32 cells");
+    for (uint32_t i = 0; i < n; ++i)
+        if (sv_index[i] != 0xFFFFFFFFu && sv_index[i] >= c->num_sv)
+            return svjg::set_error(SVJG_E_ARG, "svjg_cohort_genotype: sv_index out of range");
+    SVJG_CUDA(cudaSetDevice(c->t->device));
+    // the LUT is uploaded again only when its contents change
+    const size_t n_lut = size_t(lut_nmax + 1) * (lut_nmax + 2) / 2;
+    if (c->lut.size() != n_lut || memcmp(c->lut.data(), lut, n_lut * 8) != 0) {
+        if (c->d_lut) SVJG_CUDA(cudaFree(c->d_lut));
+        c->d_lut = nullptr;
+        c->lut.clear();
+        SVJG_CUDA(cudaMalloc(&c->d_lut, n_lut * 8));
+        SVJG_CUDA(cudaMemcpy(c->d_lut, lut, n_lut * 8, cudaMemcpyHostToDevice));
+        c->lut.assign(lut, lut + n_lut);
+    }
+    auto up = [](size_t x) { return (x + 255) & ~size_t(255); };
+    const size_t b_idx = size_t(n) * 4, b_ty = n, b_pl = cells * 24, b_gt = cells, b_ad = cells * 8, b_fl = cells;
+    const size_t o_ty = up(b_idx), o_pl = o_ty + up(b_ty), o_gt = o_pl + up(b_pl), o_ad = o_gt + up(b_gt),
+                 o_fl = o_ad + up(b_ad), total = o_fl + up(b_fl);
+    if (c->blk_cap < total) {
+        if (c->d_blk) SVJG_CUDA(cudaFree(c->d_blk));
+        c->d_blk = nullptr;
+        c->blk_cap = 0;
+        SVJG_CUDA(cudaMalloc(&c->d_blk, total));
+        c->blk_cap = total;
+    }
+    uint8_t *d = c->d_blk;
+    cudaStream_t st = c->stream;
+    SVJG_CUDA(cudaMemcpyAsync(d, sv_index, b_idx, cudaMemcpyHostToDevice, st));
+    SVJG_CUDA(cudaMemcpyAsync(d + o_ty, svtype, b_ty, cudaMemcpyHostToDevice, st));
+    const int threads = 128;
+    const uint32_t blocks = uint32_t((cells + threads - 1) / threads);
+    genotype_cohort_kernel<<<blocks, threads, 0, st>>>(c->d_counts, c->num_sv, c->n_samples, reinterpret_cast<const uint32_t *>(d),
+                                                       d + o_ty, uint32_t(cells), min_support, log10_1me, log10_e, log10_half,
+                                                       c->d_lut, lut_nmax, reinterpret_cast<int64_t *>(d + o_pl), d + o_gt,
+                                                       reinterpret_cast<uint32_t *>(d + o_ad), d + o_fl);
+    SVJG_CUDA(cudaGetLastError());
+    SVJG_CUDA(cudaMemcpyAsync(pl, d + o_pl, b_pl, cudaMemcpyDeviceToHost, st));
+    SVJG_CUDA(cudaMemcpyAsync(gt, d + o_gt, b_gt, cudaMemcpyDeviceToHost, st));
+    SVJG_CUDA(cudaMemcpyAsync(ad2, d + o_ad, b_ad, cudaMemcpyDeviceToHost, st));
+    SVJG_CUDA(cudaMemcpyAsync(flags, d + o_fl, b_fl, cudaMemcpyDeviceToHost, st));
+    SVJG_CUDA(cudaStreamSynchronize(st));
+    return SVJG_OK;
 }
 
 // ---------------------------------------------------------------------------

@@ -33,6 +33,18 @@ struct svjg_tables {
     svjg::JsonKeys *json_keys = nullptr;
 };
 
+// counters of S samples against one catalogue (api.cu), genotyped block by block (genotype.cu)
+struct svjg_cohort {
+    svjg_tables *t = nullptr;
+    uint32_t n_samples = 0, num_sv = 0;
+    uint32_t *d_counts = nullptr;             // [n_samples][num_sv][2], sample-major
+    cudaStream_t stream = nullptr;
+    std::vector<double> lut;                  // host copy of what d_lut holds
+    double *d_lut = nullptr;
+    uint8_t *d_blk = nullptr;                 // inputs and results of the last block
+    size_t blk_cap = 0;
+};
+
 namespace svjg {
 // where the bytes of a file lie on the device(s): range k = file offsets [start[k], start[k + 1]) at base[k]
 // (device 0's own memory or a peer's, read over NVLink).  One range for a file resident on one device.

@@ -7,6 +7,7 @@
 // byte, or a POS/END of more than 18 digits, is answered with SVJG_E_UNSUPPORTED and the caller uses
 // the Python statement instead.
 #include <cstdio>
+#include <algorithm>
 #include <cstring>
 #include <string>
 #include <string_view>
@@ -29,7 +30,7 @@ const char FORMAT_LINES[] =
     "##FORMAT=<ID=AD,Number=2,Type=Float,Description=\"Number of informative read alignments supporting each allele "
     "(after normalization by breakpoint number for unbalanced SVs)\">\n"
     "##FORMAT=<ID=PL,Number=3,Type=Integer,Description=\"Phred-scaled likelihood for each genotype\">\n"
-    "#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO\tFORMAT\tSAMPLE\n";
+    "#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO\tFORMAT\t";      // then the sample names and "\n"
 
 struct Rec {
     uint64_t head_off;   // into text
@@ -344,33 +345,40 @@ inline char *put_mem(char *o, const char *p, size_t n) {
 }
 }  // namespace
 
-extern "C" int svjg_vcf_format(const svjg_vcf *v, const uint8_t *gt, const uint8_t *flags, const uint32_t *ad2,
-                               const int64_t *pl, char **out, uint64_t *out_len, uint64_t *n_genotyped) {
-    if (!v || !out || !out_len) return set_error(SVJG_E_ARG, "svjg_vcf_format: NULL argument");
-    const size_t n = v->recs.size();
+// Records [lo, hi) with one column per sample; the arrays hold those records' cells, [hi - lo][S].
+extern "C" int svjg_vcf_format_cohort(const svjg_vcf *v, uint32_t lo, uint32_t hi, uint32_t n_samples, const char *names,
+                                      uint64_t names_len, const uint8_t *gt, const uint8_t *flags, const uint32_t *ad2,
+                                      const int64_t *pl, char **out, uint64_t *out_len, uint64_t *n_genotyped) {
+    if (!v || !out || !out_len || !names || !n_genotyped) return set_error(SVJG_E_ARG, "svjg_vcf_format: NULL argument");
+    const size_t n_all = v->recs.size();
+    if (lo > hi || hi > n_all || n_samples == 0) return set_error(SVJG_E_ARG, "svjg_vcf_format: bad record range or sample count");
+    const size_t S = n_samples, n = size_t(hi - lo), n_cells = n * S;
     if (n && (!gt || !flags || !ad2 || !pl)) return set_error(SVJG_E_ARG, "svjg_vcf_format: NULL argument");
-    for (size_t i = 0; i < n; ++i)
-        if ((flags[i] & SVJG_GT_GENOTYPED) && gt[i] > 3) return set_error(SVJG_E_ARG, "svjg_vcf_format: gt code out of range");
+    for (size_t k = 0; k < n_cells; ++k)
+        if ((flags[k] & SVJG_GT_GENOTYPED) && gt[k] > 3) return set_error(SVJG_E_ARG, "svjg_vcf_format: gt code out of range");
     static const char *GT_TEXT[4] = {"0/0", "0/1", "1/1", "./."};
-    // upper bound: every head and header line is a piece of the text; the sample column is at most
-    // 13 + 3 + 1 + 22 + 1 + 45 + 1 + 62 + 1 bytes; untouched pages of the block cost nothing
-    size_t cap = v->text.size() + n * 160 + 16;
-    for (const Hdr &h : v->hdrs)
-        if (h.len == UINT32_MAX) cap += sizeof FORMAT_LINES;
-    char *buf = (char *)malloc(cap);
-    if (!buf) return set_error(SVJG_E_NOMEM, "svjg_vcf_format: out of memory");
     const char *text = v->text.data();
+    // the header lines of the range: those in front of its records and, for the last range, the ones behind them
+    size_t h_lo = 0;
+    while (h_lo < v->hdrs.size() && v->hdrs[h_lo].before < lo) ++h_lo;
+    size_t h_hi = h_lo;
+    while (h_hi < v->hdrs.size() && (hi == n_all || v->hdrs[h_hi].before < hi)) ++h_hi;
+    const size_t col_hdr = sizeof FORMAT_LINES - 1 + names_len + 1;
+    auto hdr_len = [&](const Hdr &h) -> uint64_t { return h.len == UINT32_MAX ? col_hdr : h.len; };
     auto put_hdr = [&](char *o, const Hdr &h) {
-        return h.len == UINT32_MAX ? put_mem(o, FORMAT_LINES, sizeof FORMAT_LINES - 1) : put_mem(o, text + h.off, h.len);
+        if (h.len != UINT32_MAX) return put_mem(o, text + h.off, h.len);
+        o = put_mem(o, FORMAT_LINES, sizeof FORMAT_LINES - 1);
+        o = put_mem(o, names, names_len);
+        *o++ = '\n';
+        return o;
     };
-    // the sample column of record i (at most 150 bytes)
-    auto put_sample = [&](char *o, size_t i) {
-        o = put_mem(o, "\tGT:DP:AD:PL\t", 13);
-        const uint8_t f = flags[i];
+    // the text of cell k (at most 136 bytes)
+    auto put_sample = [&](char *o, size_t k) {
+        const uint8_t f = flags[k];
         if (f & SVJG_GT_GENOTYPED) {
-            const uint64_t t1 = ad2[2 * i], t2 = ad2[2 * i + 1];
+            const uint64_t t1 = ad2[2 * k], t2 = ad2[2 * k + 1];
             const bool h0 = f & SVJG_GT_HALVED_0, h1 = f & SVJG_GT_HALVED_1;
-            o = put_mem(o, GT_TEXT[gt[i]], 3);
+            o = put_mem(o, GT_TEXT[gt[k]], 3);
             *o++ = ':';
             o = put_half(o, t1 + t2, h0 || h1);
             *o++ = ':';
@@ -378,52 +386,66 @@ extern "C" int svjg_vcf_format(const svjg_vcf *v, const uint8_t *gt, const uint8
             *o++ = ',';
             o = put_half(o, t2, h1);
             *o++ = ':';
-            o = put_i64(o, pl[3 * i]);
+            o = put_i64(o, pl[3 * k]);
             *o++ = ',';
-            o = put_i64(o, pl[3 * i + 1]);
+            o = put_i64(o, pl[3 * k + 1]);
             *o++ = ',';
-            o = put_i64(o, pl[3 * i + 2]);
+            o = put_i64(o, pl[3 * k + 2]);
         } else {
             o = put_mem(o, "./.:0:0,0:.,.,.", 15);
+        }
+        return o;
+    };
+    // what follows the head of record lo + j: the FORMAT column and one column per sample
+    auto put_columns = [&](char *o, size_t j) {
+        o = put_mem(o, "\tGT:DP:AD:PL", 12);
+        for (size_t s = 0; s < S; ++s) {
+            *o++ = '\t';
+            o = put_sample(o, j * S + s);
         }
         *o++ = '\n';
         return o;
     };
-    // where every record starts: its head is copied as it is, the sample column is rendered once to learn
-    // its length (cheap next to the copies); then the records are filled in by several threads
-    std::vector<uint64_t> at(n + 1, 0);
-    uint64_t genotyped = 0;
+    // where every record starts: its head is copied as it is, the cells are rendered once to learn their
+    // length (cheap next to the copies); then the records are filled in by several threads
+    std::vector<uint64_t> at(n + 1, 0), genotyped(S, 0);
     {
-        char tmp[192];
-        size_t hi = 0;
+        char tmp[160];
+        size_t h = h_lo;
         uint64_t pos = 0;
-        for (size_t i = 0; i < n; ++i) {
-            while (hi < v->hdrs.size() && v->hdrs[hi].before <= i) {
-                const Hdr &h = v->hdrs[hi++];
-                pos += h.len == UINT32_MAX ? sizeof FORMAT_LINES - 1 : h.len;
+        for (size_t j = 0; j < n; ++j) {
+            while (h < h_hi && v->hdrs[h].before <= lo + j) pos += hdr_len(v->hdrs[h++]);
+            at[j] = pos;
+            pos += v->recs[lo + j].head_len + 13 + S;
+            for (size_t s = 0; s < S; ++s) {
+                const size_t k = j * S + s;
+                genotyped[s] += (flags[k] & SVJG_GT_GENOTYPED) != 0;
+                pos += uint64_t(put_sample(tmp, k) - tmp);
             }
-            at[i] = pos;
-            genotyped += (flags[i] & SVJG_GT_GENOTYPED) != 0;
-            pos += v->recs[i].head_len + uint64_t(put_sample(tmp, i) - tmp);
         }
         at[n] = pos;
     }
-    auto fill = [&](size_t lo, size_t hi_rec) {
-        size_t hi = 0;
-        while (hi < v->hdrs.size() && v->hdrs[hi].before < lo) ++hi;          // header lines in front of record lo: not ours
-        // (those with before == lo sit right in front of record lo: ours, they end where it starts)
-        for (size_t i = lo; i < hi_rec; ++i) {
+    uint64_t tail = 0;
+    {
+        size_t h = h_lo;
+        while (h < h_hi && (n != 0 && v->hdrs[h].before <= hi - 1)) ++h;
+        for (; h < h_hi; ++h) tail += hdr_len(v->hdrs[h]);
+    }
+    char *buf = (char *)malloc(at[n] + tail + 1);
+    if (!buf) return set_error(SVJG_E_NOMEM, "svjg_vcf_format: out of memory");
+    auto fill = [&](size_t a, size_t b) {
+        size_t h = h_lo;
+        while (h < h_hi && v->hdrs[h].before < lo + a) ++h;               // header lines in front of record a: not ours
+        // (those with before == lo + a sit right in front of it: ours, they end where it starts)
+        for (size_t j = a; j < b; ++j) {
             uint64_t back = 0;
-            size_t h2 = hi;
-            while (h2 < v->hdrs.size() && v->hdrs[h2].before <= i) {
-                back += v->hdrs[h2].len == UINT32_MAX ? sizeof FORMAT_LINES - 1 : v->hdrs[h2].len;
-                ++h2;
-            }
-            char *o = buf + at[i] - back;
-            while (hi < h2) o = put_hdr(o, v->hdrs[hi++]);
-            const Rec &r = v->recs[i];
+            size_t h2 = h;
+            while (h2 < h_hi && v->hdrs[h2].before <= lo + j) back += hdr_len(v->hdrs[h2++]);
+            char *o = buf + at[j] - back;
+            while (h < h2) o = put_hdr(o, v->hdrs[h++]);
+            const Rec &r = v->recs[lo + j];
             o = put_mem(o, text + r.head_off, r.head_len);
-            put_sample(o, i);
+            put_columns(o, j);
         }
     };
     const uint64_t body = at[n];
@@ -443,17 +465,27 @@ extern "C" int svjg_vcf_format(const svjg_vcf *v, const uint8_t *gt, const uint8
         fill(cutv[0], cutv[1]);
         for (auto &th : pool) th.join();
     }
-    // header lines behind the last record
+    // header lines behind the last record of the range
     char *o = buf + at[n];
     {
-        size_t hi = 0;
-        while (hi < v->hdrs.size() && (n == 0 ? false : v->hdrs[hi].before <= n - 1)) ++hi;
-        while (hi < v->hdrs.size()) o = put_hdr(o, v->hdrs[hi++]);
+        size_t h = h_lo;
+        while (h < h_hi && (n != 0 && v->hdrs[h].before <= hi - 1)) ++h;
+        while (h < h_hi) o = put_hdr(o, v->hdrs[h++]);
     }
     *out = buf;
     *out_len = uint64_t(o - buf);
-    if (n_genotyped) *n_genotyped = genotyped;
+    for (size_t s = 0; s < S; ++s) n_genotyped[s] += genotyped[s];
     return SVJG_OK;
+}
+
+extern "C" int svjg_vcf_format(const svjg_vcf *v, const uint8_t *gt, const uint8_t *flags, const uint32_t *ad2,
+                               const int64_t *pl, char **out, uint64_t *out_len, uint64_t *n_genotyped) {
+    if (!v) return set_error(SVJG_E_ARG, "svjg_vcf_format: NULL argument");
+    uint64_t genotyped = 0;
+    const int rc = svjg_vcf_format_cohort(v, 0, uint32_t(v->recs.size()), 1, "SAMPLE", 6, gt, flags, ad2, pl, out, out_len,
+                                          &genotyped);
+    if (rc == SVJG_OK && n_genotyped) *n_genotyped = genotyped;
+    return rc;
 }
 
 extern "C" void svjg_buffer_free(char *p) { free(p); }

@@ -232,6 +232,103 @@ def genotype_main(argv=None):
     return 0
 
 
+def _sample_name(path):
+    import os
+    name = os.path.basename(path)
+    if name.endswith(".gz"):
+        name = name[:-3]
+    if name.endswith(".gaf"):
+        name = name[:-4]
+    return name
+
+
+def _read_sample(files):
+    """The files of one sample as the filter front-end reads them (gzip / bgzip inflated, text-mode line ends),
+    each page-locked in place."""
+    from . import alnfilter, gzio
+    return [alnfilter.RegisteredBytes(alnfilter.translate_newlines(gzio.read_bytes(f))) for f in files]
+
+
+def cohort_main(argv=None):
+    """genotype-cohort.py (an extension; the reference genotypes one sample per run): many samples' GAF files
+    against one catalogue, one multi-sample VCF whose column s is what filter-alignments.py + predict-genotype.py
+    write for sample s alone.  The tables are loaded and the device started once; the counters of every sample stay
+    on the device."""
+    ap = argparse.ArgumentParser(description="Genotype one SV catalogue in many samples")
+    ap.add_argument("-p", "--prefix", metavar="<prefix>", type=str, required=False,
+                    help="<prefix>_svs_edges.json holds the link -> SV table")
+    ap.add_argument("-g", "--gfa", metavar="<graph_file>", required=True, help="variant graph in gfa format")
+    ap.add_argument("-v", "--vcf", metavar="<vcffile>", required=True, help="the SV catalogue in vcf format")
+    ap.add_argument("-a", "--gaf", metavar="<align_file>", nargs="+", required=True,
+                    help="one argument per sample; a comma-joined argument is one sample whose files are counted together")
+    ap.add_argument("-o", "--output", metavar="<output>", required=True, help="multi-sample VCF")
+    ap.add_argument("--names", metavar="<n1,n2,...>", default=None,
+                    help="sample names (default: the first file's name without .gz and .gaf)")
+    ap.add_argument("-ms", "--minsupport", metavar="<minNbAln>", type=int, default=3,
+                    help="Minimum number of alignments to genotype a SV (default: 3>=)")
+    ap.add_argument("-e", "--err", type=float, default=0.00005, help="allele error probability")
+    ap.add_argument("--min-overlap", metavar="<bases>", type=int, default=None,
+                    help="aligned bases required on each side of a breakpoint (default 100)")
+    args = ap.parse_args(argv)
+    import os
+    if not args.prefix:
+        _die("-p/--prefix is required: <prefix>_svs_edges.json holds the link -> SV table")
+    if os.environ.get("SVJG_GPUS", "1").strip() != "1":
+        _die("genotype-cohort runs on one GPU: SVJG_GPUS must be 1")
+    samples = [[f for f in a.split(",")] for a in args.gaf]
+    if any(not f for files in samples for f in files):
+        _die("empty file name in -a")
+    names = args.names.split(",") if args.names is not None else [_sample_name(files[0]) for files in samples]
+    if len(names) != len(samples):
+        _die(f"{len(names)} names for {len(samples)} samples")
+    for nm in names:
+        if not nm or any(c in nm for c in "\t\r\n"):
+            _die(f"bad sample name {nm!r}: names must be non-empty and hold no tab, CR or LF")
+    if len(set(names)) != len(names):
+        _die("sample names must be unique")
+    d_over = 100 if args.min_overlap is None else args.min_overlap
+    out_path = os.path.abspath(args.output)
+    from concurrent.futures import ThreadPoolExecutor
+
+    from . import alnfilter, capi, cohort, genotype, gzio
+    tmp = None
+    try:
+        _lap("")
+        ready = _start_device()
+        vcf = gzio.read_bytes(args.vcf)
+        _lap("VCF read")
+        tables = _load_tables(args.prefix, args.gfa, ready)
+        _lap("tables + context")
+        co = cohort.Cohort(tables, len(samples))
+        with ThreadPoolExecutor(1) as pool:
+            # sample k + 1 is read, inflated, translated and page-locked while sample k is filtered
+            nxt = pool.submit(_read_sample, samples[0])
+            for k, files in enumerate(samples):
+                bufs = nxt.result()
+                nxt = pool.submit(_read_sample, samples[k + 1]) if k + 1 < len(samples) else None
+                for f, b in zip(files, bufs):
+                    try:
+                        co.filter(k, b.array, d_over=d_over)
+                    except alnfilter.InputError as exc:
+                        raise alnfilter.InputError(f"sample {names[k]!r}, file {f}: {exc}") from None
+                del bufs
+                _lap(f"sample {k} filtered")
+        import tempfile
+        fd, tmp = tempfile.mkstemp(prefix="." + os.path.basename(out_path) + ".", dir=os.path.dirname(out_path))
+        with os.fdopen(fd, "wb") as out:
+            _, n_gt = cohort.genotype_cohort_vcf(tables, co, vcf, names, args.minsupport, args.err, out=out)
+        os.replace(tmp, out_path)
+        tmp = None
+        _lap("genotypes + VCF written")
+    except (alnfilter.InputError, genotype.VcfError, capi.SvjgError, OSError, ValueError) as exc:
+        if tmp is not None:
+            os.unlink(tmp)
+        _die(str(exc))
+    for nm, n in zip(names, n_gt):
+        print(f"Genotyped svs in {nm}: {n}")
+    return 0
+
+
 class _MapperOutput:
     """File-like view (read(n) only) of what ends up in <prefix>.gaf: what the file already holds (the
     reference appends, svjedi-graph.py:100-104), then the standard output of one mapper process after the
