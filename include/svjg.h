@@ -247,7 +247,15 @@ int svjg_genotype_host(const uint32_t *counts, uint32_t num_counts, const uint32
  *                           counts exceed lut_nmax get SVJG_GT_NEED_K; the caller recomputes those cells from their
  *                           counters, e.g. with svjg_genotype_host).  Outputs are host arrays [n][S]: pl [n][S][3],
  *                           gt, flags [n][S], ad2 [n][S][2].  The LUT and the block buffers are cached in the handle.
- *                           Synchronous. */
+ *                           Synchronous.
+ *   svjg_cohort_site_stats  population statistics of the records of the last svjg_cohort_genotype call (n must be
+ *                           its record count), from the gt codes that call left on the device; only these 32 B per
+ *                           record come back.  gcount [n][4] u32 = (r0, h, r2, m): cells with 0/0, 0/1, 1/1 and the
+ *                           rest (./.).  hwe [n], exchet [n]: the HWE exact test and the excess-heterozygosity p of
+ *                           (r0, h, r2) (Wigginton, Cutler & Abecasis 2005, in the fixed double-precision form of
+ *                           DESIGN.md §8a; 1 and 1 when no allele is rare, NS = 0 included).  SVJG_E_ARG when
+ *                           4 (S + 1)^2 >= 2^53.  The gt codes on the device are final: the NEED_K cells a caller
+ *                           recomputes keep their genotype.  Synchronous. */
 typedef struct svjg_cohort svjg_cohort;
 int svjg_cohort_create(svjg_tables *t, uint32_t n_samples, svjg_cohort **out);
 void svjg_cohort_free(svjg_cohort *c);
@@ -258,6 +266,7 @@ int svjg_cohort_load_counts(svjg_cohort *c, uint32_t sample, const uint32_t *cou
 int svjg_cohort_genotype(svjg_cohort *c, const uint32_t *sv_index, const uint8_t *svtype, uint32_t n, int64_t min_support,
                          double log10_1me, double log10_e, double log10_half, const double *lut, uint32_t lut_nmax,
                          int64_t *pl, uint8_t *gt, uint32_t *ad2, uint8_t *flags);
+int svjg_cohort_site_stats(svjg_cohort *c, uint32_t n, uint32_t *gcount, double *hwe, double *exchet);
 
 /* Page-locked host memory (cudaHostAlloc) for file buffers and results: copies to and from it run
  * at PCIe speed.  For callers that do not want a tensor library just to pin memory. */
@@ -359,6 +368,31 @@ int svjg_vcf_format(const svjg_vcf *v, const uint8_t *gt, const uint8_t *flags, 
 int svjg_vcf_format_cohort(const svjg_vcf *v, uint32_t lo, uint32_t hi, uint32_t n_samples, const char *names,
                            uint64_t names_len, const uint8_t *gt, const uint8_t *flags, const uint32_t *ad2,
                            const int64_t *pl, char **out, uint64_t *out_len, uint64_t *n_genotyped);
+/* svjg_vcf_format_cohort_tags: svjg_vcf_format_cohort with population INFO tags; svjg_vcf_format_cohort is this with
+ * tags = 0 (then gcount, hwe and exchet may be NULL).  `tags` is a mask of SVJG_TAG_*; the tags are written in the
+ * order of the bits whatever the mask, with the ##INFO descriptions of bcftools +fill-tags.  gcount [hi - lo][4],
+ * hwe and exchet [hi - lo] are svjg_cohort_site_stats's arrays for the range (r0 + h + r2 + m must be n_samples).
+ *   NS = r0 + h + r2, AN = 2 NS, AC = h + 2 r2, AF = AC / AN ("." when AN = 0), AC_Het = h, AC_Hom = 2 r2,
+ *   F_MISSING = m / S, HWE and ExcHet ("." when NS = 0).  Floats are C's "%.6g" of the double.  The genotype codes
+ *   are biallelic: a record whose ALT holds a comma gets "." for the Number=A tags (AC, AF, AC_Het, AC_Hom, HWE,
+ *   ExcHet).
+ * INFO: the items of the record's INFO (split on ';'; "." or empty is no item) whose key (the text before the first
+ * '=') is a selected tag are dropped, the others kept in order, then TAG=value is appended per selected tag.  Header:
+ * the catalogue's ##INFO lines of a selected ID are dropped; the new ones are written in front of the ##FORMAT
+ * lines.  The bytes do not depend on how the records are cut into ranges. */
+#define SVJG_TAG_NS 0x001u
+#define SVJG_TAG_AN 0x002u
+#define SVJG_TAG_AC 0x004u
+#define SVJG_TAG_AF 0x008u
+#define SVJG_TAG_AC_HET 0x010u
+#define SVJG_TAG_AC_HOM 0x020u
+#define SVJG_TAG_F_MISSING 0x040u
+#define SVJG_TAG_HWE 0x080u
+#define SVJG_TAG_EXCHET 0x100u
+int svjg_vcf_format_cohort_tags(const svjg_vcf *v, uint32_t lo, uint32_t hi, uint32_t n_samples, const char *names,
+                                uint64_t names_len, const uint8_t *gt, const uint8_t *flags, const uint32_t *ad2,
+                                const int64_t *pl, uint32_t tags, const uint32_t *gcount, const double *hwe,
+                                const double *exchet, char **out, uint64_t *out_len, uint64_t *n_genotyped);
 void svjg_buffer_free(char *p);
 
 /* ---- output (host) ------------------------------------------------------------

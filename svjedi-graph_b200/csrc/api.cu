@@ -378,6 +378,7 @@ extern "C" void svjg_cohort_free(svjg_cohort *c) {
     if (c->d_counts) cudaFree(c->d_counts);
     if (c->d_lut) cudaFree(c->d_lut);
     if (c->d_blk) cudaFree(c->d_blk);
+    if (c->d_site) cudaFree(c->d_site);
     if (c->stream) cudaStreamDestroy(c->stream);
     delete c;
 }

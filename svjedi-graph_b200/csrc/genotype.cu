@@ -255,6 +255,108 @@ __global__ void genotype_cohort_kernel(const uint32_t *__restrict__ counts, uint
     genotype_one(n0, n1, idx, svtype[i], min_support, la, lb, lh, lut, lut_nmax, nullptr, c, pl, gt, ad2, flags);
 }
 
+// One term step of the Wigginton-Cutler-Abecasis walk: v * D / E with D and E exact integers (below 2^53), each
+// operation one IEEE double rounded to nearest (the Python statement computes the same doubles, DESIGN.md §8a).
+__device__ __forceinline__ double hwe_step(double v, uint64_t d, uint64_t e) {
+    return __ddiv_rn(__dmul_rn(v, double(d)), double(e));
+}
+
+// HWE exact test and excess-heterozygosity p of r0 / h / r2 genotype counts (Wigginton, Cutler & Abecasis 2005) in
+// the streaming form of DESIGN.md §8a: the terms, indexed by het count k, are walked down from `mid`, then up from
+// it, twice.  Pass 1 sums them all (and those with k >= h); pass 2 sums those no larger than the observed one.  A
+// walk stops at its first zero term: every later one is zero too, and adding zero changes no sum.
+__device__ void site_exact_tests(uint32_t r0, uint32_t h, uint32_t r2, double &hwe, double &exchet) {
+    const uint64_t N = uint64_t(r0) + h + r2;
+    const uint64_t rare = 2ull * min(r0, r2) + h;
+    if (rare == 0) {                                   // N == 0 included
+        hwe = exchet = 1.0;
+        return;
+    }
+    uint64_t mid = rare * (2 * N - rare) / (2 * N);
+    if ((mid ^ rare) & 1) ++mid;
+    double sum = 1.0, acc_exc = mid >= h ? 1.0 : 0.0, v_obs = mid == h ? 1.0 : 0.0;
+    for (int pass = 0; pass < 2; ++pass) {
+        double acc_hwe = 1.0 <= v_obs ? 1.0 : 0.0;
+        {   // down
+            uint64_t k = mid, homr = (rare - mid) / 2, homc = N - mid - homr;
+            double v = 1.0;
+            while (k >= 2) {
+                v = hwe_step(v, k * (k - 1), 4 * (homr + 1) * (homc + 1));
+                k -= 2;
+                ++homr;
+                ++homc;
+                if (pass == 0) {
+                    sum = __dadd_rn(sum, v);
+                    if (k >= h) acc_exc = __dadd_rn(acc_exc, v);
+                    if (k == h) v_obs = v;
+                } else if (v <= v_obs) {
+                    acc_hwe = __dadd_rn(acc_hwe, v);
+                }
+                if (v == 0.0) break;
+            }
+        }
+        {   // up
+            uint64_t k = mid, homr = (rare - mid) / 2, homc = N - mid - homr;
+            double v = 1.0;
+            while (k + 2 <= rare) {
+                v = hwe_step(v, 4 * homr * homc, (k + 2) * (k + 1));
+                k += 2;
+                --homr;
+                --homc;
+                if (pass == 0) {
+                    sum = __dadd_rn(sum, v);
+                    if (k >= h) acc_exc = __dadd_rn(acc_exc, v);
+                    if (k == h) v_obs = v;
+                } else if (v <= v_obs) {
+                    acc_hwe = __dadd_rn(acc_hwe, v);
+                }
+                if (v == 0.0) break;
+            }
+        }
+        if (pass == 1) hwe = fmin(1.0, __ddiv_rn(acc_hwe, sum));
+    }
+    exchet = fmin(1.0, __ddiv_rn(acc_exc, sum));
+}
+
+// Site statistics of a block of records from the genotype codes the cohort kernel left on the device ([n][S]).
+// A block of SITE_THREADS records: each warp counts the 0/0, 0/1 and 1/1 cells of its records (coalesced byte loads
+// along the row, one warp reduction), then every thread runs the exact tests of one record, which are serial per
+// record.  Results: gcount[i] = (r0, h, r2, missing), hwe[i], exchet[i].
+constexpr int SITE_THREADS = 256;
+__global__ void __launch_bounds__(SITE_THREADS)
+cohort_site_stats_kernel(const uint8_t *__restrict__ gt, uint32_t n, uint32_t n_samples, uint4 *__restrict__ gcount,
+                         double *__restrict__ hwe, double *__restrict__ exchet) {
+    __shared__ uint32_t cnt[3][SITE_THREADS];
+    const uint32_t base = blockIdx.x * SITE_THREADS, lane = threadIdx.x & 31;
+    for (uint32_t r = threadIdx.x >> 5; r < SITE_THREADS && base + r < n; r += SITE_THREADS / 32) {
+        const uint8_t *row = gt + size_t(base + r) * n_samples;
+        uint32_t c0 = 0, c1 = 0, c2 = 0;
+        for (uint32_t s = lane; s < n_samples; s += 32) {
+            const uint32_t g = row[s];
+            c0 += g == 0;
+            c1 += g == 1;
+            c2 += g == 2;
+        }
+        c0 = __reduce_add_sync(0xFFFFFFFFu, c0);
+        c1 = __reduce_add_sync(0xFFFFFFFFu, c1);
+        c2 = __reduce_add_sync(0xFFFFFFFFu, c2);
+        if (lane == 0) {
+            cnt[0][r] = c0;
+            cnt[1][r] = c1;
+            cnt[2][r] = c2;
+        }
+    }
+    __syncthreads();
+    const uint32_t i = base + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t r0 = cnt[0][threadIdx.x], h = cnt[1][threadIdx.x], r2 = cnt[2][threadIdx.x];
+    gcount[i] = make_uint4(r0, h, r2, n_samples - r0 - h - r2);
+    double p_hwe, p_exc;
+    site_exact_tests(r0, h, r2, p_hwe, p_exc);
+    hwe[i] = p_hwe;
+    exchet[i] = p_exc;
+}
+
 }  // namespace
 
 extern "C" int svjg_genotype_device(const uint32_t *d_counts, const uint32_t *d_sv_index, const uint8_t *d_svtype,
@@ -340,6 +442,7 @@ extern "C" int svjg_cohort_genotype(svjg_cohort *c, const uint32_t *sv_index, co
                                     const double *lut, uint32_t lut_nmax, int64_t *pl, uint8_t *gt, uint32_t *ad2,
                                     uint8_t *flags) {
     if (!c) return svjg::set_error(SVJG_E_ARG, "svjg_cohort_genotype: NULL cohort");
+    c->blk_n = 0;                          // set again once this block's cells are complete
     if (n == 0) return SVJG_OK;
     if (!sv_index || !svtype || !lut || !pl || !gt || !ad2 || !flags)
         return svjg::set_error(SVJG_E_ARG, "svjg_cohort_genotype: NULL argument");
@@ -387,6 +490,44 @@ extern "C" int svjg_cohort_genotype(svjg_cohort *c, const uint32_t *sv_index, co
     SVJG_CUDA(cudaMemcpyAsync(gt, d + o_gt, b_gt, cudaMemcpyDeviceToHost, st));
     SVJG_CUDA(cudaMemcpyAsync(ad2, d + o_ad, b_ad, cudaMemcpyDeviceToHost, st));
     SVJG_CUDA(cudaMemcpyAsync(flags, d + o_fl, b_fl, cudaMemcpyDeviceToHost, st));
+    SVJG_CUDA(cudaStreamSynchronize(st));
+    c->blk_n = n;
+    c->blk_gt = o_gt;
+    return SVJG_OK;
+}
+
+// Site statistics of the block of the last svjg_cohort_genotype call, from its gt codes where the kernel left them
+// on the device: 32 B per record come back, not the cells.
+extern "C" int svjg_cohort_site_stats(svjg_cohort *c, uint32_t n, uint32_t *gcount, double *hwe, double *exchet) {
+    if (!c) return svjg::set_error(SVJG_E_ARG, "svjg_cohort_site_stats: NULL cohort");
+    if (n != c->blk_n)
+        return svjg::set_error(SVJG_E_ARG, "svjg_cohort_site_stats: n is not the record count of the last svjg_cohort_genotype call");
+    if (n == 0) return SVJG_OK;
+    if (!gcount || !hwe || !exchet) return svjg::set_error(SVJG_E_ARG, "svjg_cohort_site_stats: NULL argument");
+    // every D and E of the exact tests must be exact in a double
+    const uint64_t s1 = uint64_t(c->n_samples) + 1;
+    if (s1 >= (1ull << 26) || 4 * s1 * s1 >= (1ull << 53))
+        return svjg::set_error(SVJG_E_ARG, "svjg_cohort_site_stats: 4 (S + 1)^2 must be below 2^53");
+    SVJG_CUDA(cudaSetDevice(c->t->device));
+    auto up = [](size_t x) { return (x + 255) & ~size_t(255); };
+    const size_t b_cnt = size_t(n) * 16, b_p = size_t(n) * 8, o_hwe = up(b_cnt), o_exc = o_hwe + up(b_p), total = o_exc + up(b_p);
+    if (c->site_cap < total) {
+        if (c->d_site) SVJG_CUDA(cudaFree(c->d_site));
+        c->d_site = nullptr;
+        c->site_cap = 0;
+        SVJG_CUDA(cudaMalloc(&c->d_site, total));
+        c->site_cap = total;
+    }
+    uint8_t *d = c->d_site;
+    cudaStream_t st = c->stream;
+    const uint32_t blocks = uint32_t((uint64_t(n) + SITE_THREADS - 1) / SITE_THREADS);
+    cohort_site_stats_kernel<<<blocks, SITE_THREADS, 0, st>>>(c->d_blk + c->blk_gt, n, c->n_samples, reinterpret_cast<uint4 *>(d),
+                                                              reinterpret_cast<double *>(d + o_hwe),
+                                                              reinterpret_cast<double *>(d + o_exc));
+    SVJG_CUDA(cudaGetLastError());
+    SVJG_CUDA(cudaMemcpyAsync(gcount, d, b_cnt, cudaMemcpyDeviceToHost, st));
+    SVJG_CUDA(cudaMemcpyAsync(hwe, d + o_hwe, b_p, cudaMemcpyDeviceToHost, st));
+    SVJG_CUDA(cudaMemcpyAsync(exchet, d + o_exc, b_p, cudaMemcpyDeviceToHost, st));
     SVJG_CUDA(cudaStreamSynchronize(st));
     return SVJG_OK;
 }

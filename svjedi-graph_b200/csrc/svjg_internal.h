@@ -43,6 +43,10 @@ struct svjg_cohort {
     double *d_lut = nullptr;
     uint8_t *d_blk = nullptr;                 // inputs and results of the last block
     size_t blk_cap = 0;
+    uint32_t blk_n = 0;                       // records of the last block genotyped (0: none)
+    size_t blk_gt = 0;                        // offset of its gt codes [blk_n][n_samples] in d_blk
+    uint8_t *d_site = nullptr;                // site statistics of the last block (svjg_cohort_site_stats)
+    size_t site_cap = 0;
 };
 
 namespace svjg {

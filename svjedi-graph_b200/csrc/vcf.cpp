@@ -343,34 +343,157 @@ inline char *put_mem(char *o, const char *p, size_t n) {
     memcpy(o, p, n);
     return o + n;
 }
+
+// The population INFO tags of a cohort VCF, in the order they are written (bit k of the mask is entry k), with the
+// header lines bcftools +fill-tags writes for them, so that filter expressions written for those read the same.
+struct InfoTag {
+    sv id;
+    bool per_alt;       // Number=A
+    const char *hdr;
+};
+const InfoTag INFO_TAGS[] = {
+    {"NS", false, "##INFO=<ID=NS,Number=1,Type=Integer,Description=\"Number of samples with data\">\n"},
+    {"AN", false, "##INFO=<ID=AN,Number=1,Type=Integer,Description=\"Total number of alleles in called genotypes\">\n"},
+    {"AC", true, "##INFO=<ID=AC,Number=A,Type=Integer,Description=\"Allele count in genotypes\">\n"},
+    {"AF", true, "##INFO=<ID=AF,Number=A,Type=Float,Description=\"Allele frequency\">\n"},
+    {"AC_Het", true, "##INFO=<ID=AC_Het,Number=A,Type=Integer,Description=\"Allele counts in heterozygous genotypes\">\n"},
+    {"AC_Hom", true, "##INFO=<ID=AC_Hom,Number=A,Type=Integer,Description=\"Allele counts in homozygous genotypes\">\n"},
+    {"F_MISSING", false, "##INFO=<ID=F_MISSING,Number=1,Type=Float,Description=\"Fraction of missing genotypes\">\n"},
+    {"HWE", true, "##INFO=<ID=HWE,Number=A,Type=Float,Description=\"HWE test (PMID:15789306); 1=good, 0=bad\">\n"},
+    {"ExcHet", true, "##INFO=<ID=ExcHet,Number=A,Type=Float,Description=\"Test excess heterozygosity; 1=good, 0=bad\">\n"},
+};
+constexpr uint32_t N_INFO_TAGS = sizeof INFO_TAGS / sizeof INFO_TAGS[0];
+
+bool selected_tag(uint32_t tags, sv key) {
+    for (uint32_t t = 0; t < N_INFO_TAGS; ++t)
+        if ((tags >> t & 1) && key == INFO_TAGS[t].id) return true;
+    return false;
+}
+
+// "##INFO=<ID=X," or "##INFO=<ID=X>" for a selected X
+bool info_header_of(uint32_t tags, sv line) {
+    if (!starts_with(line, "##INFO=<ID=")) return false;
+    const sv rest = line.substr(11);
+    const size_t e = rest.find_first_of(",>");
+    return e != sv::npos && selected_tag(tags, rest.substr(0, e));
+}
+
+// The value text of tag t for counts g = (r0, h, r2, m) of S cells; "." where it has none
+size_t tag_value(char *o, uint32_t t, const uint32_t *g, uint64_t S, double hwe, double exchet, bool multi_alt) {
+    if (INFO_TAGS[t].per_alt && multi_alt) {
+        *o = '.';
+        return 1;
+    }
+    const uint64_t r0 = g[0], h = g[1], r2 = g[2], m = g[3], ns = r0 + h + r2;
+    auto num = [&](uint64_t x) { return size_t(put_u64(o, x) - o); };
+    auto flt = [&](bool have, double x) -> size_t {
+        if (!have) {
+            *o = '.';
+            return 1;
+        }
+        return size_t(snprintf(o, 32, "%.6g", x));
+    };
+    switch (1u << t) {
+        case SVJG_TAG_NS: return num(ns);
+        case SVJG_TAG_AN: return num(2 * ns);
+        case SVJG_TAG_AC: return num(h + 2 * r2);
+        case SVJG_TAG_AF: return flt(ns != 0, double(h + 2 * r2) / double(2 * ns));
+        case SVJG_TAG_AC_HET: return num(h);
+        case SVJG_TAG_AC_HOM: return num(2 * r2);
+        case SVJG_TAG_F_MISSING: return flt(true, double(m) / double(S));
+        case SVJG_TAG_HWE: return flt(ns != 0, hwe);
+        default: return flt(ns != 0, exchet);
+    }
+}
 }  // namespace
 
 // Records [lo, hi) with one column per sample; the arrays hold those records' cells, [hi - lo][S].
-extern "C" int svjg_vcf_format_cohort(const svjg_vcf *v, uint32_t lo, uint32_t hi, uint32_t n_samples, const char *names,
-                                      uint64_t names_len, const uint8_t *gt, const uint8_t *flags, const uint32_t *ad2,
-                                      const int64_t *pl, char **out, uint64_t *out_len, uint64_t *n_genotyped) {
+extern "C" int svjg_vcf_format_cohort_tags(const svjg_vcf *v, uint32_t lo, uint32_t hi, uint32_t n_samples, const char *names,
+                                           uint64_t names_len, const uint8_t *gt, const uint8_t *flags, const uint32_t *ad2,
+                                           const int64_t *pl, uint32_t tags, const uint32_t *gcount, const double *hwe,
+                                           const double *exchet, char **out, uint64_t *out_len, uint64_t *n_genotyped) {
     if (!v || !out || !out_len || !names || !n_genotyped) return set_error(SVJG_E_ARG, "svjg_vcf_format: NULL argument");
     const size_t n_all = v->recs.size();
     if (lo > hi || hi > n_all || n_samples == 0) return set_error(SVJG_E_ARG, "svjg_vcf_format: bad record range or sample count");
     const size_t S = n_samples, n = size_t(hi - lo), n_cells = n * S;
     if (n && (!gt || !flags || !ad2 || !pl)) return set_error(SVJG_E_ARG, "svjg_vcf_format: NULL argument");
+    if (tags >> N_INFO_TAGS) return set_error(SVJG_E_ARG, "svjg_vcf_format: unknown INFO tag bit");
+    // every tag needs the counts (HWE and ExcHet are "." when NS = 0)
+    if (n && tags && (!gcount || ((tags & SVJG_TAG_HWE) && !hwe) || ((tags & SVJG_TAG_EXCHET) && !exchet)))
+        return set_error(SVJG_E_ARG, "svjg_vcf_format: NULL site statistics");
+    if (tags) {
+        for (size_t j = 0; j < n; ++j)
+            if (uint64_t(gcount[4 * j]) + gcount[4 * j + 1] + gcount[4 * j + 2] + gcount[4 * j + 3] != S)
+                return set_error(SVJG_E_ARG, "svjg_vcf_format: genotype counts do not add up to the sample count");
+    }
     for (size_t k = 0; k < n_cells; ++k)
         if ((flags[k] & SVJG_GT_GENOTYPED) && gt[k] > 3) return set_error(SVJG_E_ARG, "svjg_vcf_format: gt code out of range");
     static const char *GT_TEXT[4] = {"0/0", "0/1", "1/1", "./."};
     const char *text = v->text.data();
+    std::string info_hdr;                  // the ##INFO lines of the selected tags, in front of the ##FORMAT lines
+    for (uint32_t t = 0; t < N_INFO_TAGS; ++t)
+        if (tags >> t & 1) info_hdr += INFO_TAGS[t].hdr;
     // the header lines of the range: those in front of its records and, for the last range, the ones behind them
     size_t h_lo = 0;
     while (h_lo < v->hdrs.size() && v->hdrs[h_lo].before < lo) ++h_lo;
     size_t h_hi = h_lo;
     while (h_hi < v->hdrs.size() && (hi == n_all || v->hdrs[h_hi].before < hi)) ++h_hi;
-    const size_t col_hdr = sizeof FORMAT_LINES - 1 + names_len + 1;
-    auto hdr_len = [&](const Hdr &h) -> uint64_t { return h.len == UINT32_MAX ? col_hdr : h.len; };
+    const size_t col_hdr = info_hdr.size() + sizeof FORMAT_LINES - 1 + names_len + 1;
+    auto dropped = [&](const Hdr &h) { return tags && info_header_of(tags, sv(text + h.off, h.len)); };
+    auto hdr_len = [&](const Hdr &h) -> uint64_t { return h.len == UINT32_MAX ? col_hdr : dropped(h) ? 0 : h.len; };
     auto put_hdr = [&](char *o, const Hdr &h) {
-        if (h.len != UINT32_MAX) return put_mem(o, text + h.off, h.len);
+        if (h.len != UINT32_MAX) return dropped(h) ? o : put_mem(o, text + h.off, h.len);
+        o = put_mem(o, info_hdr.data(), info_hdr.size());
         o = put_mem(o, FORMAT_LINES, sizeof FORMAT_LINES - 1);
         o = put_mem(o, names, names_len);
         *o++ = '\n';
         return o;
+    };
+    // columns 1-8 of record lo + j: as the catalogue has them, or with the INFO column rewritten for the tags.
+    // o == nullptr: the length only
+    auto put_head = [&](char *o, size_t j) -> uint64_t {
+        const Rec &r = v->recs[lo + j];
+        const sv head(text + r.head_off, r.head_len);
+        uint64_t len = 0;
+        auto put = [&](const char *p, size_t k) {
+            if (o) memcpy(o + len, p, k);
+            len += k;
+        };
+        if (!tags) {
+            put(head.data(), head.size());
+            return len;
+        }
+        const size_t t7 = head.rfind('\t');            // the head has 8 columns: INFO is the last
+        put(head.data(), t7 + 1);
+        const sv info = head.substr(t7 + 1);
+        bool first = true;
+        if (!info.empty() && info != ".") {
+            for (size_t a = 0;;) {
+                size_t b = info.find(';', a);
+                if (b == sv::npos) b = info.size();
+                const sv item = info.substr(a, b - a);
+                if (!selected_tag(tags, item.substr(0, item.find('=')))) {
+                    if (!first) put(";", 1);
+                    put(item.data(), item.size());
+                    first = false;
+                }
+                if (b == info.size()) break;
+                a = b + 1;
+            }
+        }
+        size_t a = 0;
+        for (int c = 0; c < 4; ++c) a = head.find('\t', a) + 1;   // ALT: column 5
+        const bool multi_alt = head.substr(a, head.find('\t', a) - a).find(',') != sv::npos;
+        char val[40];
+        for (uint32_t t = 0; t < N_INFO_TAGS; ++t) {
+            if (!(tags >> t & 1)) continue;
+            if (!first) put(";", 1);
+            first = false;
+            put(INFO_TAGS[t].id.data(), INFO_TAGS[t].id.size());
+            put("=", 1);
+            put(val, tag_value(val, t, gcount + 4 * j, S, hwe ? hwe[j] : 0.0, exchet ? exchet[j] : 0.0, multi_alt));
+        }
+        return len;
     };
     // the text of cell k (at most 136 bytes)
     auto put_sample = [&](char *o, size_t k) {
@@ -416,7 +539,7 @@ extern "C" int svjg_vcf_format_cohort(const svjg_vcf *v, uint32_t lo, uint32_t h
         for (size_t j = 0; j < n; ++j) {
             while (h < h_hi && v->hdrs[h].before <= lo + j) pos += hdr_len(v->hdrs[h++]);
             at[j] = pos;
-            pos += v->recs[lo + j].head_len + 13 + S;
+            pos += put_head(nullptr, j) + 13 + S;
             for (size_t s = 0; s < S; ++s) {
                 const size_t k = j * S + s;
                 genotyped[s] += (flags[k] & SVJG_GT_GENOTYPED) != 0;
@@ -443,8 +566,7 @@ extern "C" int svjg_vcf_format_cohort(const svjg_vcf *v, uint32_t lo, uint32_t h
             while (h2 < h_hi && v->hdrs[h2].before <= lo + j) back += hdr_len(v->hdrs[h2++]);
             char *o = buf + at[j] - back;
             while (h < h2) o = put_hdr(o, v->hdrs[h++]);
-            const Rec &r = v->recs[lo + j];
-            o = put_mem(o, text + r.head_off, r.head_len);
+            o += put_head(o, j);
             put_columns(o, j);
         }
     };
@@ -476,6 +598,13 @@ extern "C" int svjg_vcf_format_cohort(const svjg_vcf *v, uint32_t lo, uint32_t h
     *out_len = uint64_t(o - buf);
     for (size_t s = 0; s < S; ++s) n_genotyped[s] += genotyped[s];
     return SVJG_OK;
+}
+
+extern "C" int svjg_vcf_format_cohort(const svjg_vcf *v, uint32_t lo, uint32_t hi, uint32_t n_samples, const char *names,
+                                      uint64_t names_len, const uint8_t *gt, const uint8_t *flags, const uint32_t *ad2,
+                                      const int64_t *pl, char **out, uint64_t *out_len, uint64_t *n_genotyped) {
+    return svjg_vcf_format_cohort_tags(v, lo, hi, n_samples, names, names_len, gt, flags, ad2, pl, 0, nullptr, nullptr, nullptr,
+                                       out, out_len, n_genotyped);
 }
 
 extern "C" int svjg_vcf_format(const svjg_vcf *v, const uint8_t *gt, const uint8_t *flags, const uint32_t *ad2,

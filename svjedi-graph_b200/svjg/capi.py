@@ -93,6 +93,7 @@ def _load():
         "svjg_cohort_load_counts": (C.c_int, [vp, C.c_uint32, u32p]),
         "svjg_cohort_genotype": (C.c_int, [vp, u32p, u8p, C.c_uint32, C.c_int64, C.c_double, C.c_double, C.c_double, f64p,
                                            C.c_uint32, i64p, u8p, u32p, u8p]),
+        "svjg_cohort_site_stats": (C.c_int, [vp, C.c_uint32, u32p, f64p, f64p]),
         "svjg_host_alloc": (C.c_int, [C.c_uint64, C.POINTER(C.c_void_p)]),
         "svjg_host_free": (C.c_int, [vp]),
         "svjg_host_register": (C.c_int, [vp, C.c_uint64]),
@@ -126,6 +127,9 @@ def _load():
                                       C.POINTER(C.c_uint64)]),
         "svjg_vcf_format_cohort": (C.c_int, [vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_char_p, C.c_uint64, u8p, u8p, u32p,
                                              i64p, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64), u64p]),
+        "svjg_vcf_format_cohort_tags": (C.c_int, [vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_char_p, C.c_uint64, u8p, u8p,
+                                                  u32p, i64p, C.c_uint32, u32p, f64p, f64p, C.POINTER(C.c_void_p),
+                                                  C.POINTER(C.c_uint64), u64p]),
         "svjg_buffer_free": (None, [vp]),
         "svjg_emit_informative_json": (C.c_int, [vp, u8p, C.c_uint64, u32p, u64p, u32p, C.c_uint64, C.c_char_p]),
         "svjg_emit_informative_json_mem": (C.c_int, [vp, u8p, C.c_uint64, u32p, u64p, u32p, C.c_uint64,

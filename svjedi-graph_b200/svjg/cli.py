@@ -269,10 +269,21 @@ def cohort_main(argv=None):
     ap.add_argument("-e", "--err", type=float, default=0.00005, help="allele error probability")
     ap.add_argument("--min-overlap", metavar="<bases>", type=int, default=None,
                     help="aligned bases required on each side of a breakpoint (default 100)")
+    ap.add_argument("--info-tags", metavar="<LIST>", default=None,
+                    help="population INFO tags computed over the samples, a comma list of NS, AN, AC, AF, AC_Het, "
+                         "AC_Hom, F_MISSING, HWE, ExcHet, or all (written in that order; default: none, the catalogue's "
+                         "INFO as it is)")
     args = ap.parse_args(argv)
     import os
     if not args.prefix:
         _die("-p/--prefix is required: <prefix>_svs_edges.json holds the link -> SV table")
+    info_tags = ()
+    if args.info_tags is not None:
+        from .cohort import parse_info_tags
+        try:
+            info_tags = parse_info_tags(args.info_tags)
+        except ValueError as exc:
+            _die(f"--info-tags: {exc}")
     if os.environ.get("SVJG_GPUS", "1").strip() != "1":
         _die("genotype-cohort runs on one GPU: SVJG_GPUS must be 1")
     samples = [[f for f in a.split(",")] for a in args.gaf]
@@ -316,7 +327,8 @@ def cohort_main(argv=None):
         import tempfile
         fd, tmp = tempfile.mkstemp(prefix="." + os.path.basename(out_path) + ".", dir=os.path.dirname(out_path))
         with os.fdopen(fd, "wb") as out:
-            _, n_gt = cohort.genotype_cohort_vcf(tables, co, vcf, names, args.minsupport, args.err, out=out)
+            _, n_gt = cohort.genotype_cohort_vcf(tables, co, vcf, names, args.minsupport, args.err, out=out,
+                                                 info_tags=info_tags)
         os.replace(tmp, out_path)
         tmp = None
         _lap("genotypes + VCF written")

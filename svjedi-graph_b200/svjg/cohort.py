@@ -14,6 +14,32 @@ from . import alnfilter, capi, genotype
 
 CELL_BYTES = 24 + 1 + 8 + 1          # pl, gt, ad2, flags of one cell
 BLOCK_BYTES = 256 << 20              # cell arrays of one block of records, at most
+# population INFO tags of --info-tags, in the order they are written: bit k of svjg_vcf_format_cohort_tags's mask
+INFO_TAGS = ("NS", "AN", "AC", "AF", "AC_Het", "AC_Hom", "F_MISSING", "HWE", "ExcHet")
+
+
+def parse_info_tags(text):
+    """--info-tags: a comma list of INFO_TAGS names (any order), or "all".  Returns the names in the order they are
+    written; ValueError for an unknown or repeated name or an empty list."""
+    if text == "all":
+        return INFO_TAGS
+    names = text.split(",")
+    for nm in names:
+        if nm not in INFO_TAGS:
+            raise ValueError(f"unknown INFO tag {nm!r} (tags: {','.join(INFO_TAGS)}, or all)")
+    if len(set(names)) != len(names):
+        raise ValueError("an INFO tag is named twice")
+    return tuple(t for t in INFO_TAGS if t in names)
+
+
+def info_tags_mask(names):
+    """The tag mask of svjg_vcf_format_cohort_tags for INFO_TAGS names."""
+    mask = 0
+    for nm in names:
+        if nm not in INFO_TAGS:
+            raise ValueError(f"unknown INFO tag {nm!r}")
+        mask |= 1 << INFO_TAGS.index(nm)
+    return mask
 
 
 class Cohort:
@@ -67,15 +93,22 @@ class Cohort:
 
 
 class _Block:
-    """Page-locked result arrays of one block of records: the copies from the device run at PCIe speed."""
+    """Page-locked result arrays of one block of records: the copies from the device run at PCIe speed.  With
+    ``n_records``, also the site statistics of that many records (svjg_cohort_site_stats, 32 B per record)."""
 
-    def __init__(self, n_cells):
+    def __init__(self, n_cells, n_records=0):
         n_cells = max(int(n_cells), 1)
         self._mem = [alnfilter.PinnedBytes(n_cells * b) for b in (24, 1, 8, 1)]
         self.pl = self._mem[0].array.view(np.int64).reshape(n_cells, 3)
         self.gt = self._mem[1].array
         self.ad2 = self._mem[2].array.view(np.uint32).reshape(n_cells, 2)
         self.flags = self._mem[3].array
+        if n_records:
+            n_records = int(n_records)
+            self._mem += [alnfilter.PinnedBytes(n_records * b) for b in (16, 8, 8)]
+            self.gcount = self._mem[4].array.view(np.uint32).reshape(n_records, 4)
+            self.hwe = self._mem[5].array.view(np.float64)
+            self.exchet = self._mem[6].array.view(np.float64)
 
 
 def _genotype_block(cohort, idx, ty, min_support, e, blk):
@@ -101,14 +134,26 @@ def _genotype_block(cohort, idx, ty, min_support, e, blk):
     return gt, fl, ad, pl
 
 
+def _site_stats(cohort, n, blk):
+    """(gcount [n][4] = r0, h, r2, missing; hwe [n]; exchet [n]) of the block _genotype_block genotyped last, from
+    the gt codes on the device.  Those are final: the NEED_K patch above recomputes PL and flags, never the genotype,
+    which genotype_one fixes before it looks up log10 C(n, k)."""
+    g, hw, ex = blk.gcount[:n], blk.hwe[:n], blk.exchet[:n]
+    capi.check(capi.lib.svjg_cohort_site_stats(cohort._h, n, g.ctypes.data, hw.ctypes.data, ex.ctypes.data))
+    return g, hw, ex
+
+
 def genotype_cohort_vcf(tables, cohort, vcf_bytes, names, min_support=genotype.MIN_SUPPORT, e=genotype.ERR, out=None,
-                        block_records=None):
+                        block_records=None, info_tags=()):
     """predict-genotype.py's decision_vcf for every sample of ``cohort``: the multi-sample VCF, whose column s is
     the SAMPLE column of sample s's single-sample VCF.  ``vcf_bytes``: the catalogue VCF's bytes (or lines).
     ``names``: one column name per sample.  Returns (text, [genotyped SVs per sample]); with ``out`` (a binary file
     object) each block's text is written there as it is made and the text returned is None.  ``block_records``:
-    records per block (default: cell arrays of about 256 MiB); the bytes do not depend on it."""
+    records per block (default: cell arrays of about 256 MiB); the bytes do not depend on it.  ``info_tags``: INFO_TAGS
+    names; their values are computed on the device from each block's genotypes (svjg_cohort_site_stats) and written
+    into the INFO column, and their ##INFO lines in front of the ##FORMAT lines (svjg_vcf_format_cohort_tags)."""
     S = cohort.n_samples
+    mask = info_tags_mask(info_tags)
     if len(names) != S:
         raise ValueError(f"{len(names)} names for {S} samples")
     v = genotype.NativeVcf.from_input(vcf_bytes)
@@ -119,7 +164,7 @@ def genotype_cohort_vcf(tables, cohort, vcf_bytes, names, min_support=genotype.M
     ty = np.ascontiguousarray(v.svtype)
     n = v.n
     step = int(block_records) if block_records else max(1, BLOCK_BYTES // (CELL_BYTES * S))
-    blk = _Block(min(step, max(n, 1)) * S)
+    blk = _Block(min(step, max(n, 1)) * S, min(step, max(n, 1)) if mask else 0)
     if not 0 < e < 1:
         # math.log10 raises inside likelihood() only once a record passes the gate (predict-genotype.py:216), as in
         # genotype.genotype_host: a cohort in which no cell passes it is written with "./." everywhere
@@ -134,10 +179,13 @@ def genotype_cohort_vcf(tables, cohort, vcf_bytes, names, min_support=genotype.M
     for lo in range(0, n, step) if n else [0]:
         hi = min(n, lo + step)
         gt, fl, ad, pl = _genotype_block(cohort, idx[lo:hi], ty[lo:hi], min_support, e, blk)
+        site = [None] * 3
+        if mask:
+            site = [a.ctypes.data for a in _site_stats(cohort, hi - lo, blk)]
         buf, n_out = C.c_void_p(), C.c_uint64()
-        capi.check(capi.lib.svjg_vcf_format_cohort(v._h, lo, hi, S, joined, len(joined), gt.ctypes.data, fl.ctypes.data,
-                                                   ad.ctypes.data, pl.ctypes.data, C.byref(buf), C.byref(n_out),
-                                                   n_gt.ctypes.data))
+        capi.check(capi.lib.svjg_vcf_format_cohort_tags(v._h, lo, hi, S, joined, len(joined), gt.ctypes.data,
+                                                        fl.ctypes.data, ad.ctypes.data, pl.ctypes.data, mask, *site,
+                                                        C.byref(buf), C.byref(n_out), n_gt.ctypes.data))
         try:
             if out is not None:
                 if n_out.value:
