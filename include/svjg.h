@@ -268,6 +268,32 @@ int svjg_cohort_genotype(svjg_cohort *c, const uint32_t *sv_index, const uint8_t
                          int64_t *pl, uint8_t *gt, uint32_t *ad2, uint8_t *flags);
 int svjg_cohort_site_stats(svjg_cohort *c, uint32_t n, uint32_t *gcount, double *hwe, double *exchet);
 
+/* Sex-chromosome ploidy (DESIGN.md §8a).  The ploidy of cell (record i, sample s) is table[rclass[i]][sample_sex[s]],
+ * 0, 1 or 2; the caller maps its rules (e.g. a bcftools --ploidy-file) to per-record classes.
+ *   svjg_cohort_set_ploidy       the table [n_classes][n_sexes] u8 (n_classes <= 255, n_sexes <= 64, entries <= 2) and
+ *                                sample_sex [n_samples] u8 (< n_sexes), kept on the device with the handle
+ *   svjg_cohort_genotype_ploidy  svjg_cohort_genotype with rclass [n] u8 (< n_classes).  Ploidy 2: the diploid cell,
+ *                                gt 0-3.  Ploidy 1: gate, normalisation, ad2 and flags of the diploid cell; gt
+ *                                SVJG_GT_HAP_REF if L0 > L2, SVJG_GT_HAP_ALT if L2 > L0, SVJG_GT_HAP_MISSING on a tie,
+ *                                below min_support or outside the gate; pl[0] and pl[2] are the diploid PL0 and PL2
+ *                                (pl[1] is the diploid PL1: not part of the call).  Ploidy 0: SVJG_GT_NO_CALL, flags
+ *                                and ad2 of the diploid cell (no NEED_K: no likelihood is computed), pl 0.
+ *   svjg_cohort_site_stats_ploidy  svjg_cohort_site_stats with gcount [n][6] = (r0, h, r2, a0, a1, m): a0 / a1 count
+ *                                SVJG_GT_HAP_REF / _HAP_ALT, m every other cell; HWE and ExcHet of (r0, h, r2) */
+#define SVJG_GT_HAP_REF 4
+#define SVJG_GT_HAP_ALT 5
+#define SVJG_GT_HAP_MISSING 6
+#define SVJG_GT_NO_CALL 7
+#define SVJG_PLOIDY_MAX_CLASSES 255
+#define SVJG_PLOIDY_MAX_SEXES 64
+int svjg_cohort_set_ploidy(svjg_cohort *c, uint32_t n_classes, uint32_t n_sexes, const uint8_t *table,
+                           const uint8_t *sample_sex);
+int svjg_cohort_genotype_ploidy(svjg_cohort *c, const uint32_t *sv_index, const uint8_t *svtype, const uint8_t *rclass,
+                                uint32_t n, int64_t min_support, double log10_1me, double log10_e, double log10_half,
+                                const double *lut, uint32_t lut_nmax, int64_t *pl, uint8_t *gt, uint32_t *ad2,
+                                uint8_t *flags);
+int svjg_cohort_site_stats_ploidy(svjg_cohort *c, uint32_t n, uint32_t *gcount, double *hwe, double *exchet);
+
 /* Page-locked host memory (cudaHostAlloc) for file buffers and results: copies to and from it run
  * at PCIe speed.  For callers that do not want a tensor library just to pin memory. */
 int svjg_host_alloc(uint64_t bytes, void **out);
@@ -357,6 +383,11 @@ const uint8_t *svjg_vcf_svtype(const svjg_vcf *v);
 const char *svjg_vcf_key(const svjg_vcf *v, uint32_t i, uint32_t *len);   /* NULL: the record has no key */
 int svjg_vcf_index_tables(const svjg_vcf *v, const svjg_tables *t, uint32_t *sv_index);
 int svjg_vcf_index_counts(const svjg_vcf *v, const svjg_aln_counts *c, uint32_t *sv_index, uint8_t *svtype);
+/* svjg_vcf_loci: chrom[i] = index of record i's CHROM column among the distinct CHROMs in order of first appearance,
+ * pos[i] = its POS column, which must be 1 to 18 ASCII digits (SVJG_E_INPUT otherwise, naming the record).  *names:
+ * the distinct CHROMs joined by '\n' (a CHROM holds no newline), *names_len bytes, released with svjg_buffer_free;
+ * *n_chroms of them. */
+int svjg_vcf_loci(const svjg_vcf *v, uint32_t *chrom, int64_t *pos, char **names, uint64_t *names_len, uint32_t *n_chroms);
 int svjg_vcf_format(const svjg_vcf *v, const uint8_t *gt, const uint8_t *flags, const uint32_t *ad2,
                     const int64_t *pl, char **out, uint64_t *out_len, uint64_t *n_genotyped);
 /* svjg_vcf_format_cohort: the text of records [lo, hi) of a multi-sample VCF (svjg_cohort_genotype's arrays of those
@@ -393,6 +424,20 @@ int svjg_vcf_format_cohort_tags(const svjg_vcf *v, uint32_t lo, uint32_t hi, uin
                                 uint64_t names_len, const uint8_t *gt, const uint8_t *flags, const uint32_t *ad2,
                                 const int64_t *pl, uint32_t tags, const uint32_t *gcount, const double *hwe,
                                 const double *exchet, char **out, uint64_t *out_len, uint64_t *n_genotyped);
+/* svjg_vcf_format_cohort_ploidy: the text of svjg_cohort_genotype_ploidy's cells; svjg_vcf_format_cohort_tags is
+ * this formatter with ploidy off (codes 0-3 only, gcount [n][4], no AC_Hemi, PL Number=3).  Here gcount is
+ * svjg_cohort_site_stats_ploidy's [hi - lo][6] and the ##FORMAT line of PL says Number=G, whatever the cells.  Cells:
+ *   codes 0-3                 as svjg_vcf_format_cohort
+ *   SVJG_GT_HAP_* genotyped   "0", "1" or "." : DP : AD : PL0,PL2     (not genotyped: ".:0:0,0:.,.")
+ *   SVJG_GT_NO_CALL genotyped ".:DP:AD:."                              (not genotyped: ".:0:0,0:.")
+ * n_genotyped counts the genotyped cells of codes 0-6.  Tags: NS = r0 + h + r2 + a0 + a1, AN = 2 (r0 + h + r2) + a0 +
+ * a1, AC = h + 2 r2 + a1, AF = AC / AN, AC_Het = h, AC_Hom = 2 r2, F_MISSING = m / S, HWE and ExcHet ("." when
+ * r0 + h + r2 = 0), AC_Hemi = a1 (Number=A), written in the bit order. */
+#define SVJG_TAG_AC_HEMI 0x200u
+int svjg_vcf_format_cohort_ploidy(const svjg_vcf *v, uint32_t lo, uint32_t hi, uint32_t n_samples, const char *names,
+                                  uint64_t names_len, const uint8_t *gt, const uint8_t *flags, const uint32_t *ad2,
+                                  const int64_t *pl, uint32_t tags, const uint32_t *gcount, const double *hwe,
+                                  const double *exchet, char **out, uint64_t *out_len, uint64_t *n_genotyped);
 void svjg_buffer_free(char *p);
 
 /* ---- output (host) ------------------------------------------------------------

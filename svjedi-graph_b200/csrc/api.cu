@@ -379,6 +379,7 @@ extern "C" void svjg_cohort_free(svjg_cohort *c) {
     if (c->d_lut) cudaFree(c->d_lut);
     if (c->d_blk) cudaFree(c->d_blk);
     if (c->d_site) cudaFree(c->d_site);
+    if (c->d_ploidy) cudaFree(c->d_ploidy);
     if (c->stream) cudaStreamDestroy(c->stream);
     delete c;
 }

@@ -11,6 +11,7 @@
 
 #include <algorithm>
 #include <cstring>
+#include <string>
 
 #include "svjg_internal.h"
 
@@ -98,14 +99,20 @@ __device__ int64_t pl_of(const F192 &x) {
 // The genotype of one SV of one sample from its two counters: the gate of predict-genotype.py:216,
 // allele_normalization, the likelihoods, the unique argmax, -ms, the rounded counts, log10 C(n, k) and PL.
 // Results go to gt[o], flags[o], ad2[2o..], pl[3o..]; k_override[o] is read when k_override is given.
+// PLOIDY: the cell has `ploidy` copies (else 2, and `ploidy` is not read: the plain instance is the reference's diploid
+// call statement for statement).  Ploidy 1 calls between the "REF" and "ALT" sums L0 and L2 only (gt SVJG_GT_HAP_REF /
+// _HAP_ALT / _HAP_MISSING); ploidy 0 makes no call and computes no likelihood, but keeps DP and AD (SVJG_GT_NO_CALL).
+// DESIGN.md §8a, "Sex-chromosome ploidy".
+template <bool PLOIDY>
 __device__ __forceinline__ void genotype_one(uint32_t n0, uint32_t n1, uint32_t idx, uint32_t ty, int64_t min_support,
                                              double la, double lb, double lh, const double *lut, uint32_t lut_nmax,
                                              const double *k_override, size_t o, int64_t *pl, uint8_t *gt,
-                                             uint32_t *ad2, uint8_t *flags) {
+                                             uint32_t *ad2, uint8_t *flags, uint32_t ploidy) {
     // predict-genotype.py:216 — a key is "in the dict" once it has at least one hit
     bool gate = (ty & 0x3F) <= 3 && !(ty & 0x80) && ty != 255 && idx != 0xFFFFFFFFu && ((n0 | n1) != 0 || (ty & 0x40));
     if (!gate) {
-        gt[o] = 3;
+        if constexpr (PLOIDY) gt[o] = ploidy == 2 ? 3 : ploidy == 1 ? SVJG_GT_HAP_MISSING : SVJG_GT_NO_CALL;
+        else gt[o] = 3;
         flags[o] = 0;
         ad2[2 * o] = 0;
         ad2[2 * o + 1] = 0;
@@ -123,6 +130,16 @@ __device__ __forceinline__ void genotype_one(uint32_t n0, uint32_t n1, uint32_t 
         t2 = n1;
         fl |= SVJG_GT_HALVED_1;
     }
+    if constexpr (PLOIDY) {
+        if (ploidy == 0) {
+            gt[o] = SVJG_GT_NO_CALL;
+            flags[o] = uint8_t(fl);
+            ad2[2 * o] = uint32_t(t1);
+            ad2[2 * o + 1] = uint32_t(t2);
+            pl[3 * o] = pl[3 * o + 1] = pl[3 * o + 2] = 0;
+            return;
+        }
+    }
     double c1 = double(t1) * 0.5, c2 = double(t2) * 0.5, cs = double(t1 + t2) * 0.5;   // exact
     bool ok = true;
     // :295-297 — each product is the double the reference computes
@@ -136,6 +153,12 @@ __device__ __forceinline__ void genotype_one(uint32_t n0, uint32_t n1, uint32_t 
     else if (c01 < 0 && c12 > 0) g = 1;
     else if (c02 < 0 && c12 < 0) g = 2;
     if (int64_t(t1 + t2) < 2 * min_support) g = 3;                                       // :310
+    if constexpr (PLOIDY) {
+        if (ploidy == 1) {   // the same rule restricted to {L0, L2}
+            g = c02 > 0 ? SVJG_GT_HAP_REF : c02 < 0 ? SVJG_GT_HAP_ALT : SVJG_GT_HAP_MISSING;
+            if (int64_t(t1 + t2) < 2 * min_support) g = SVJG_GT_HAP_MISSING;
+        }
+    }
     // rc = int(round(c, 0)), half to even (:291-292)
     uint64_t r1 = (t1 >> 1) + ((t1 & 1) ? ((t1 >> 1) & 1) : 0);
     uint64_t r2 = (t2 >> 1) + ((t2 & 1) ? ((t2 >> 1) & 1) : 0);
@@ -231,17 +254,21 @@ __global__ void genotype_kernel(const uint32_t *__restrict__ counts, const __gri
             n1 = c.y;
         }
     }
-    genotype_one(n0, n1, idx, ty, min_support, la, lb, lh, lut, lut_nmax, k_override, i, pl, gt, ad2, flags);
+    genotype_one<false>(n0, n1, idx, ty, min_support, la, lb, lh, lut, lut_nmax, k_override, i, pl, gt, ad2, flags, 2);
 }
 
 // One thread per cell (record i, sample s) of a block of records.  The counters are the cohort's sample-major
 // matrix ([S][num_sv][2], as the filter writes a sample's counters); the results are record-major ([n][S], the
-// order of the VCF text).
+// order of the VCF text).  PLOIDY: the cell's ploidy is ptab[rclass[i]][sex[s]] (ptab [classes][n_sexes]); without
+// it every cell is diploid and the three arrays are not read.
+template <bool PLOIDY>
 __global__ void genotype_cohort_kernel(const uint32_t *__restrict__ counts, uint32_t num_sv, uint32_t n_samples,
                                        const uint32_t *__restrict__ sv_index, const uint8_t *__restrict__ svtype,
                                        uint32_t n_cells, int64_t min_support, double la, double lb, double lh,
                                        const double *__restrict__ lut, uint32_t lut_nmax, int64_t *__restrict__ pl,
-                                       uint8_t *__restrict__ gt, uint32_t *__restrict__ ad2, uint8_t *__restrict__ flags) {
+                                       uint8_t *__restrict__ gt, uint32_t *__restrict__ ad2, uint8_t *__restrict__ flags,
+                                       const uint8_t *__restrict__ rclass, const uint8_t *__restrict__ sex,
+                                       const uint8_t *__restrict__ ptab, uint32_t n_sexes) {
     const uint32_t c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= n_cells) return;
     const uint32_t i = c / n_samples, s = c - i * n_samples;
@@ -252,7 +279,9 @@ __global__ void genotype_cohort_kernel(const uint32_t *__restrict__ counts, uint
         n0 = v.x;
         n1 = v.y;
     }
-    genotype_one(n0, n1, idx, svtype[i], min_support, la, lb, lh, lut, lut_nmax, nullptr, c, pl, gt, ad2, flags);
+    const uint32_t ploidy = PLOIDY ? uint32_t(ptab[rclass[i] * n_sexes + sex[s]]) : 2u;
+    genotype_one<PLOIDY>(n0, n1, idx, svtype[i], min_support, la, lb, lh, lut, lut_nmax, nullptr, c, pl, gt, ad2, flags,
+                         ploidy);
 }
 
 // One term step of the Wigginton-Cutler-Abecasis walk: v * D / E with D and E exact integers (below 2^53), each
@@ -320,37 +349,59 @@ __device__ void site_exact_tests(uint32_t r0, uint32_t h, uint32_t r2, double &h
 
 // Site statistics of a block of records from the genotype codes the cohort kernel left on the device ([n][S]).
 // A block of SITE_THREADS records: each warp counts the 0/0, 0/1 and 1/1 cells of its records (coalesced byte loads
-// along the row, one warp reduction), then every thread runs the exact tests of one record, which are serial per
-// record.  Results: gcount[i] = (r0, h, r2, missing), hwe[i], exchet[i].
+// along the row, one warp reduction per code), then every thread runs the exact tests of one record, which are serial
+// per record.  Results: gcount[i] = (r0, h, r2, missing), or with PLOIDY (r0, h, r2, a0, a1, missing) where a0 / a1
+// count the haploid calls; hwe[i], exchet[i] of (r0, h, r2).
 constexpr int SITE_THREADS = 256;
+template <bool PLOIDY>
 __global__ void __launch_bounds__(SITE_THREADS)
-cohort_site_stats_kernel(const uint8_t *__restrict__ gt, uint32_t n, uint32_t n_samples, uint4 *__restrict__ gcount,
+cohort_site_stats_kernel(const uint8_t *__restrict__ gt, uint32_t n, uint32_t n_samples, uint32_t *__restrict__ gcount,
                          double *__restrict__ hwe, double *__restrict__ exchet) {
-    __shared__ uint32_t cnt[3][SITE_THREADS];
+    __shared__ uint32_t cnt[PLOIDY ? 5 : 3][SITE_THREADS];
     const uint32_t base = blockIdx.x * SITE_THREADS, lane = threadIdx.x & 31;
     for (uint32_t r = threadIdx.x >> 5; r < SITE_THREADS && base + r < n; r += SITE_THREADS / 32) {
         const uint8_t *row = gt + size_t(base + r) * n_samples;
-        uint32_t c0 = 0, c1 = 0, c2 = 0;
+        uint32_t c0 = 0, c1 = 0, c2 = 0, a0 = 0, a1 = 0;
         for (uint32_t s = lane; s < n_samples; s += 32) {
             const uint32_t g = row[s];
             c0 += g == 0;
             c1 += g == 1;
             c2 += g == 2;
+            if constexpr (PLOIDY) {
+                a0 += g == SVJG_GT_HAP_REF;
+                a1 += g == SVJG_GT_HAP_ALT;
+            }
         }
         c0 = __reduce_add_sync(0xFFFFFFFFu, c0);
         c1 = __reduce_add_sync(0xFFFFFFFFu, c1);
         c2 = __reduce_add_sync(0xFFFFFFFFu, c2);
+        if constexpr (PLOIDY) {
+            a0 = __reduce_add_sync(0xFFFFFFFFu, a0);
+            a1 = __reduce_add_sync(0xFFFFFFFFu, a1);
+        }
         if (lane == 0) {
             cnt[0][r] = c0;
             cnt[1][r] = c1;
             cnt[2][r] = c2;
+            if constexpr (PLOIDY) {
+                cnt[3][r] = a0;
+                cnt[4][r] = a1;
+            }
         }
     }
     __syncthreads();
     const uint32_t i = base + threadIdx.x;
     if (i >= n) return;
     const uint32_t r0 = cnt[0][threadIdx.x], h = cnt[1][threadIdx.x], r2 = cnt[2][threadIdx.x];
-    gcount[i] = make_uint4(r0, h, r2, n_samples - r0 - h - r2);
+    if constexpr (PLOIDY) {
+        const uint32_t a0 = cnt[3][threadIdx.x], a1 = cnt[4][threadIdx.x];
+        uint2 *g = reinterpret_cast<uint2 *>(gcount + 6 * size_t(i));
+        g[0] = make_uint2(r0, h);
+        g[1] = make_uint2(r2, a0);
+        g[2] = make_uint2(a1, n_samples - r0 - h - r2 - a0 - a1);
+    } else {
+        reinterpret_cast<uint4 *>(gcount)[i] = make_uint4(r0, h, r2, n_samples - r0 - h - r2);
+    }
     double p_hwe, p_exc;
     site_exact_tests(r0, h, r2, p_hwe, p_exc);
     hwe[i] = p_hwe;
@@ -437,22 +488,52 @@ extern "C" int svjg_genotype_host(const uint32_t *counts, uint32_t num_counts, c
 // ---------------------------------------------------------------------------
 // cohort: one block of records genotyped in every sample
 // ---------------------------------------------------------------------------
-extern "C" int svjg_cohort_genotype(svjg_cohort *c, const uint32_t *sv_index, const uint8_t *svtype, uint32_t n,
-                                    int64_t min_support, double log10_1me, double log10_e, double log10_half,
-                                    const double *lut, uint32_t lut_nmax, int64_t *pl, uint8_t *gt, uint32_t *ad2,
-                                    uint8_t *flags) {
-    if (!c) return svjg::set_error(SVJG_E_ARG, "svjg_cohort_genotype: NULL cohort");
+extern "C" int svjg_cohort_set_ploidy(svjg_cohort *c, uint32_t n_classes, uint32_t n_sexes, const uint8_t *table,
+                                      const uint8_t *sample_sex) {
+    if (!c || !table || !sample_sex) return svjg::set_error(SVJG_E_ARG, "svjg_cohort_set_ploidy: NULL argument");
+    if (n_classes == 0 || n_classes > SVJG_PLOIDY_MAX_CLASSES || n_sexes == 0 || n_sexes > SVJG_PLOIDY_MAX_SEXES)
+        return svjg::set_error(SVJG_E_ARG, "svjg_cohort_set_ploidy: 1 to 255 classes and 1 to 64 sexes");
+    const size_t n_tab = size_t(n_classes) * n_sexes;
+    for (size_t k = 0; k < n_tab; ++k)
+        if (table[k] > 2) return svjg::set_error(SVJG_E_ARG, "svjg_cohort_set_ploidy: a ploidy other than 0, 1 or 2");
+    for (uint32_t s = 0; s < c->n_samples; ++s)
+        if (sample_sex[s] >= n_sexes) return svjg::set_error(SVJG_E_ARG, "svjg_cohort_set_ploidy: sample sex out of range");
+    SVJG_CUDA(cudaSetDevice(c->t->device));
+    if (c->d_ploidy) SVJG_CUDA(cudaFree(c->d_ploidy));
+    c->d_ploidy = nullptr;
+    c->n_classes = c->n_sexes = 0;
+    // [n_classes][n_sexes] table, then the sex of every sample
+    SVJG_CUDA(cudaMalloc(&c->d_ploidy, n_tab + c->n_samples));
+    SVJG_CUDA(cudaMemcpy(c->d_ploidy, table, n_tab, cudaMemcpyHostToDevice));
+    SVJG_CUDA(cudaMemcpy(c->d_ploidy + n_tab, sample_sex, c->n_samples, cudaMemcpyHostToDevice));
+    c->n_classes = n_classes;
+    c->n_sexes = n_sexes;
+    return SVJG_OK;
+}
+
+namespace {
+// svjg_cohort_genotype (rclass == nullptr: every cell diploid) and svjg_cohort_genotype_ploidy
+int cohort_genotype(const char *fn, svjg_cohort *c, const uint32_t *sv_index, const uint8_t *svtype, const uint8_t *rclass,
+                    uint32_t n, int64_t min_support, double log10_1me, double log10_e, double log10_half, const double *lut,
+                    uint32_t lut_nmax, int64_t *pl, uint8_t *gt, uint32_t *ad2, uint8_t *flags) {
+    const std::string f = fn;
+    if (!c) return svjg::set_error(SVJG_E_ARG, f + ": NULL cohort");
     c->blk_n = 0;                          // set again once this block's cells are complete
     if (n == 0) return SVJG_OK;
     if (!sv_index || !svtype || !lut || !pl || !gt || !ad2 || !flags)
-        return svjg::set_error(SVJG_E_ARG, "svjg_cohort_genotype: NULL argument");
+        return svjg::set_error(SVJG_E_ARG, f + ": NULL argument");
     if (!(log10_1me == log10_1me) || !(log10_e == log10_e) || !(log10_half == log10_half))
-        return svjg::set_error(SVJG_E_ARG, "svjg_cohort_genotype: NaN constant");
+        return svjg::set_error(SVJG_E_ARG, f + ": NaN constant");
     const uint64_t cells = uint64_t(n) * c->n_samples;
-    if (cells >= 0xFFFFFFFFull) return svjg::set_error(SVJG_E_ARG, "svjg_cohort_genotype: block of more than 2^32 cells");
+    if (cells >= 0xFFFFFFFFull) return svjg::set_error(SVJG_E_ARG, f + ": block of more than 2^32 cells");
     for (uint32_t i = 0; i < n; ++i)
         if (sv_index[i] != 0xFFFFFFFFu && sv_index[i] >= c->num_sv)
-            return svjg::set_error(SVJG_E_ARG, "svjg_cohort_genotype: sv_index out of range");
+            return svjg::set_error(SVJG_E_ARG, f + ": sv_index out of range");
+    if (rclass) {
+        if (!c->d_ploidy) return svjg::set_error(SVJG_E_ARG, f + ": no ploidy table (svjg_cohort_set_ploidy)");
+        for (uint32_t i = 0; i < n; ++i)
+            if (rclass[i] >= c->n_classes) return svjg::set_error(SVJG_E_ARG, f + ": record class out of range");
+    }
     SVJG_CUDA(cudaSetDevice(c->t->device));
     // the LUT is uploaded again only when its contents change
     const size_t n_lut = size_t(lut_nmax + 1) * (lut_nmax + 2) / 2;
@@ -465,9 +546,10 @@ extern "C" int svjg_cohort_genotype(svjg_cohort *c, const uint32_t *sv_index, co
         c->lut.assign(lut, lut + n_lut);
     }
     auto up = [](size_t x) { return (x + 255) & ~size_t(255); };
-    const size_t b_idx = size_t(n) * 4, b_ty = n, b_pl = cells * 24, b_gt = cells, b_ad = cells * 8, b_fl = cells;
-    const size_t o_ty = up(b_idx), o_pl = o_ty + up(b_ty), o_gt = o_pl + up(b_pl), o_ad = o_gt + up(b_gt),
-                 o_fl = o_ad + up(b_ad), total = o_fl + up(b_fl);
+    const size_t b_idx = size_t(n) * 4, b_ty = n, b_cls = rclass ? n : 0, b_pl = cells * 24, b_gt = cells, b_ad = cells * 8,
+                 b_fl = cells;
+    const size_t o_ty = up(b_idx), o_cls = o_ty + up(b_ty), o_pl = o_cls + up(b_cls), o_gt = o_pl + up(b_pl),
+                 o_ad = o_gt + up(b_gt), o_fl = o_ad + up(b_ad), total = o_fl + up(b_fl);
     if (c->blk_cap < total) {
         if (c->d_blk) SVJG_CUDA(cudaFree(c->d_blk));
         c->d_blk = nullptr;
@@ -479,12 +561,16 @@ extern "C" int svjg_cohort_genotype(svjg_cohort *c, const uint32_t *sv_index, co
     cudaStream_t st = c->stream;
     SVJG_CUDA(cudaMemcpyAsync(d, sv_index, b_idx, cudaMemcpyHostToDevice, st));
     SVJG_CUDA(cudaMemcpyAsync(d + o_ty, svtype, b_ty, cudaMemcpyHostToDevice, st));
+    if (rclass) SVJG_CUDA(cudaMemcpyAsync(d + o_cls, rclass, b_cls, cudaMemcpyHostToDevice, st));
     const int threads = 128;
     const uint32_t blocks = uint32_t((cells + threads - 1) / threads);
-    genotype_cohort_kernel<<<blocks, threads, 0, st>>>(c->d_counts, c->num_sv, c->n_samples, reinterpret_cast<const uint32_t *>(d),
-                                                       d + o_ty, uint32_t(cells), min_support, log10_1me, log10_e, log10_half,
-                                                       c->d_lut, lut_nmax, reinterpret_cast<int64_t *>(d + o_pl), d + o_gt,
-                                                       reinterpret_cast<uint32_t *>(d + o_ad), d + o_fl);
+    auto kernel = rclass ? genotype_cohort_kernel<true> : genotype_cohort_kernel<false>;
+    const uint8_t *d_tab = rclass ? c->d_ploidy : nullptr;
+    kernel<<<blocks, threads, 0, st>>>(c->d_counts, c->num_sv, c->n_samples, reinterpret_cast<const uint32_t *>(d), d + o_ty,
+                                       uint32_t(cells), min_support, log10_1me, log10_e, log10_half, c->d_lut, lut_nmax,
+                                       reinterpret_cast<int64_t *>(d + o_pl), d + o_gt, reinterpret_cast<uint32_t *>(d + o_ad),
+                                       d + o_fl, rclass ? d + o_cls : nullptr,
+                                       d_tab ? d_tab + size_t(c->n_classes) * c->n_sexes : nullptr, d_tab, c->n_sexes);
     SVJG_CUDA(cudaGetLastError());
     SVJG_CUDA(cudaMemcpyAsync(pl, d + o_pl, b_pl, cudaMemcpyDeviceToHost, st));
     SVJG_CUDA(cudaMemcpyAsync(gt, d + o_gt, b_gt, cudaMemcpyDeviceToHost, st));
@@ -496,21 +582,23 @@ extern "C" int svjg_cohort_genotype(svjg_cohort *c, const uint32_t *sv_index, co
     return SVJG_OK;
 }
 
-// Site statistics of the block of the last svjg_cohort_genotype call, from its gt codes where the kernel left them
-// on the device: 32 B per record come back, not the cells.
-extern "C" int svjg_cohort_site_stats(svjg_cohort *c, uint32_t n, uint32_t *gcount, double *hwe, double *exchet) {
-    if (!c) return svjg::set_error(SVJG_E_ARG, "svjg_cohort_site_stats: NULL cohort");
+// Site statistics of the block of the last genotype call, from its gt codes where the kernel left them on the device:
+// 32 B (40 B with ploidy) per record come back, not the cells.
+int cohort_site_stats(const char *fn, bool ploidy, svjg_cohort *c, uint32_t n, uint32_t *gcount, double *hwe, double *exchet) {
+    const std::string f = fn;
+    if (!c) return svjg::set_error(SVJG_E_ARG, f + ": NULL cohort");
     if (n != c->blk_n)
-        return svjg::set_error(SVJG_E_ARG, "svjg_cohort_site_stats: n is not the record count of the last svjg_cohort_genotype call");
+        return svjg::set_error(SVJG_E_ARG, f + ": n is not the record count of the last svjg_cohort_genotype call");
     if (n == 0) return SVJG_OK;
-    if (!gcount || !hwe || !exchet) return svjg::set_error(SVJG_E_ARG, "svjg_cohort_site_stats: NULL argument");
+    if (!gcount || !hwe || !exchet) return svjg::set_error(SVJG_E_ARG, f + ": NULL argument");
     // every D and E of the exact tests must be exact in a double
     const uint64_t s1 = uint64_t(c->n_samples) + 1;
     if (s1 >= (1ull << 26) || 4 * s1 * s1 >= (1ull << 53))
-        return svjg::set_error(SVJG_E_ARG, "svjg_cohort_site_stats: 4 (S + 1)^2 must be below 2^53");
+        return svjg::set_error(SVJG_E_ARG, f + ": 4 (S + 1)^2 must be below 2^53");
     SVJG_CUDA(cudaSetDevice(c->t->device));
     auto up = [](size_t x) { return (x + 255) & ~size_t(255); };
-    const size_t b_cnt = size_t(n) * 16, b_p = size_t(n) * 8, o_hwe = up(b_cnt), o_exc = o_hwe + up(b_p), total = o_exc + up(b_p);
+    const size_t b_cnt = size_t(n) * (ploidy ? 24 : 16), b_p = size_t(n) * 8, o_hwe = up(b_cnt), o_exc = o_hwe + up(b_p),
+                 total = o_exc + up(b_p);
     if (c->site_cap < total) {
         if (c->d_site) SVJG_CUDA(cudaFree(c->d_site));
         c->d_site = nullptr;
@@ -521,15 +609,41 @@ extern "C" int svjg_cohort_site_stats(svjg_cohort *c, uint32_t n, uint32_t *gcou
     uint8_t *d = c->d_site;
     cudaStream_t st = c->stream;
     const uint32_t blocks = uint32_t((uint64_t(n) + SITE_THREADS - 1) / SITE_THREADS);
-    cohort_site_stats_kernel<<<blocks, SITE_THREADS, 0, st>>>(c->d_blk + c->blk_gt, n, c->n_samples, reinterpret_cast<uint4 *>(d),
-                                                              reinterpret_cast<double *>(d + o_hwe),
-                                                              reinterpret_cast<double *>(d + o_exc));
+    auto kernel = ploidy ? cohort_site_stats_kernel<true> : cohort_site_stats_kernel<false>;
+    kernel<<<blocks, SITE_THREADS, 0, st>>>(c->d_blk + c->blk_gt, n, c->n_samples, reinterpret_cast<uint32_t *>(d),
+                                            reinterpret_cast<double *>(d + o_hwe), reinterpret_cast<double *>(d + o_exc));
     SVJG_CUDA(cudaGetLastError());
     SVJG_CUDA(cudaMemcpyAsync(gcount, d, b_cnt, cudaMemcpyDeviceToHost, st));
     SVJG_CUDA(cudaMemcpyAsync(hwe, d + o_hwe, b_p, cudaMemcpyDeviceToHost, st));
     SVJG_CUDA(cudaMemcpyAsync(exchet, d + o_exc, b_p, cudaMemcpyDeviceToHost, st));
     SVJG_CUDA(cudaStreamSynchronize(st));
     return SVJG_OK;
+}
+}  // namespace
+
+extern "C" int svjg_cohort_genotype(svjg_cohort *c, const uint32_t *sv_index, const uint8_t *svtype, uint32_t n,
+                                    int64_t min_support, double log10_1me, double log10_e, double log10_half,
+                                    const double *lut, uint32_t lut_nmax, int64_t *pl, uint8_t *gt, uint32_t *ad2,
+                                    uint8_t *flags) {
+    return cohort_genotype("svjg_cohort_genotype", c, sv_index, svtype, nullptr, n, min_support, log10_1me, log10_e,
+                           log10_half, lut, lut_nmax, pl, gt, ad2, flags);
+}
+
+extern "C" int svjg_cohort_genotype_ploidy(svjg_cohort *c, const uint32_t *sv_index, const uint8_t *svtype,
+                                           const uint8_t *rclass, uint32_t n, int64_t min_support, double log10_1me,
+                                           double log10_e, double log10_half, const double *lut, uint32_t lut_nmax,
+                                           int64_t *pl, uint8_t *gt, uint32_t *ad2, uint8_t *flags) {
+    if (n && !rclass) return svjg::set_error(SVJG_E_ARG, "svjg_cohort_genotype_ploidy: NULL argument");
+    return cohort_genotype("svjg_cohort_genotype_ploidy", c, sv_index, svtype, rclass, n, min_support, log10_1me, log10_e,
+                           log10_half, lut, lut_nmax, pl, gt, ad2, flags);
+}
+
+extern "C" int svjg_cohort_site_stats(svjg_cohort *c, uint32_t n, uint32_t *gcount, double *hwe, double *exchet) {
+    return cohort_site_stats("svjg_cohort_site_stats", false, c, n, gcount, hwe, exchet);
+}
+
+extern "C" int svjg_cohort_site_stats_ploidy(svjg_cohort *c, uint32_t n, uint32_t *gcount, double *hwe, double *exchet) {
+    return cohort_site_stats("svjg_cohort_site_stats_ploidy", true, c, n, gcount, hwe, exchet);
 }
 
 // ---------------------------------------------------------------------------

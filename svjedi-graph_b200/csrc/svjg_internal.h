@@ -47,6 +47,8 @@ struct svjg_cohort {
     size_t blk_gt = 0;                        // offset of its gt codes [blk_n][n_samples] in d_blk
     uint8_t *d_site = nullptr;                // site statistics of the last block (svjg_cohort_site_stats)
     size_t site_cap = 0;
+    uint8_t *d_ploidy = nullptr;              // svjg_cohort_set_ploidy: table [n_classes][n_sexes], then sex [n_samples]
+    uint32_t n_classes = 0, n_sexes = 0;
 };
 
 namespace svjg {

@@ -31,6 +31,7 @@ const char FORMAT_LINES[] =
     "(after normalization by breakpoint number for unbalanced SVs)\">\n"
     "##FORMAT=<ID=PL,Number=3,Type=Integer,Description=\"Phred-scaled likelihood for each genotype\">\n"
     "#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO\tFORMAT\t";      // then the sample names and "\n"
+const char PL_NUMBER[] = "ID=PL,Number=";                               // followed by "3", or "G" with ploidy
 
 struct Rec {
     uint64_t head_off;   // into text
@@ -312,6 +313,43 @@ extern "C" int svjg_vcf_index_counts(const svjg_vcf *v, const svjg_aln_counts *c
     return SVJG_OK;
 }
 
+extern "C" int svjg_vcf_loci(const svjg_vcf *v, uint32_t *chrom, int64_t *pos, char **names, uint64_t *names_len,
+                             uint32_t *n_chroms) {
+    if (!v || !names || !names_len || !n_chroms || ((!chrom || !pos) && !v->recs.empty()))
+        return set_error(SVJG_E_ARG, "svjg_vcf_loci: NULL argument");
+    std::unordered_map<sv, uint32_t> index;
+    for (size_t i = 0; i < v->recs.size(); ++i) {
+        const sv head(v->text.data() + v->recs[i].head_off, v->recs[i].head_len);   // 8 columns
+        const size_t t0 = head.find('\t'), t1 = head.find('\t', t0 + 1);
+        const sv c = head.substr(0, t0), p = head.substr(t0 + 1, t1 - t0 - 1);
+        int64_t x = 0;
+        bool digits = !p.empty() && p.size() <= 18;
+        for (char ch : p) {
+            digits = digits && ch >= '0' && ch <= '9';
+            x = x * 10 + (ch - '0');
+        }
+        if (!digits)
+            return set_error(SVJG_E_INPUT, "VCF record " + std::to_string(i + 1) + " (CHROM " + std::string(c) + "): POS '" +
+                                               std::string(p) + "' is not a decimal integer");
+        chrom[i] = index.emplace(c, uint32_t(index.size())).first->second;
+        pos[i] = x;
+    }
+    std::vector<sv> by_index(index.size());
+    for (const auto &kv : index) by_index[kv.second] = kv.first;
+    std::string joined;
+    for (size_t k = 0; k < by_index.size(); ++k) {
+        if (k) joined.push_back('\n');
+        joined.append(by_index[k]);
+    }
+    char *buf = (char *)malloc(joined.size() + 1);
+    if (!buf) return set_error(SVJG_E_NOMEM, "svjg_vcf_loci: out of memory");
+    memcpy(buf, joined.data(), joined.size());
+    *names = buf;
+    *names_len = joined.size();
+    *n_chroms = uint32_t(by_index.size());
+    return SVJG_OK;
+}
+
 namespace {
 inline char *put_u64(char *o, uint64_t x) {
     char b[24];
@@ -361,8 +399,10 @@ const InfoTag INFO_TAGS[] = {
     {"F_MISSING", false, "##INFO=<ID=F_MISSING,Number=1,Type=Float,Description=\"Fraction of missing genotypes\">\n"},
     {"HWE", true, "##INFO=<ID=HWE,Number=A,Type=Float,Description=\"HWE test (PMID:15789306); 1=good, 0=bad\">\n"},
     {"ExcHet", true, "##INFO=<ID=ExcHet,Number=A,Type=Float,Description=\"Test excess heterozygosity; 1=good, 0=bad\">\n"},
+    {"AC_Hemi", true, "##INFO=<ID=AC_Hemi,Number=A,Type=Integer,Description=\"Allele counts in hemizygous genotypes\">\n"},
 };
 constexpr uint32_t N_INFO_TAGS = sizeof INFO_TAGS / sizeof INFO_TAGS[0];
+constexpr uint32_t N_DIPLOID_TAGS = N_INFO_TAGS - 1;     // AC_Hemi needs the ploidy formatter
 
 bool selected_tag(uint32_t tags, sv key) {
     for (uint32_t t = 0; t < N_INFO_TAGS; ++t)
@@ -378,13 +418,15 @@ bool info_header_of(uint32_t tags, sv line) {
     return e != sv::npos && selected_tag(tags, rest.substr(0, e));
 }
 
-// The value text of tag t for counts g = (r0, h, r2, m) of S cells; "." where it has none
-size_t tag_value(char *o, uint32_t t, const uint32_t *g, uint64_t S, double hwe, double exchet, bool multi_alt) {
+// The value text of tag t for counts g = (r0, h, r2, m), or with ploidy (r0, h, r2, a0, a1, m), of S cells; "." where it
+// has none
+size_t tag_value(char *o, uint32_t t, const uint32_t *g, bool ploidy, uint64_t S, double hwe, double exchet, bool multi_alt) {
     if (INFO_TAGS[t].per_alt && multi_alt) {
         *o = '.';
         return 1;
     }
-    const uint64_t r0 = g[0], h = g[1], r2 = g[2], m = g[3], ns = r0 + h + r2;
+    const uint64_t r0 = g[0], h = g[1], r2 = g[2], a0 = ploidy ? g[3] : 0, a1 = ploidy ? g[4] : 0, m = g[ploidy ? 5 : 3];
+    const uint64_t dip = r0 + h + r2, ns = dip + a0 + a1, an = 2 * dip + a0 + a1, ac = h + 2 * r2 + a1;
     auto num = [&](uint64_t x) { return size_t(put_u64(o, x) - o); };
     auto flt = [&](bool have, double x) -> size_t {
         if (!have) {
@@ -395,40 +437,49 @@ size_t tag_value(char *o, uint32_t t, const uint32_t *g, uint64_t S, double hwe,
     };
     switch (1u << t) {
         case SVJG_TAG_NS: return num(ns);
-        case SVJG_TAG_AN: return num(2 * ns);
-        case SVJG_TAG_AC: return num(h + 2 * r2);
-        case SVJG_TAG_AF: return flt(ns != 0, double(h + 2 * r2) / double(2 * ns));
+        case SVJG_TAG_AN: return num(an);
+        case SVJG_TAG_AC: return num(ac);
+        case SVJG_TAG_AF: return flt(an != 0, double(ac) / double(an));
         case SVJG_TAG_AC_HET: return num(h);
         case SVJG_TAG_AC_HOM: return num(2 * r2);
         case SVJG_TAG_F_MISSING: return flt(true, double(m) / double(S));
-        case SVJG_TAG_HWE: return flt(ns != 0, hwe);
-        default: return flt(ns != 0, exchet);
+        case SVJG_TAG_HWE: return flt(dip != 0, hwe);
+        case SVJG_TAG_EXCHET: return flt(dip != 0, exchet);
+        default: return num(a1);
     }
 }
-}  // namespace
 
-// Records [lo, hi) with one column per sample; the arrays hold those records' cells, [hi - lo][S].
-extern "C" int svjg_vcf_format_cohort_tags(const svjg_vcf *v, uint32_t lo, uint32_t hi, uint32_t n_samples, const char *names,
-                                           uint64_t names_len, const uint8_t *gt, const uint8_t *flags, const uint32_t *ad2,
-                                           const int64_t *pl, uint32_t tags, const uint32_t *gcount, const double *hwe,
-                                           const double *exchet, char **out, uint64_t *out_len, uint64_t *n_genotyped) {
+// svjg_vcf_format_cohort_ploidy, and with ploidy == false svjg_vcf_format_cohort_tags
+int format_cohort(bool ploidy, const svjg_vcf *v, uint32_t lo, uint32_t hi, uint32_t n_samples, const char *names,
+                  uint64_t names_len, const uint8_t *gt, const uint8_t *flags, const uint32_t *ad2, const int64_t *pl,
+                  uint32_t tags, const uint32_t *gcount, const double *hwe, const double *exchet, char **out,
+                  uint64_t *out_len, uint64_t *n_genotyped) {
+
     if (!v || !out || !out_len || !names || !n_genotyped) return set_error(SVJG_E_ARG, "svjg_vcf_format: NULL argument");
     const size_t n_all = v->recs.size();
     if (lo > hi || hi > n_all || n_samples == 0) return set_error(SVJG_E_ARG, "svjg_vcf_format: bad record range or sample count");
     const size_t S = n_samples, n = size_t(hi - lo), n_cells = n * S;
     if (n && (!gt || !flags || !ad2 || !pl)) return set_error(SVJG_E_ARG, "svjg_vcf_format: NULL argument");
-    if (tags >> N_INFO_TAGS) return set_error(SVJG_E_ARG, "svjg_vcf_format: unknown INFO tag bit");
+    if (tags >> (ploidy ? N_INFO_TAGS : N_DIPLOID_TAGS)) return set_error(SVJG_E_ARG, "svjg_vcf_format: unknown INFO tag bit");
+    const size_t G = ploidy ? 6 : 4;                          // counts per record in gcount
     // every tag needs the counts (HWE and ExcHet are "." when NS = 0)
     if (n && tags && (!gcount || ((tags & SVJG_TAG_HWE) && !hwe) || ((tags & SVJG_TAG_EXCHET) && !exchet)))
         return set_error(SVJG_E_ARG, "svjg_vcf_format: NULL site statistics");
     if (tags) {
-        for (size_t j = 0; j < n; ++j)
-            if (uint64_t(gcount[4 * j]) + gcount[4 * j + 1] + gcount[4 * j + 2] + gcount[4 * j + 3] != S)
-                return set_error(SVJG_E_ARG, "svjg_vcf_format: genotype counts do not add up to the sample count");
+        for (size_t j = 0; j < n; ++j) {
+            uint64_t sum = 0;
+            for (size_t q = 0; q < G; ++q) sum += gcount[G * j + q];
+            if (sum != S) return set_error(SVJG_E_ARG, "svjg_vcf_format: genotype counts do not add up to the sample count");
+        }
     }
+    // without ploidy the code of a cell outside the gate is not read; with it, it says which ploidy the cell has
     for (size_t k = 0; k < n_cells; ++k)
-        if ((flags[k] & SVJG_GT_GENOTYPED) && gt[k] > 3) return set_error(SVJG_E_ARG, "svjg_vcf_format: gt code out of range");
+        if (ploidy ? gt[k] > SVJG_GT_NO_CALL : (flags[k] & SVJG_GT_GENOTYPED) && gt[k] > 3)
+            return set_error(SVJG_E_ARG, "svjg_vcf_format: gt code out of range");
     static const char *GT_TEXT[4] = {"0/0", "0/1", "1/1", "./."};
+    static const char HAP_TEXT[3] = {'0', '1', '.'};
+    std::string format_lines(FORMAT_LINES, sizeof FORMAT_LINES - 1);
+    if (ploidy) format_lines[format_lines.find(PL_NUMBER) + sizeof PL_NUMBER - 1] = 'G';
     const char *text = v->text.data();
     std::string info_hdr;                  // the ##INFO lines of the selected tags, in front of the ##FORMAT lines
     for (uint32_t t = 0; t < N_INFO_TAGS; ++t)
@@ -438,13 +489,13 @@ extern "C" int svjg_vcf_format_cohort_tags(const svjg_vcf *v, uint32_t lo, uint3
     while (h_lo < v->hdrs.size() && v->hdrs[h_lo].before < lo) ++h_lo;
     size_t h_hi = h_lo;
     while (h_hi < v->hdrs.size() && (hi == n_all || v->hdrs[h_hi].before < hi)) ++h_hi;
-    const size_t col_hdr = info_hdr.size() + sizeof FORMAT_LINES - 1 + names_len + 1;
+    const size_t col_hdr = info_hdr.size() + format_lines.size() + names_len + 1;
     auto dropped = [&](const Hdr &h) { return tags && info_header_of(tags, sv(text + h.off, h.len)); };
     auto hdr_len = [&](const Hdr &h) -> uint64_t { return h.len == UINT32_MAX ? col_hdr : dropped(h) ? 0 : h.len; };
     auto put_hdr = [&](char *o, const Hdr &h) {
         if (h.len != UINT32_MAX) return dropped(h) ? o : put_mem(o, text + h.off, h.len);
         o = put_mem(o, info_hdr.data(), info_hdr.size());
-        o = put_mem(o, FORMAT_LINES, sizeof FORMAT_LINES - 1);
+        o = put_mem(o, format_lines.data(), format_lines.size());
         o = put_mem(o, names, names_len);
         *o++ = '\n';
         return o;
@@ -491,24 +542,47 @@ extern "C" int svjg_vcf_format_cohort_tags(const svjg_vcf *v, uint32_t lo, uint3
             first = false;
             put(INFO_TAGS[t].id.data(), INFO_TAGS[t].id.size());
             put("=", 1);
-            put(val, tag_value(val, t, gcount + 4 * j, S, hwe ? hwe[j] : 0.0, exchet ? exchet[j] : 0.0, multi_alt));
+            put(val, tag_value(val, t, gcount + G * j, ploidy, S, hwe ? hwe[j] : 0.0, exchet ? exchet[j] : 0.0, multi_alt));
         }
         return len;
     };
+    // ":DP:AD:" of a genotyped cell k
+    auto put_dp_ad = [&](char *o, size_t k) {
+        const uint8_t f = flags[k];
+        const uint64_t t1 = ad2[2 * k], t2 = ad2[2 * k + 1];
+        const bool h0 = f & SVJG_GT_HALVED_0, h1 = f & SVJG_GT_HALVED_1;
+        *o++ = ':';
+        o = put_half(o, t1 + t2, h0 || h1);
+        *o++ = ':';
+        o = put_half(o, t1, h0);
+        *o++ = ',';
+        o = put_half(o, t2, h1);
+        *o++ = ':';
+        return o;
+    };
+    // the text of a haploid (codes 4-6) or ploidy-0 (code 7) cell k
+    auto put_haploid = [&](char *o, size_t k) {
+        const bool genotyped = flags[k] & SVJG_GT_GENOTYPED;
+        if (gt[k] == SVJG_GT_NO_CALL) {
+            if (!genotyped) return put_mem(o, ".:0:0,0:.", 9);
+            *o++ = '.';
+            o = put_dp_ad(o, k);
+            *o++ = '.';
+            return o;
+        }
+        if (!genotyped) return put_mem(o, ".:0:0,0:.,.", 11);
+        *o++ = HAP_TEXT[gt[k] - SVJG_GT_HAP_REF];
+        o = put_dp_ad(o, k);
+        o = put_i64(o, pl[3 * k]);
+        *o++ = ',';
+        return put_i64(o, pl[3 * k + 2]);
+    };
     // the text of cell k (at most 136 bytes)
     auto put_sample = [&](char *o, size_t k) {
-        const uint8_t f = flags[k];
-        if (f & SVJG_GT_GENOTYPED) {
-            const uint64_t t1 = ad2[2 * k], t2 = ad2[2 * k + 1];
-            const bool h0 = f & SVJG_GT_HALVED_0, h1 = f & SVJG_GT_HALVED_1;
+        if (ploidy && gt[k] >= SVJG_GT_HAP_REF) return put_haploid(o, k);
+        if (flags[k] & SVJG_GT_GENOTYPED) {
             o = put_mem(o, GT_TEXT[gt[k]], 3);
-            *o++ = ':';
-            o = put_half(o, t1 + t2, h0 || h1);
-            *o++ = ':';
-            o = put_half(o, t1, h0);
-            *o++ = ',';
-            o = put_half(o, t2, h1);
-            *o++ = ':';
+            o = put_dp_ad(o, k);
             o = put_i64(o, pl[3 * k]);
             *o++ = ',';
             o = put_i64(o, pl[3 * k + 1]);
@@ -542,7 +616,7 @@ extern "C" int svjg_vcf_format_cohort_tags(const svjg_vcf *v, uint32_t lo, uint3
             pos += put_head(nullptr, j) + 13 + S;
             for (size_t s = 0; s < S; ++s) {
                 const size_t k = j * S + s;
-                genotyped[s] += (flags[k] & SVJG_GT_GENOTYPED) != 0;
+                genotyped[s] += (flags[k] & SVJG_GT_GENOTYPED) && !(ploidy && gt[k] == SVJG_GT_NO_CALL);
                 pos += uint64_t(put_sample(tmp, k) - tmp);
             }
         }
@@ -598,6 +672,25 @@ extern "C" int svjg_vcf_format_cohort_tags(const svjg_vcf *v, uint32_t lo, uint3
     *out_len = uint64_t(o - buf);
     for (size_t s = 0; s < S; ++s) n_genotyped[s] += genotyped[s];
     return SVJG_OK;
+}
+}  // namespace
+
+// Records [lo, hi) with one column per sample; the arrays hold those records' cells, [hi - lo][S].
+extern "C" int svjg_vcf_format_cohort_tags(const svjg_vcf *v, uint32_t lo, uint32_t hi, uint32_t n_samples, const char *names,
+                                           uint64_t names_len, const uint8_t *gt, const uint8_t *flags, const uint32_t *ad2,
+                                           const int64_t *pl, uint32_t tags, const uint32_t *gcount, const double *hwe,
+                                           const double *exchet, char **out, uint64_t *out_len, uint64_t *n_genotyped) {
+    return format_cohort(false, v, lo, hi, n_samples, names, names_len, gt, flags, ad2, pl, tags, gcount, hwe, exchet, out,
+                         out_len, n_genotyped);
+}
+
+extern "C" int svjg_vcf_format_cohort_ploidy(const svjg_vcf *v, uint32_t lo, uint32_t hi, uint32_t n_samples,
+                                             const char *names, uint64_t names_len, const uint8_t *gt, const uint8_t *flags,
+                                             const uint32_t *ad2, const int64_t *pl, uint32_t tags, const uint32_t *gcount,
+                                             const double *hwe, const double *exchet, char **out, uint64_t *out_len,
+                                             uint64_t *n_genotyped) {
+    return format_cohort(true, v, lo, hi, n_samples, names, names_len, gt, flags, ad2, pl, tags, gcount, hwe, exchet, out,
+                         out_len, n_genotyped);
 }
 
 extern "C" int svjg_vcf_format_cohort(const svjg_vcf *v, uint32_t lo, uint32_t hi, uint32_t n_samples, const char *names,

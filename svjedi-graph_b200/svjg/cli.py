@@ -271,17 +271,25 @@ def cohort_main(argv=None):
                     help="aligned bases required on each side of a breakpoint (default 100)")
     ap.add_argument("--info-tags", metavar="<LIST>", default=None,
                     help="population INFO tags computed over the samples, a comma list of NS, AN, AC, AF, AC_Het, "
-                         "AC_Hom, F_MISSING, HWE, ExcHet, or all (written in that order; default: none, the catalogue's "
-                         "INFO as it is)")
+                         "AC_Hom, F_MISSING, HWE, ExcHet, AC_Hemi (with --ploidy-file), or all (written in that order; "
+                         "default: none, the catalogue's INFO as it is)")
+    ap.add_argument("--ploidy-file", metavar="<file>", default=None,
+                    help="ploidy rules as bcftools call --ploidy-file takes them: CHROM FROM TO SEX PLOIDY per line "
+                         "(1-based, inclusive; PLOIDY 0, 1 or 2), '* * * SEX PLOIDY' for a sex's default, otherwise 2. "
+                         "A record's CHROM and POS decide its ploidy. Needs --sample-sex")
+    ap.add_argument("--sample-sex", metavar="<file>", default=None,
+                    help="NAME SEX per line, every sample once (other names are ignored). Needs --ploidy-file")
     args = ap.parse_args(argv)
     import os
     if not args.prefix:
         _die("-p/--prefix is required: <prefix>_svs_edges.json holds the link -> SV table")
+    if (args.ploidy_file is None) != (args.sample_sex is None):
+        _die("--ploidy-file and --sample-sex are given together or not at all")
     info_tags = ()
     if args.info_tags is not None:
         from .cohort import parse_info_tags
         try:
-            info_tags = parse_info_tags(args.info_tags)
+            info_tags = parse_info_tags(args.info_tags, ploidy=args.ploidy_file is not None)
         except ValueError as exc:
             _die(f"--info-tags: {exc}")
     if os.environ.get("SVJG_GPUS", "1").strip() != "1":
@@ -297,6 +305,14 @@ def cohort_main(argv=None):
             _die(f"bad sample name {nm!r}: names must be non-empty and hold no tab, CR or LF")
     if len(set(names)) != len(names):
         _die("sample names must be unique")
+    ploidy = None
+    if args.ploidy_file is not None:
+        from .cohort import PloidyRules
+        try:
+            with open(args.ploidy_file) as fp, open(args.sample_sex) as fs:
+                ploidy = PloidyRules(fp.read(), fs.read(), names, args.ploidy_file, args.sample_sex)
+        except (OSError, ValueError) as exc:
+            _die(str(exc))
     d_over = 100 if args.min_overlap is None else args.min_overlap
     out_path = os.path.abspath(args.output)
     from concurrent.futures import ThreadPoolExecutor
@@ -308,6 +324,12 @@ def cohort_main(argv=None):
         ready = _start_device()
         vcf = gzio.read_bytes(args.vcf)
         _lap("VCF read")
+        if ploidy is not None:
+            # a catalogue the rules cannot place is refused before any sample is filtered
+            v = genotype.NativeVcf.from_input(vcf)
+            if v is not None:
+                ploidy.record_classes(v)
+                vcf = v
         tables = _load_tables(args.prefix, args.gfa, ready)
         _lap("tables + context")
         co = cohort.Cohort(tables, len(samples))
@@ -328,7 +350,7 @@ def cohort_main(argv=None):
         fd, tmp = tempfile.mkstemp(prefix="." + os.path.basename(out_path) + ".", dir=os.path.dirname(out_path))
         with os.fdopen(fd, "wb") as out:
             _, n_gt = cohort.genotype_cohort_vcf(tables, co, vcf, names, args.minsupport, args.err, out=out,
-                                                 info_tags=info_tags)
+                                                 info_tags=info_tags, ploidy=ploidy)
         os.replace(tmp, out_path)
         tmp = None
         _lap("genotypes + VCF written")

@@ -7,6 +7,7 @@ from __future__ import annotations
 
 import ctypes as C
 import math
+import re
 
 import numpy as np
 
@@ -16,30 +17,138 @@ CELL_BYTES = 24 + 1 + 8 + 1          # pl, gt, ad2, flags of one cell
 BLOCK_BYTES = 256 << 20              # cell arrays of one block of records, at most
 # population INFO tags of --info-tags, in the order they are written: bit k of svjg_vcf_format_cohort_tags's mask
 INFO_TAGS = ("NS", "AN", "AC", "AF", "AC_Het", "AC_Hom", "F_MISSING", "HWE", "ExcHet")
+# with ploidy rules (svjg_vcf_format_cohort_ploidy): one more, bit 9
+PLOIDY_INFO_TAGS = INFO_TAGS + ("AC_Hemi",)
 
 
-def parse_info_tags(text):
-    """--info-tags: a comma list of INFO_TAGS names (any order), or "all".  Returns the names in the order they are
-    written; ValueError for an unknown or repeated name or an empty list."""
+def parse_info_tags(text, ploidy=False):
+    """--info-tags: a comma list of tag names (any order), or "all": INFO_TAGS, or PLOIDY_INFO_TAGS with ``ploidy``.
+    Returns the names in the order they are written; ValueError for an unknown or repeated name, an empty list, or
+    AC_Hemi without ploidy rules."""
+    tags = PLOIDY_INFO_TAGS if ploidy else INFO_TAGS
     if text == "all":
-        return INFO_TAGS
+        return tags
     names = text.split(",")
     for nm in names:
-        if nm not in INFO_TAGS:
-            raise ValueError(f"unknown INFO tag {nm!r} (tags: {','.join(INFO_TAGS)}, or all)")
+        if nm == "AC_Hemi" and not ploidy:
+            raise ValueError("AC_Hemi counts haploid calls: it needs --ploidy-file and --sample-sex")
+        if nm not in tags:
+            raise ValueError(f"unknown INFO tag {nm!r} (tags: {','.join(tags)}, or all)")
     if len(set(names)) != len(names):
         raise ValueError("an INFO tag is named twice")
-    return tuple(t for t in INFO_TAGS if t in names)
+    return tuple(t for t in tags if t in names)
 
 
 def info_tags_mask(names):
-    """The tag mask of svjg_vcf_format_cohort_tags for INFO_TAGS names."""
+    """The tag mask of svjg_vcf_format_cohort_tags / _ploidy for PLOIDY_INFO_TAGS names."""
     mask = 0
     for nm in names:
-        if nm not in INFO_TAGS:
+        if nm not in PLOIDY_INFO_TAGS:
             raise ValueError(f"unknown INFO tag {nm!r}")
-        mask |= 1 << INFO_TAGS.index(nm)
+        mask |= 1 << PLOIDY_INFO_TAGS.index(nm)
     return mask
+
+
+def _table_lines(text):
+    """(line number, whitespace-split columns) of the lines of a rule file that are not blank or '#' comments."""
+    for k, line in enumerate(text.splitlines(), 1):
+        cols = line.split()
+        if cols and not cols[0].startswith("#"):
+            yield k, cols
+
+
+_DECIMAL = re.compile(r"[0-9]+")
+
+
+class PloidyRules:
+    """Sex-chromosome ploidy of a cohort's cells (DESIGN.md §8a).  ``ploidy_text``: the rules in the format of
+    ``bcftools call --ploidy-file``, one ``CHROM FROM TO SEX PLOIDY`` per line (1-based, inclusive), ``* * * SEX
+    PLOIDY`` for the default of a sex.  ``sex_text``: ``NAME SEX`` lines; every name of ``names`` (the cohort) must be
+    listed exactly once, other names are ignored.  Both take '#' comments and blank lines.  ValueError, naming the
+    file and the line, for a file the contract refuses.
+
+    The ploidy of cell (record, sample) is that of the rule for the sample's sex whose CHROM is the record's CHROM
+    column and whose [FROM, TO] holds the record's POS column, else the sex's default, else 2.  The record's CHROM and
+    POS alone decide: an SV that starts in a PAR and ends outside it follows its POS."""
+
+    def __init__(self, ploidy_text, sex_text, names, ploidy_source="ploidy file", sex_source="sample-sex file"):
+        self.rules = {}                   # (chrom, sex) -> (from [k], to [k], ploidy [k]) sorted by from
+        self.defaults = {}                # sex -> ploidy
+        labels = set()
+        spans = {}
+        for k, cols in _table_lines(ploidy_text):
+            where = f"{ploidy_source} line {k}"
+            if len(cols) != 5:
+                raise ValueError(f"{where}: {len(cols)} columns, a rule is CHROM FROM TO SEX PLOIDY")
+            chrom, lo, hi, sex, ploidy = cols
+            if ploidy not in ("0", "1", "2"):
+                raise ValueError(f"{where}: ploidy {ploidy!r}, it must be 0, 1 or 2")
+            labels.add(sex)
+            if chrom == "*" and lo == "*" and hi == "*":
+                if sex in self.defaults:
+                    raise ValueError(f"{where}: a second default ('* * *') for sex {sex!r}")
+                self.defaults[sex] = int(ploidy)
+                continue
+            if not (_DECIMAL.fullmatch(lo) and _DECIMAL.fullmatch(hi)):
+                raise ValueError(f"{where}: FROM and TO must be decimal integers ('* * *' for a default)")
+            lo, hi = int(lo), int(hi)
+            if lo > hi:
+                raise ValueError(f"{where}: FROM {lo} > TO {hi}")
+            spans.setdefault((chrom, sex), []).append((lo, hi, int(ploidy), k))
+        for (chrom, sex), rs in spans.items():
+            rs.sort()
+            for a, b in zip(rs, rs[1:]):
+                if b[0] <= a[1]:
+                    raise ValueError(f"{ploidy_source} lines {a[3]} and {b[3]}: two rules for {chrom} and sex {sex!r} "
+                                     "overlap")
+            self.rules[chrom, sex] = tuple(np.array([r[q] for r in rs], np.int64) for q in range(3))
+        cohort = {nm: None for nm in names}
+        for k, cols in _table_lines(sex_text):
+            if len(cols) != 2:
+                raise ValueError(f"{sex_source} line {k}: {len(cols)} columns, a line is NAME SEX")
+            nm, sex = cols
+            if nm in cohort:
+                if cohort[nm] is not None:
+                    raise ValueError(f"{sex_source} line {k}: sample {nm!r} is listed twice")
+                cohort[nm] = sex
+        missing = [nm for nm, sex in cohort.items() if sex is None]
+        if missing:
+            raise ValueError(f"{sex_source}: no sex for sample {missing[0]!r}" +
+                             (f" and {len(missing) - 1} more" if len(missing) > 1 else ""))
+        self.sample_sex = [cohort[nm] for nm in names]
+        labels.update(self.sample_sex)
+        if len(labels) > capi.PLOIDY_MAX_SEXES:
+            raise ValueError(f"{len(labels)} sex labels in the two files: at most {capi.PLOIDY_MAX_SEXES}")
+        self.sexes = sorted(set(self.sample_sex))                 # the columns of the class table
+        self.sex_index = np.array([self.sexes.index(x) for x in self.sample_sex], np.uint8)
+
+    def record_classes(self, v):
+        """(rclass [n] uint8, table [n_classes][len(sexes)] uint8) of the records of NativeVcf ``v``: record i has
+        ploidy table[rclass[i]][k] in a sample of sex sexes[k].  VcfError for a POS that is not a decimal integer,
+        ValueError beyond 255 classes."""
+        chrom, pos, names = v.loci()
+        order = np.argsort(chrom, kind="stable")
+        bounds = np.searchsorted(chrom[order], np.arange(len(names) + 1))
+        where = {nm: k for k, nm in enumerate(names)}
+        cols = []
+        for sex in self.sexes:
+            col = np.full(v.n, self.defaults.get(sex, 2), np.uint8)
+            for (c, x), (lo, hi, pl) in self.rules.items():
+                if x != sex or c not in where:
+                    continue
+                recs = order[bounds[where[c]]:bounds[where[c] + 1]]
+                p = pos[recs]
+                j = np.searchsorted(lo, p, side="right") - 1           # the last rule that starts at or before POS
+                inside = (j >= 0) & (p <= hi[np.maximum(j, 0)])
+                col[recs[inside]] = pl[j[inside]]
+            cols.append(col)
+        rows = np.ascontiguousarray(np.stack(cols, axis=1)) if v.n else np.full((1, len(self.sexes)), 2, np.uint8)
+        table, rclass = np.unique(rows.view(np.dtype((np.void, rows.shape[1]))).ravel(), return_inverse=True)
+        if len(table) > capi.PLOIDY_MAX_CLASSES:
+            raise ValueError(f"the ploidy rules give the catalogue's records {len(table)} distinct ploidy vectors: "
+                             f"at most {capi.PLOIDY_MAX_CLASSES}")
+        table = np.frombuffer(table.tobytes(), np.uint8).reshape(len(table), len(self.sexes))
+        return np.ascontiguousarray(rclass.reshape(-1)[:v.n], np.uint8), np.ascontiguousarray(table)
 
 
 class Cohort:
@@ -94,9 +203,10 @@ class Cohort:
 
 class _Block:
     """Page-locked result arrays of one block of records: the copies from the device run at PCIe speed.  With
-    ``n_records``, also the site statistics of that many records (svjg_cohort_site_stats, 32 B per record)."""
+    ``n_records``, also the site statistics of that many records (svjg_cohort_site_stats, 32 B per record; with
+    ``ploidy``, svjg_cohort_site_stats_ploidy, 40 B)."""
 
-    def __init__(self, n_cells, n_records=0):
+    def __init__(self, n_cells, n_records=0, ploidy=False):
         n_cells = max(int(n_cells), 1)
         self._mem = [alnfilter.PinnedBytes(n_cells * b) for b in (24, 1, 8, 1)]
         self.pl = self._mem[0].array.view(np.int64).reshape(n_cells, 3)
@@ -105,24 +215,32 @@ class _Block:
         self.flags = self._mem[3].array
         if n_records:
             n_records = int(n_records)
-            self._mem += [alnfilter.PinnedBytes(n_records * b) for b in (16, 8, 8)]
-            self.gcount = self._mem[4].array.view(np.uint32).reshape(n_records, 4)
+            g = 6 if ploidy else 4
+            self._mem += [alnfilter.PinnedBytes(n_records * b) for b in (4 * g, 8, 8)]
+            self.gcount = self._mem[4].array.view(np.uint32).reshape(n_records, g)
             self.hwe = self._mem[5].array.view(np.float64)
             self.exchet = self._mem[6].array.view(np.float64)
 
 
-def _genotype_block(cohort, idx, ty, min_support, e, blk):
-    """(gt, flags, ad2, pl) of the records ``idx`` / ``ty`` in every sample, [n * S] cells in record-major order.
+def _genotype_block(cohort, idx, ty, min_support, e, blk, rclass=None):
+    """(gt, flags, ad2, pl) of the records ``idx`` / ``ty`` in every sample, [n * S] cells in record-major order;
+    with ``rclass``, the ploidy classes of the records (svjg_cohort_genotype_ploidy, after svjg_cohort_set_ploidy).
     Cells whose rounded counts are beyond the LUT are recomputed by genotype.genotype_host from their counters,
-    which ad2 and the halving flags give back exactly."""
+    which ad2 and the halving flags give back exactly.  A haploid cell keeps the device's code: the device fixes the
+    call before it looks up log10 C(n, k), so only PL (of which the text shows PL0 and PL2) comes from the host."""
     n, S = len(idx), cohort.n_samples
     cells = n * S
     gt, fl, ad, pl = blk.gt[:cells], blk.flags[:cells], blk.ad2[:cells], blk.pl[:cells]
     la, lb, lh = math.log10(1 - e), math.log10(e), math.log10(1 / 2)
     lut = genotype.log10comb_lut()
-    capi.check(capi.lib.svjg_cohort_genotype(cohort._h, idx.ctypes.data, ty.ctypes.data, n, int(min_support), la, lb, lh,
-                                             lut.ctypes.data, genotype.LUT_NMAX, pl.ctypes.data, gt.ctypes.data,
-                                             ad.ctypes.data, fl.ctypes.data))
+    if rclass is None:
+        capi.check(capi.lib.svjg_cohort_genotype(cohort._h, idx.ctypes.data, ty.ctypes.data, n, int(min_support), la, lb,
+                                                 lh, lut.ctypes.data, genotype.LUT_NMAX, pl.ctypes.data, gt.ctypes.data,
+                                                 ad.ctypes.data, fl.ctypes.data))
+    else:
+        capi.check(capi.lib.svjg_cohort_genotype_ploidy(cohort._h, idx.ctypes.data, ty.ctypes.data, rclass.ctypes.data, n,
+                                                        int(min_support), la, lb, lh, lut.ctypes.data, genotype.LUT_NMAX,
+                                                        pl.ctypes.data, gt.ctypes.data, ad.ctypes.data, fl.ctypes.data))
     need = np.nonzero(fl & capi.GT_NEED_K)[0]
     if need.size:
         f = fl[need]
@@ -130,47 +248,62 @@ def _genotype_block(cohort, idx, ty, min_support, e, blk):
         n1 = np.where(f & capi.GT_HALVED_1, ad[need, 1], ad[need, 1] >> 1)
         g2, f2, a2, p2 = genotype.genotype_host(np.stack([n0, n1], axis=1), np.arange(need.size, dtype=np.uint32),
                                                 ty[need // S], min_support, e)
-        gt[need], fl[need], ad[need], pl[need] = g2, f2, a2, p2
+        gt[need] = np.where(gt[need] >= capi.GT_HAP_REF, gt[need], g2)
+        fl[need], ad[need], pl[need] = f2, a2, p2
     return gt, fl, ad, pl
 
 
-def _site_stats(cohort, n, blk):
-    """(gcount [n][4] = r0, h, r2, missing; hwe [n]; exchet [n]) of the block _genotype_block genotyped last, from
-    the gt codes on the device.  Those are final: the NEED_K patch above recomputes PL and flags, never the genotype,
-    which genotype_one fixes before it looks up log10 C(n, k)."""
+def _site_stats(cohort, n, blk, ploidy=False):
+    """(gcount [n][4] = r0, h, r2, missing, or with ``ploidy`` [n][6] = r0, h, r2, a0, a1, missing; hwe [n];
+    exchet [n]) of the block _genotype_block genotyped last, from the gt codes on the device.  Those are final: the
+    NEED_K patch above recomputes PL and flags, never the genotype, which genotype_one fixes before it looks up
+    log10 C(n, k)."""
     g, hw, ex = blk.gcount[:n], blk.hwe[:n], blk.exchet[:n]
-    capi.check(capi.lib.svjg_cohort_site_stats(cohort._h, n, g.ctypes.data, hw.ctypes.data, ex.ctypes.data))
+    fn = capi.lib.svjg_cohort_site_stats_ploidy if ploidy else capi.lib.svjg_cohort_site_stats
+    capi.check(fn(cohort._h, n, g.ctypes.data, hw.ctypes.data, ex.ctypes.data))
     return g, hw, ex
 
 
 def genotype_cohort_vcf(tables, cohort, vcf_bytes, names, min_support=genotype.MIN_SUPPORT, e=genotype.ERR, out=None,
-                        block_records=None, info_tags=()):
+                        block_records=None, info_tags=(), ploidy=None):
     """predict-genotype.py's decision_vcf for every sample of ``cohort``: the multi-sample VCF, whose column s is
-    the SAMPLE column of sample s's single-sample VCF.  ``vcf_bytes``: the catalogue VCF's bytes (or lines).
+    the SAMPLE column of sample s's single-sample VCF.  ``vcf_bytes``: the catalogue VCF's bytes (or lines, or a
+    genotype.NativeVcf of them).
     ``names``: one column name per sample.  Returns (text, [genotyped SVs per sample]); with ``out`` (a binary file
     object) each block's text is written there as it is made and the text returned is None.  ``block_records``:
     records per block (default: cell arrays of about 256 MiB); the bytes do not depend on it.  ``info_tags``: INFO_TAGS
     names; their values are computed on the device from each block's genotypes (svjg_cohort_site_stats) and written
-    into the INFO column, and their ##INFO lines in front of the ##FORMAT lines (svjg_vcf_format_cohort_tags)."""
+    into the INFO column, and their ##INFO lines in front of the ##FORMAT lines (svjg_vcf_format_cohort_tags).
+    ``ploidy``: a PloidyRules for the samples of ``names``; the cells are called with their ploidy and the text is
+    that of svjg_vcf_format_cohort_ploidy (PL Number=G, AC_Hemi available)."""
     S = cohort.n_samples
     mask = info_tags_mask(info_tags)
     if len(names) != S:
         raise ValueError(f"{len(names)} names for {S} samples")
-    v = genotype.NativeVcf.from_input(vcf_bytes)
+    if ploidy is None and "AC_Hemi" in info_tags:
+        raise ValueError("AC_Hemi counts haploid calls: it needs ploidy rules")
+    v = vcf_bytes if isinstance(vcf_bytes, genotype.NativeVcf) else genotype.NativeVcf.from_input(vcf_bytes)
     if v is None:
         raise genotype.VcfError("the VCF has non-ASCII bytes or a POS/END of more than 18 digits: "
                                 "cohort genotyping takes only VCFs the native parser reads")
     idx = np.ascontiguousarray(v.index_tables(tables))
     ty = np.ascontiguousarray(v.svtype)
     n = v.n
+    rclass = None
+    if ploidy is not None:
+        rclass, table = ploidy.record_classes(v)
+        capi.check(capi.lib.svjg_cohort_set_ploidy(cohort._h, table.shape[0], table.shape[1], table.ctypes.data,
+                                                   ploidy.sex_index.ctypes.data))
     step = int(block_records) if block_records else max(1, BLOCK_BYTES // (CELL_BYTES * S))
-    blk = _Block(min(step, max(n, 1)) * S, min(step, max(n, 1)) if mask else 0)
+    blk = _Block(min(step, max(n, 1)) * S, min(step, max(n, 1)) if mask else 0, ploidy is not None)
     if not 0 < e < 1:
         # math.log10 raises inside likelihood() only once a record passes the gate (predict-genotype.py:216), as in
-        # genotype.genotype_host: a cohort in which no cell passes it is written with "./." everywhere
+        # genotype.genotype_host: a cohort in which no cell passes it is written with "./." everywhere.  A cell of
+        # ploidy 0 computes no likelihood, so it does not count.
         for lo in range(0, n, step):
-            if (_genotype_block(cohort, idx[lo:lo + step], ty[lo:lo + step], min_support, genotype.ERR, blk)[1]
-                    & capi.GT_GENOTYPED).any():
+            gt, fl = _genotype_block(cohort, idx[lo:lo + step], ty[lo:lo + step], min_support, genotype.ERR, blk,
+                                     None if rclass is None else rclass[lo:lo + step])[:2]
+            if ((fl & capi.GT_GENOTYPED).astype(bool) & (gt != capi.GT_NO_CALL)).any():
                 raise genotype.VcfError("error rate must be in (0, 1)")
         e = genotype.ERR
     joined = "\t".join(names).encode()
@@ -178,14 +311,15 @@ def genotype_cohort_vcf(tables, cohort, vcf_bytes, names, min_support=genotype.M
     pieces = []
     for lo in range(0, n, step) if n else [0]:
         hi = min(n, lo + step)
-        gt, fl, ad, pl = _genotype_block(cohort, idx[lo:hi], ty[lo:hi], min_support, e, blk)
+        gt, fl, ad, pl = _genotype_block(cohort, idx[lo:hi], ty[lo:hi], min_support, e, blk,
+                                         None if rclass is None else rclass[lo:hi])
         site = [None] * 3
         if mask:
-            site = [a.ctypes.data for a in _site_stats(cohort, hi - lo, blk)]
+            site = [a.ctypes.data for a in _site_stats(cohort, hi - lo, blk, rclass is not None)]
         buf, n_out = C.c_void_p(), C.c_uint64()
-        capi.check(capi.lib.svjg_vcf_format_cohort_tags(v._h, lo, hi, S, joined, len(joined), gt.ctypes.data,
-                                                        fl.ctypes.data, ad.ctypes.data, pl.ctypes.data, mask, *site,
-                                                        C.byref(buf), C.byref(n_out), n_gt.ctypes.data))
+        fmt = capi.lib.svjg_vcf_format_cohort_ploidy if rclass is not None else capi.lib.svjg_vcf_format_cohort_tags
+        capi.check(fmt(v._h, lo, hi, S, joined, len(joined), gt.ctypes.data, fl.ctypes.data, ad.ctypes.data,
+                       pl.ctypes.data, mask, *site, C.byref(buf), C.byref(n_out), n_gt.ctypes.data))
         try:
             if out is not None:
                 if n_out.value:

@@ -193,6 +193,22 @@ class NativeVcf:
         p = capi.lib.svjg_vcf_key(self._h, i, C.byref(n))
         return None if not p else C.string_at(p, n.value).decode("ascii")
 
+    def loci(self):
+        """(chrom [n] uint32: index into the names, pos [n] int64, [distinct CHROM names in order of first appearance])
+        from the CHROM and POS columns; VcfError for a POS that is not 1 to 18 decimal digits."""
+        chrom, pos = np.empty(max(self.n, 1), np.uint32), np.empty(max(self.n, 1), np.int64)
+        buf, n_bytes, n_chroms = C.c_void_p(), C.c_uint64(), C.c_uint32()
+        rc = capi.lib.svjg_vcf_loci(self._h, chrom.ctypes.data, pos.ctypes.data, C.byref(buf), C.byref(n_bytes),
+                                    C.byref(n_chroms))
+        if rc == capi.E_INPUT:
+            raise VcfError(capi.lib.svjg_last_error().decode("utf-8", "replace"))
+        capi.check(rc)
+        try:
+            names = C.string_at(buf.value, n_bytes.value).decode("ascii").split("\n") if n_chroms.value else []
+        finally:
+            capi.lib.svjg_buffer_free(buf)
+        return chrom[:self.n], pos[:self.n], names
+
     def index_tables(self, tables):
         idx = np.empty(max(self.n, 1), np.uint32)
         capi.check(capi.lib.svjg_vcf_index_tables(self._h, tables._h, idx.ctypes.data))
