@@ -294,6 +294,31 @@ int svjg_cohort_genotype_ploidy(svjg_cohort *c, const uint32_t *sv_index, const 
                                 uint8_t *flags);
 int svjg_cohort_site_stats_ploidy(svjg_cohort *c, uint32_t n, uint32_t *gcount, double *hwe, double *exchet);
 
+/* Genotype posteriors (DESIGN.md §8a): the ALT allele frequency of each record by EM over its cells' likelihoods, and
+ * each cell's posterior under the Hardy-Weinberg prior at that frequency.
+ *   svjg_cohort_posteriors  for the n records of the last svjg_cohort_genotype(_ploidy) call (n must be its record
+ *                           count), from the pl / gt / flags that call left on the device.  First the n_patch cells
+ *                           patch_cell [n_patch] u32 (record-major cell index) get pl patch_pl [n_patch][3] i64 and
+ *                           lose SVJG_GT_NEED_K there (the caller's recomputed PLs).  plw [plw_n] f64 is
+ *                           T[k] = 10^(-k/10), k < SVJG_POST_PLW_N (= plw_n), cached in the handle.
+ *                           A cell contributes when it is SVJG_GT_GENOTYPED and its code is not SVJG_GT_NO_CALL: codes
+ *                           0-3 are diploid, 4-6 haploid.  Weights w_g = T[PL_g - min PL] (0 beyond the table; a
+ *                           haploid cell uses PL0 and PL2).  From f = 0.5 the EM step f = sum(e) / (sum of the
+ *                           ploidies) runs until |f_new - f| <= SVJG_POST_TOL or SVJG_POST_MAX_ITERS steps, in the
+ *                           fixed double-precision order of DESIGN.md §8a.  Outputs: af [n] f64 (NaN when no cell
+ *                           contributes), gp [n][S][3] f64 (haploid: GP1 = 0; non-contributing cells 0),
+ *                           gq [n][S] u8 (floored phred of the called genotype's posterior error, at most
+ *                           SVJG_POST_GQ_MAX; SVJG_POST_GQ_NONE for a missing call or a non-contributing cell) and,
+ *                           when iters is not NULL, iters [n] u8 (EM steps, 0 with no estimate).  SVJG_E_ARG when a
+ *                           contributing cell still has SVJG_GT_NEED_K after the patch.  Synchronous. */
+#define SVJG_POST_PLW_N 4096
+#define SVJG_POST_MAX_ITERS 100
+#define SVJG_POST_TOL 1e-10
+#define SVJG_POST_GQ_MAX 99
+#define SVJG_POST_GQ_NONE 255
+int svjg_cohort_posteriors(svjg_cohort *c, uint32_t n, uint32_t n_patch, const uint32_t *patch_cell, const int64_t *patch_pl,
+                           const double *plw, uint32_t plw_n, double *af, double *gp, uint8_t *gq, uint8_t *iters);
+
 /* Page-locked host memory (cudaHostAlloc) for file buffers and results: copies to and from it run
  * at PCIe speed.  For callers that do not want a tensor library just to pin memory. */
 int svjg_host_alloc(uint64_t bytes, void **out);
@@ -438,6 +463,19 @@ int svjg_vcf_format_cohort_ploidy(const svjg_vcf *v, uint32_t lo, uint32_t hi, u
                                   uint64_t names_len, const uint8_t *gt, const uint8_t *flags, const uint32_t *ad2,
                                   const int64_t *pl, uint32_t tags, const uint32_t *gcount, const double *hwe,
                                   const double *exchet, char **out, uint64_t *out_len, uint64_t *n_genotyped);
+/* svjg_vcf_format_cohort_post: svjg_vcf_format_cohort_ploidy (ploidy = 1) or _tags (ploidy = 0) with the genotype
+ * posteriors of svjg_cohort_posteriors for the range: af [hi - lo], gp [hi - lo][S][3], gq [hi - lo][S].  With af, gp
+ * and gq NULL it is that formatter, byte for byte.  With them:
+ *   FORMAT is GT:DP:AD:PL:GP:GQ, with ##FORMAT lines of GP (Number=G) and GQ after the PL line; a genotyped cell of
+ *   ploidy 2 or 1 gets ":GP0,GP1,GP2:GQ" or ":GP0,GP2:GQ" after its text (GQ "." when it is SVJG_POST_GQ_NONE), every
+ *   other cell ":.:.".  INFO: AF_EM=af after the selected tags ("." when af is NaN); its ##INFO line after theirs; a
+ *   catalogue's AF_EM items and ##INFO lines are dropped.  A record whose ALT holds a comma gets "." for AF_EM and
+ *   ":.:." in every cell.  Floats are "%.6g". */
+int svjg_vcf_format_cohort_post(const svjg_vcf *v, uint32_t lo, uint32_t hi, uint32_t n_samples, const char *names,
+                                uint64_t names_len, const uint8_t *gt, const uint8_t *flags, const uint32_t *ad2,
+                                const int64_t *pl, uint32_t ploidy, uint32_t tags, const uint32_t *gcount,
+                                const double *hwe, const double *exchet, const double *af, const double *gp,
+                                const uint8_t *gq, char **out, uint64_t *out_len, uint64_t *n_genotyped);
 void svjg_buffer_free(char *p);
 
 /* ---- output (host) ------------------------------------------------------------

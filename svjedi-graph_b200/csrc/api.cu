@@ -380,6 +380,8 @@ extern "C" void svjg_cohort_free(svjg_cohort *c) {
     if (c->d_blk) cudaFree(c->d_blk);
     if (c->d_site) cudaFree(c->d_site);
     if (c->d_ploidy) cudaFree(c->d_ploidy);
+    if (c->d_plw) cudaFree(c->d_plw);
+    if (c->d_post) cudaFree(c->d_post);
     if (c->stream) cudaStreamDestroy(c->stream);
     delete c;
 }

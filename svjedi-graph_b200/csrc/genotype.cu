@@ -408,6 +408,205 @@ cohort_site_stats_kernel(const uint8_t *__restrict__ gt, uint32_t n, uint32_t n_
     exchet[i] = p_exc;
 }
 
+// ---- genotype posteriors: the allele frequency of a record by EM over its cells' likelihoods, then GP and GQ at it
+// (DESIGN.md §8a, "Genotype posteriors").  Every operation is one IEEE double rounded to nearest (intrinsics: no
+// contraction), in the order of the statement in tests/test_cohort_posteriors.py.
+constexpr int POST_WARPS = 8;                  // records (one per warp) of a thread block
+enum : uint32_t { CELL_OUT = 0, CELL_HAP = 1, CELL_DIP = 2 };
+
+// The kind of cell k and its weights w_g = T[PL_g - min PL] (0 beyond the table).  A contributing cell that still has
+// NEED_K (its PL was never patched) sets *bad.
+__device__ __forceinline__ uint32_t post_weights(const int64_t *__restrict__ pl, const uint8_t *__restrict__ gt,
+                                                 const uint8_t *__restrict__ flags, const double *__restrict__ T, size_t k,
+                                                 double &w0, double &w1, double &w2, uint32_t *bad) {
+    w0 = w1 = w2 = 0.0;
+    const uint8_t f = flags[k], g = gt[k];
+    if (!(f & SVJG_GT_GENOTYPED) || g == SVJG_GT_NO_CALL) return CELL_OUT;
+    if (f & SVJG_GT_NEED_K) atomicOr(bad, 1u);
+    const int64_t p0 = pl[3 * k], p1 = pl[3 * k + 1], p2 = pl[3 * k + 2];
+    auto wt = [&](int64_t d) { return d > SVJG_POST_PLW_N - 1 ? 0.0 : __ldg(T + d); };
+    if (g >= SVJG_GT_HAP_REF) {
+        const int64_t m = min(p0, p2);
+        w0 = wt(p0 - m);
+        w2 = wt(p2 - m);
+        return CELL_HAP;
+    }
+    const int64_t m = min(min(p0, p1), p2);
+    w0 = wt(p0 - m);
+    w1 = wt(p1 - m);
+    w2 = wt(p2 - m);
+    return CELL_DIP;
+}
+
+// The genotype terms of a cell at f (q = 1 - f; P = q*q, (f*q)*2, f*f): a, b, c and den.  Haploid: a = w0*q, b = 0,
+// c = w2*f, den = a + c.
+struct PostPriors {
+    double f, q, p0, p1, p2;
+};
+__device__ __forceinline__ PostPriors post_priors(double f) {
+    const double q = __dsub_rn(1.0, f);
+    return {f, q, __dmul_rn(q, q), __dmul_rn(__dmul_rn(f, q), 2.0), __dmul_rn(f, f)};
+}
+__device__ __forceinline__ void post_terms(uint32_t kind, double w0, double w1, double w2, const PostPriors &p, double &a,
+                                           double &b, double &c, double &den) {
+    if (kind == CELL_DIP) {
+        a = __dmul_rn(w0, p.p0);
+        b = __dmul_rn(w1, p.p1);
+        c = __dmul_rn(w2, p.p2);
+        den = __dadd_rn(__dadd_rn(a, b), c);
+    } else {
+        a = __dmul_rn(w0, p.q);
+        b = 0.0;
+        c = __dmul_rn(w2, p.f);
+        den = __dadd_rn(a, c);
+    }
+}
+// expected ALT allele count of a contributing cell: (b + 2c) / den, or c / den for a haploid one
+__device__ __forceinline__ double post_e(uint32_t kind, double w0, double w1, double w2, const PostPriors &p) {
+    double a, b, c, den;
+    post_terms(kind, w0, w1, w2, p, a, b, c, den);
+    return kind == CELL_DIP ? __ddiv_rn(__dadd_rn(b, __dmul_rn(c, 2.0)), den) : __ddiv_rn(c, den);
+}
+
+// GP of cell k at f̂ into gp[3k..] (haploid: GP1 = 0) and GQ into gq[k]: the largest q <= 99 with err <= T[q], where
+// err is the other genotypes' terms over den (T is decreasing, so the q that pass are a prefix: a binary search);
+// SVJG_POST_GQ_NONE for a missing call or a cell that does not contribute.
+__device__ __forceinline__ void post_cell_out(uint32_t kind, double w0, double w1, double w2, const PostPriors &p,
+                                              uint8_t g, const double *__restrict__ T, double *__restrict__ gp,
+                                              uint8_t *__restrict__ gq, size_t k) {
+    if (kind == CELL_OUT) {
+        gp[3 * k] = gp[3 * k + 1] = gp[3 * k + 2] = 0.0;
+        gq[k] = SVJG_POST_GQ_NONE;
+        return;
+    }
+    double a, b, c, den;
+    post_terms(kind, w0, w1, w2, p, a, b, c, den);
+    gp[3 * k] = __ddiv_rn(a, den);
+    gp[3 * k + 1] = kind == CELL_DIP ? __ddiv_rn(b, den) : 0.0;
+    gp[3 * k + 2] = __ddiv_rn(c, den);
+    double other;
+    switch (g) {
+        case 0: other = __dadd_rn(b, c); break;
+        case 1: other = __dadd_rn(a, c); break;
+        case 2: other = __dadd_rn(a, b); break;
+        case SVJG_GT_HAP_REF: other = c; break;
+        case SVJG_GT_HAP_ALT: other = a; break;
+        default: gq[k] = SVJG_POST_GQ_NONE; return;   // ./. and . (below -ms, or a tie)
+    }
+    const double err = __ddiv_rn(other, den);
+    uint32_t lo = 0, hi = SVJG_POST_GQ_MAX;            // err <= T[lo] holds (err <= 1 = T[0])
+    while (lo < hi) {
+        const uint32_t mid = (lo + hi + 1) / 2;
+        if (err <= __ldg(T + mid)) lo = mid;
+        else hi = mid - 1;
+    }
+    gq[k] = uint8_t(lo);
+}
+
+__device__ __forceinline__ double warp_sum(double x) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) x = __dadd_rn(x, __shfl_xor_sync(0xFFFFFFFFu, x, o));
+    return x;
+}
+
+// One warp per record i of the block the last cohort genotype call left on the device (pl [n][S][3], gt, flags
+// [n][S]).  Lane l owns the cells s = l (mod 32).  CPL > 0: S <= 32 CPL, and a lane keeps the weights and kinds of its
+// cells in registers.  CPL == 0: any S; the weights are written once into the cell's gp slots and its kind into its
+// gq byte, read back (from L2) in every iteration and overwritten by the results at the end.
+// Results: af[i] = f̂ (NaN when no cell contributes), iters[i] = EM iterations (0 then), gp [n][S][3], gq [n][S].
+template <int CPL>
+__global__ void __launch_bounds__(POST_WARPS * 32)
+cohort_posterior_kernel(const int64_t *__restrict__ pl, const uint8_t *__restrict__ gt, const uint8_t *__restrict__ flags,
+                        uint32_t n, uint32_t S, const double *__restrict__ T, double *__restrict__ af,
+                        uint8_t *__restrict__ iters, double *__restrict__ gp, uint8_t *__restrict__ gq,
+                        uint32_t *__restrict__ bad) {
+    const uint32_t i = blockIdx.x * POST_WARPS + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (i >= n) return;                                // whole warps leave together
+    const size_t row = size_t(i) * S;
+    double w[CPL > 0 ? CPL : 1][3];
+    uint32_t kind[CPL > 0 ? CPL : 1];
+    uint32_t ploidy_sum = 0;
+    if constexpr (CPL > 0) {
+#pragma unroll
+        for (int j = 0; j < CPL; ++j) {
+            const uint32_t s = lane + 32 * j;
+            kind[j] = CELL_OUT;
+            w[j][0] = w[j][1] = w[j][2] = 0.0;
+            if (s < S) kind[j] = post_weights(pl, gt, flags, T, row + s, w[j][0], w[j][1], w[j][2], bad);
+            ploidy_sum += kind[j];
+        }
+    } else {
+        for (uint32_t s = lane; s < S; s += 32) {
+            double w0, w1, w2;
+            const uint32_t kd = post_weights(pl, gt, flags, T, row + s, w0, w1, w2, bad);
+            gp[3 * (row + s)] = w0;
+            gp[3 * (row + s) + 1] = w1;
+            gp[3 * (row + s) + 2] = w2;
+            gq[row + s] = uint8_t(kd);
+            ploidy_sum += kd;
+        }
+    }
+    ploidy_sum = __reduce_add_sync(0xFFFFFFFFu, ploidy_sum);
+    double f = __longlong_as_double(0x7FF8000000000000ll);
+    uint32_t it = 0;
+    if (ploidy_sum) {
+        const double A = double(ploidy_sum);
+        f = 0.5;
+        for (;;) {
+            const PostPriors p = post_priors(f);
+            double x = 0.0;
+            if constexpr (CPL > 0) {
+#pragma unroll
+                for (int j = 0; j < CPL; ++j)
+                    if (kind[j] != CELL_OUT) x = __dadd_rn(x, post_e(kind[j], w[j][0], w[j][1], w[j][2], p));
+            } else {
+                for (uint32_t s = lane; s < S; s += 32) {
+                    const uint32_t kd = gq[row + s];
+                    if (kd != CELL_OUT) {
+                        const double *wk = gp + 3 * (row + s);
+                        x = __dadd_rn(x, post_e(kd, wk[0], wk[1], wk[2], p));
+                    }
+                }
+            }
+            const double f_new = __ddiv_rn(warp_sum(x), A);
+            ++it;
+            const bool done = fabs(__dsub_rn(f_new, f)) <= SVJG_POST_TOL || it == SVJG_POST_MAX_ITERS;
+            f = f_new;
+            if (done) break;
+        }
+    }
+    if (lane == 0) {
+        af[i] = f;
+        iters[i] = uint8_t(it);
+    }
+    const PostPriors p = post_priors(f);
+    if constexpr (CPL > 0) {
+#pragma unroll
+        for (int j = 0; j < CPL; ++j) {
+            const uint32_t s = lane + 32 * j;
+            if (s < S) post_cell_out(kind[j], w[j][0], w[j][1], w[j][2], p, gt[row + s], T, gp, gq, row + s);
+        }
+    } else {
+        for (uint32_t s = lane; s < S; s += 32) {
+            const size_t k = row + s;
+            const uint32_t kd = gq[k];
+            post_cell_out(kd, gp[3 * k], gp[3 * k + 1], gp[3 * k + 2], p, gt[k], T, gp, gq, k);
+        }
+    }
+}
+
+// The host's PL of the NEED_K cells of the block (svjg_cohort_posteriors' patch) scattered into it, NEED_K cleared
+__global__ void cohort_patch_kernel(const uint32_t *__restrict__ cell, const int64_t *__restrict__ patch_pl, uint32_t m,
+                                    int64_t *__restrict__ pl, uint8_t *__restrict__ flags) {
+    const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= m) return;
+    const size_t c = cell[k];
+    pl[3 * c] = patch_pl[3 * size_t(k)];
+    pl[3 * c + 1] = patch_pl[3 * size_t(k) + 1];
+    pl[3 * c + 2] = patch_pl[3 * size_t(k) + 2];
+    flags[c] &= uint8_t(~SVJG_GT_NEED_K);
+}
+
 }  // namespace
 
 extern "C" int svjg_genotype_device(const uint32_t *d_counts, const uint32_t *d_sv_index, const uint8_t *d_svtype,
@@ -579,6 +778,8 @@ int cohort_genotype(const char *fn, svjg_cohort *c, const uint32_t *sv_index, co
     SVJG_CUDA(cudaStreamSynchronize(st));
     c->blk_n = n;
     c->blk_gt = o_gt;
+    c->blk_pl = o_pl;
+    c->blk_fl = o_fl;
     return SVJG_OK;
 }
 
@@ -644,6 +845,76 @@ extern "C" int svjg_cohort_site_stats(svjg_cohort *c, uint32_t n, uint32_t *gcou
 
 extern "C" int svjg_cohort_site_stats_ploidy(svjg_cohort *c, uint32_t n, uint32_t *gcount, double *hwe, double *exchet) {
     return cohort_site_stats("svjg_cohort_site_stats_ploidy", true, c, n, gcount, hwe, exchet);
+}
+
+// Genotype posteriors of the block of the last genotype call, from its pl / gt / flags where that call left them on the
+// device: the host's PLs of the NEED_K cells go in first, then one warp per record runs the EM and writes GP and GQ.
+extern "C" int svjg_cohort_posteriors(svjg_cohort *c, uint32_t n, uint32_t n_patch, const uint32_t *patch_cell,
+                                      const int64_t *patch_pl, const double *plw, uint32_t plw_n, double *af, double *gp,
+                                      uint8_t *gq, uint8_t *iters) {
+    const std::string f = "svjg_cohort_posteriors";
+    if (!c) return svjg::set_error(SVJG_E_ARG, f + ": NULL cohort");
+    if (n != c->blk_n)
+        return svjg::set_error(SVJG_E_ARG, f + ": n is not the record count of the last svjg_cohort_genotype call");
+    if (n == 0) return SVJG_OK;
+    if (!plw || !af || !gp || !gq || (n_patch && (!patch_cell || !patch_pl)))
+        return svjg::set_error(SVJG_E_ARG, f + ": NULL argument");
+    if (plw_n != SVJG_POST_PLW_N) return svjg::set_error(SVJG_E_ARG, f + ": the weight table must have SVJG_POST_PLW_N entries");
+    const uint64_t cells = uint64_t(n) * c->n_samples;
+    for (uint32_t k = 0; k < n_patch; ++k)
+        if (patch_cell[k] >= cells) return svjg::set_error(SVJG_E_ARG, f + ": patch cell out of range");
+    SVJG_CUDA(cudaSetDevice(c->t->device));
+    cudaStream_t st = c->stream;
+    // the table is uploaded again only when its contents change
+    if (c->plw.size() != plw_n || memcmp(c->plw.data(), plw, size_t(plw_n) * 8) != 0) {
+        if (c->d_plw) SVJG_CUDA(cudaFree(c->d_plw));
+        c->d_plw = nullptr;
+        c->plw.clear();
+        SVJG_CUDA(cudaMalloc(&c->d_plw, size_t(plw_n) * 8));
+        SVJG_CUDA(cudaMemcpy(c->d_plw, plw, size_t(plw_n) * 8, cudaMemcpyHostToDevice));
+        c->plw.assign(plw, plw + plw_n);
+    }
+    auto up = [](size_t x) { return (x + 255) & ~size_t(255); };
+    const size_t b_pc = size_t(n_patch) * 4, b_pp = size_t(n_patch) * 24, b_af = size_t(n) * 8, b_it = n,
+                 b_gp = cells * 24, b_gq = cells;
+    const size_t o_pp = up(b_pc), o_af = o_pp + up(b_pp), o_it = o_af + up(b_af), o_gp = o_it + up(b_it),
+                 o_gq = o_gp + up(b_gp), o_bad = o_gq + up(b_gq), total = o_bad + 256;
+    if (c->post_cap < total) {
+        if (c->d_post) SVJG_CUDA(cudaFree(c->d_post));
+        c->d_post = nullptr;
+        c->post_cap = 0;
+        SVJG_CUDA(cudaMalloc(&c->d_post, total));
+        c->post_cap = total;
+    }
+    uint8_t *d = c->d_post, *blk = c->d_blk;
+    int64_t *d_pl = reinterpret_cast<int64_t *>(blk + c->blk_pl);
+    uint32_t *d_bad = reinterpret_cast<uint32_t *>(d + o_bad);
+    if (n_patch) {
+        SVJG_CUDA(cudaMemcpyAsync(d, patch_cell, b_pc, cudaMemcpyHostToDevice, st));
+        SVJG_CUDA(cudaMemcpyAsync(d + o_pp, patch_pl, b_pp, cudaMemcpyHostToDevice, st));
+        cohort_patch_kernel<<<(n_patch + 255) / 256, 256, 0, st>>>(reinterpret_cast<const uint32_t *>(d),
+                                                                  reinterpret_cast<const int64_t *>(d + o_pp), n_patch,
+                                                                  d_pl, blk + c->blk_fl);
+        SVJG_CUDA(cudaGetLastError());
+    }
+    SVJG_CUDA(cudaMemsetAsync(d_bad, 0, 4, st));
+    // weights in registers while a lane has at most 4 cells, else written once into the gp slots and read from L2
+    const uint32_t S = c->n_samples;
+    auto kernel = S <= 32 ? cohort_posterior_kernel<1> : S <= 64 ? cohort_posterior_kernel<2>
+                : S <= 128 ? cohort_posterior_kernel<4> : cohort_posterior_kernel<0>;
+    kernel<<<(n + POST_WARPS - 1) / POST_WARPS, POST_WARPS * 32, 0, st>>>(
+        d_pl, blk + c->blk_gt, blk + c->blk_fl, n, S, c->d_plw, reinterpret_cast<double *>(d + o_af), d + o_it,
+        reinterpret_cast<double *>(d + o_gp), d + o_gq, d_bad);
+    SVJG_CUDA(cudaGetLastError());
+    uint32_t bad = 0;
+    SVJG_CUDA(cudaMemcpyAsync(af, d + o_af, b_af, cudaMemcpyDeviceToHost, st));
+    if (iters) SVJG_CUDA(cudaMemcpyAsync(iters, d + o_it, b_it, cudaMemcpyDeviceToHost, st));
+    SVJG_CUDA(cudaMemcpyAsync(gp, d + o_gp, b_gp, cudaMemcpyDeviceToHost, st));
+    SVJG_CUDA(cudaMemcpyAsync(gq, d + o_gq, b_gq, cudaMemcpyDeviceToHost, st));
+    SVJG_CUDA(cudaMemcpyAsync(&bad, d_bad, 4, cudaMemcpyDeviceToHost, st));
+    SVJG_CUDA(cudaStreamSynchronize(st));
+    if (bad) return svjg::set_error(SVJG_E_ARG, f + ": a contributing cell still has SVJG_GT_NEED_K (no PL patched in)");
+    return SVJG_OK;
 }
 
 // ---------------------------------------------------------------------------

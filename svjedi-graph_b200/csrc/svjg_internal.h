@@ -45,8 +45,13 @@ struct svjg_cohort {
     size_t blk_cap = 0;
     uint32_t blk_n = 0;                       // records of the last block genotyped (0: none)
     size_t blk_gt = 0;                        // offset of its gt codes [blk_n][n_samples] in d_blk
+    size_t blk_pl = 0, blk_fl = 0;            // offsets of its pl [blk_n][n_samples][3] and flags [blk_n][n_samples]
     uint8_t *d_site = nullptr;                // site statistics of the last block (svjg_cohort_site_stats)
     size_t site_cap = 0;
+    std::vector<double> plw;                  // host copy of what d_plw holds: T[k] = 10^(-k/10) (svjg_cohort_posteriors)
+    double *d_plw = nullptr;
+    uint8_t *d_post = nullptr;                // inputs and results of the last svjg_cohort_posteriors call
+    size_t post_cap = 0;
     uint8_t *d_ploidy = nullptr;              // svjg_cohort_set_ploidy: table [n_classes][n_sexes], then sex [n_samples]
     uint32_t n_classes = 0, n_sexes = 0;
 };

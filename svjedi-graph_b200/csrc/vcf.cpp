@@ -32,6 +32,15 @@ const char FORMAT_LINES[] =
     "##FORMAT=<ID=PL,Number=3,Type=Integer,Description=\"Phred-scaled likelihood for each genotype\">\n"
     "#CHROM\tPOS\tID\tREF\tALT\tQUAL\tFILTER\tINFO\tFORMAT\t";      // then the sample names and "\n"
 const char PL_NUMBER[] = "ID=PL,Number=";                               // followed by "3", or "G" with ploidy
+// genotype posteriors (svjg_vcf_format_cohort_post): after the PL line, and the INFO line of the EM frequency
+const char POST_FORMAT_LINES[] =
+    "##FORMAT=<ID=GP,Number=G,Type=Float,Description=\"Genotype posterior probabilities under a Hardy-Weinberg prior at "
+    "the allele frequency AF_EM\">\n"
+    "##FORMAT=<ID=GQ,Number=1,Type=Integer,Description=\"Phred-scaled posterior probability that the genotype call is "
+    "wrong (floored, at most 99)\">\n";
+const char AF_EM_INFO_LINE[] =
+    "##INFO=<ID=AF_EM,Number=A,Type=Float,Description=\"ALT allele frequency estimated by EM over the samples' genotype "
+    "likelihoods\">\n";
 
 struct Rec {
     uint64_t head_off;   // into text
@@ -410,14 +419,6 @@ bool selected_tag(uint32_t tags, sv key) {
     return false;
 }
 
-// "##INFO=<ID=X," or "##INFO=<ID=X>" for a selected X
-bool info_header_of(uint32_t tags, sv line) {
-    if (!starts_with(line, "##INFO=<ID=")) return false;
-    const sv rest = line.substr(11);
-    const size_t e = rest.find_first_of(",>");
-    return e != sv::npos && selected_tag(tags, rest.substr(0, e));
-}
-
 // The value text of tag t for counts g = (r0, h, r2, m), or with ploidy (r0, h, r2, a0, a1, m), of S cells; "." where it
 // has none
 size_t tag_value(char *o, uint32_t t, const uint32_t *g, bool ploidy, uint64_t S, double hwe, double exchet, bool multi_alt) {
@@ -449,17 +450,34 @@ size_t tag_value(char *o, uint32_t t, const uint32_t *g, bool ploidy, uint64_t S
     }
 }
 
-// svjg_vcf_format_cohort_ploidy, and with ploidy == false svjg_vcf_format_cohort_tags
+// "%.6g" of a probability x in [0, 1]: 0 and the values that print as 1 without snprintf (most cells of a confident
+// call), the rest with it
+inline char *put_prob(char *o, double x) {
+    if (x == 0.0) {
+        *o++ = '0';
+        return o;
+    }
+    if (x >= 0.99999951) {      // clear of the rounding boundary 0.9999995: "1"
+        *o++ = '1';
+        return o;
+    }
+    return o + snprintf(o, 16, "%.6g", x);
+}
+
+// svjg_vcf_format_cohort_post; with af == gp == gq == NULL svjg_vcf_format_cohort_ploidy, and with ploidy == false
+// svjg_vcf_format_cohort_tags
 int format_cohort(bool ploidy, const svjg_vcf *v, uint32_t lo, uint32_t hi, uint32_t n_samples, const char *names,
                   uint64_t names_len, const uint8_t *gt, const uint8_t *flags, const uint32_t *ad2, const int64_t *pl,
-                  uint32_t tags, const uint32_t *gcount, const double *hwe, const double *exchet, char **out,
-                  uint64_t *out_len, uint64_t *n_genotyped) {
+                  uint32_t tags, const uint32_t *gcount, const double *hwe, const double *exchet, const double *af,
+                  const double *gp, const uint8_t *gq, char **out, uint64_t *out_len, uint64_t *n_genotyped) {
 
     if (!v || !out || !out_len || !names || !n_genotyped) return set_error(SVJG_E_ARG, "svjg_vcf_format: NULL argument");
     const size_t n_all = v->recs.size();
     if (lo > hi || hi > n_all || n_samples == 0) return set_error(SVJG_E_ARG, "svjg_vcf_format: bad record range or sample count");
     const size_t S = n_samples, n = size_t(hi - lo), n_cells = n * S;
     if (n && (!gt || !flags || !ad2 || !pl)) return set_error(SVJG_E_ARG, "svjg_vcf_format: NULL argument");
+    const bool post = af || gp || gq;
+    if (post && n && !(af && gp && gq)) return set_error(SVJG_E_ARG, "svjg_vcf_format: af, gp and gq go together");
     if (tags >> (ploidy ? N_INFO_TAGS : N_DIPLOID_TAGS)) return set_error(SVJG_E_ARG, "svjg_vcf_format: unknown INFO tag bit");
     const size_t G = ploidy ? 6 : 4;                          // counts per record in gcount
     // every tag needs the counts (HWE and ExcHet are "." when NS = 0)
@@ -476,21 +494,37 @@ int format_cohort(bool ploidy, const svjg_vcf *v, uint32_t lo, uint32_t hi, uint
     for (size_t k = 0; k < n_cells; ++k)
         if (ploidy ? gt[k] > SVJG_GT_NO_CALL : (flags[k] & SVJG_GT_GENOTYPED) && gt[k] > 3)
             return set_error(SVJG_E_ARG, "svjg_vcf_format: gt code out of range");
+    if (post)
+        for (size_t k = 0; k < n_cells; ++k)
+            if (gq[k] > SVJG_POST_GQ_MAX && gq[k] != SVJG_POST_GQ_NONE)
+                return set_error(SVJG_E_ARG, "svjg_vcf_format: GQ out of range");
     static const char *GT_TEXT[4] = {"0/0", "0/1", "1/1", "./."};
     static const char HAP_TEXT[3] = {'0', '1', '.'};
     std::string format_lines(FORMAT_LINES, sizeof FORMAT_LINES - 1);
     if (ploidy) format_lines[format_lines.find(PL_NUMBER) + sizeof PL_NUMBER - 1] = 'G';
+    if (post) format_lines.insert(format_lines.find("#CHROM"), POST_FORMAT_LINES);
     const char *text = v->text.data();
     std::string info_hdr;                  // the ##INFO lines of the selected tags, in front of the ##FORMAT lines
     for (uint32_t t = 0; t < N_INFO_TAGS; ++t)
         if (tags >> t & 1) info_hdr += INFO_TAGS[t].hdr;
+    if (post) info_hdr += AF_EM_INFO_LINE;
+    // the column text of FORMAT and its length with the tab in front
+    const sv fmt_col = post ? sv("\tGT:DP:AD:PL:GP:GQ") : sv("\tGT:DP:AD:PL");
+    // INFO keys the formatter writes itself: the selected tags and, with posteriors, AF_EM
+    auto own_key = [&](sv key) { return selected_tag(tags, key) || (post && key == "AF_EM"); };
+    auto own_info_line = [&](sv line) {     // "##INFO=<ID=X," or "##INFO=<ID=X>" for such an X
+        if (!starts_with(line, "##INFO=<ID=")) return false;
+        const sv rest = line.substr(11);
+        const size_t e = rest.find_first_of(",>");
+        return e != sv::npos && own_key(rest.substr(0, e));
+    };
     // the header lines of the range: those in front of its records and, for the last range, the ones behind them
     size_t h_lo = 0;
     while (h_lo < v->hdrs.size() && v->hdrs[h_lo].before < lo) ++h_lo;
     size_t h_hi = h_lo;
     while (h_hi < v->hdrs.size() && (hi == n_all || v->hdrs[h_hi].before < hi)) ++h_hi;
     const size_t col_hdr = info_hdr.size() + format_lines.size() + names_len + 1;
-    auto dropped = [&](const Hdr &h) { return tags && info_header_of(tags, sv(text + h.off, h.len)); };
+    auto dropped = [&](const Hdr &h) { return (tags || post) && own_info_line(sv(text + h.off, h.len)); };
     auto hdr_len = [&](const Hdr &h) -> uint64_t { return h.len == UINT32_MAX ? col_hdr : dropped(h) ? 0 : h.len; };
     auto put_hdr = [&](char *o, const Hdr &h) {
         if (h.len != UINT32_MAX) return dropped(h) ? o : put_mem(o, text + h.off, h.len);
@@ -500,8 +534,14 @@ int format_cohort(bool ploidy, const svjg_vcf *v, uint32_t lo, uint32_t hi, uint
         *o++ = '\n';
         return o;
     };
-    // columns 1-8 of record lo + j: as the catalogue has them, or with the INFO column rewritten for the tags.
-    // o == nullptr: the length only
+    // a record whose ALT (column 5) holds a comma: its cells are biallelic codes, so Number=A values are "."
+    auto multi_alt_of = [&](sv head) {
+        size_t a = 0;
+        for (int c = 0; c < 4; ++c) a = head.find('\t', a) + 1;
+        return head.substr(a, head.find('\t', a) - a).find(',') != sv::npos;
+    };
+    // columns 1-8 of record lo + j: as the catalogue has them, or with the INFO column rewritten for the tags and
+    // AF_EM.  o == nullptr: the length only
     auto put_head = [&](char *o, size_t j) -> uint64_t {
         const Rec &r = v->recs[lo + j];
         const sv head(text + r.head_off, r.head_len);
@@ -510,7 +550,7 @@ int format_cohort(bool ploidy, const svjg_vcf *v, uint32_t lo, uint32_t hi, uint
             if (o) memcpy(o + len, p, k);
             len += k;
         };
-        if (!tags) {
+        if (!tags && !post) {
             put(head.data(), head.size());
             return len;
         }
@@ -523,7 +563,7 @@ int format_cohort(bool ploidy, const svjg_vcf *v, uint32_t lo, uint32_t hi, uint
                 size_t b = info.find(';', a);
                 if (b == sv::npos) b = info.size();
                 const sv item = info.substr(a, b - a);
-                if (!selected_tag(tags, item.substr(0, item.find('=')))) {
+                if (!own_key(item.substr(0, item.find('=')))) {
                     if (!first) put(";", 1);
                     put(item.data(), item.size());
                     first = false;
@@ -532,9 +572,7 @@ int format_cohort(bool ploidy, const svjg_vcf *v, uint32_t lo, uint32_t hi, uint
                 a = b + 1;
             }
         }
-        size_t a = 0;
-        for (int c = 0; c < 4; ++c) a = head.find('\t', a) + 1;   // ALT: column 5
-        const bool multi_alt = head.substr(a, head.find('\t', a) - a).find(',') != sv::npos;
+        const bool multi_alt = multi_alt_of(head);
         char val[40];
         for (uint32_t t = 0; t < N_INFO_TAGS; ++t) {
             if (!(tags >> t & 1)) continue;
@@ -543,6 +581,12 @@ int format_cohort(bool ploidy, const svjg_vcf *v, uint32_t lo, uint32_t hi, uint
             put(INFO_TAGS[t].id.data(), INFO_TAGS[t].id.size());
             put("=", 1);
             put(val, tag_value(val, t, gcount + G * j, ploidy, S, hwe ? hwe[j] : 0.0, exchet ? exchet[j] : 0.0, multi_alt));
+        }
+        if (post) {
+            if (!first) put(";", 1);
+            put("AF_EM=", 6);
+            if (multi_alt || af[j] != af[j]) put(".", 1);                 // NaN: no cell contributes
+            else put(val, size_t(snprintf(val, sizeof val, "%.6g", af[j])));
         }
         return len;
     };
@@ -577,10 +621,30 @@ int format_cohort(bool ploidy, const svjg_vcf *v, uint32_t lo, uint32_t hi, uint
         *o++ = ',';
         return put_i64(o, pl[3 * k + 2]);
     };
-    // the text of cell k (at most 136 bytes)
+    // with posteriors, the records whose GP and GQ are "." in every cell (ALT with a comma)
+    std::vector<uint8_t> multi(post ? n : 0);
+    for (size_t j = 0; j < multi.size(); ++j) multi[j] = multi_alt_of(sv(text + v->recs[lo + j].head_off, v->recs[lo + j].head_len));
+    // ":GP:GQ" of cell k: ":GP0,GP1,GP2:GQ" (haploid ":GP0,GP2:GQ") for a genotyped cell of ploidy 1 or 2, else ":.:."
+    auto put_post = [&](char *o, size_t k) {
+        if (!(flags[k] & SVJG_GT_GENOTYPED) || gt[k] == SVJG_GT_NO_CALL || multi[k / S]) return put_mem(o, ":.:.", 4);
+        *o++ = ':';
+        o = put_prob(o, gp[3 * k]);
+        *o++ = ',';
+        if (gt[k] < SVJG_GT_HAP_REF) {
+            o = put_prob(o, gp[3 * k + 1]);
+            *o++ = ',';
+        }
+        o = put_prob(o, gp[3 * k + 2]);
+        *o++ = ':';
+        if (gq[k] == SVJG_POST_GQ_NONE) *o++ = '.';
+        else o = put_u64(o, gq[k]);
+        return o;
+    };
+    // the text of cell k (at most 136 bytes, and 178 with posteriors: 3 GP values of up to 12 characters)
     auto put_sample = [&](char *o, size_t k) {
-        if (ploidy && gt[k] >= SVJG_GT_HAP_REF) return put_haploid(o, k);
-        if (flags[k] & SVJG_GT_GENOTYPED) {
+        if (ploidy && gt[k] >= SVJG_GT_HAP_REF) {
+            o = put_haploid(o, k);
+        } else if (flags[k] & SVJG_GT_GENOTYPED) {
             o = put_mem(o, GT_TEXT[gt[k]], 3);
             o = put_dp_ad(o, k);
             o = put_i64(o, pl[3 * k]);
@@ -591,11 +655,11 @@ int format_cohort(bool ploidy, const svjg_vcf *v, uint32_t lo, uint32_t hi, uint
         } else {
             o = put_mem(o, "./.:0:0,0:.,.,.", 15);
         }
-        return o;
+        return post ? put_post(o, k) : o;
     };
     // what follows the head of record lo + j: the FORMAT column and one column per sample
     auto put_columns = [&](char *o, size_t j) {
-        o = put_mem(o, "\tGT:DP:AD:PL", 12);
+        o = put_mem(o, fmt_col.data(), fmt_col.size());
         for (size_t s = 0; s < S; ++s) {
             *o++ = '\t';
             o = put_sample(o, j * S + s);
@@ -603,22 +667,37 @@ int format_cohort(bool ploidy, const svjg_vcf *v, uint32_t lo, uint32_t hi, uint
         *o++ = '\n';
         return o;
     };
+    unsigned hw_thr = std::max(1u, std::min(16u, std::thread::hardware_concurrency()));
     // where every record starts: its head is copied as it is, the cells are rendered once to learn their
-    // length (cheap next to the copies); then the records are filled in by several threads
+    // length (by several threads, over ranges of records); then the records are filled in by several threads
     std::vector<uint64_t> at(n + 1, 0), genotyped(S, 0);
     {
-        char tmp[160];
+        const unsigned m_thr = n_cells < (1u << 18) || n < 64 ? 1 : hw_thr;
+        std::vector<uint64_t> cells_len(n, 0), gen(size_t(m_thr) * S, 0);
+        auto measure = [&](unsigned p) {
+            char tmp[256];
+            uint64_t *g = gen.data() + size_t(p) * S;
+            for (size_t j = n * p / m_thr; j < n * (p + 1) / m_thr; ++j) {
+                uint64_t len = 0;
+                for (size_t s = 0; s < S; ++s) {
+                    const size_t k = j * S + s;
+                    g[s] += (flags[k] & SVJG_GT_GENOTYPED) && !(ploidy && gt[k] == SVJG_GT_NO_CALL);
+                    len += uint64_t(put_sample(tmp, k) - tmp);
+                }
+                cells_len[j] = len;
+            }
+        };
+        std::vector<std::thread> pool;
+        for (unsigned p = 1; p < m_thr; ++p) pool.emplace_back(measure, p);
+        measure(0);
+        for (auto &th : pool) th.join();
+        for (size_t q = 0; q < gen.size(); ++q) genotyped[q % S] += gen[q];
         size_t h = h_lo;
         uint64_t pos = 0;
         for (size_t j = 0; j < n; ++j) {
             while (h < h_hi && v->hdrs[h].before <= lo + j) pos += hdr_len(v->hdrs[h++]);
             at[j] = pos;
-            pos += put_head(nullptr, j) + 13 + S;
-            for (size_t s = 0; s < S; ++s) {
-                const size_t k = j * S + s;
-                genotyped[s] += (flags[k] & SVJG_GT_GENOTYPED) && !(ploidy && gt[k] == SVJG_GT_NO_CALL);
-                pos += uint64_t(put_sample(tmp, k) - tmp);
-            }
+            pos += put_head(nullptr, j) + fmt_col.size() + 1 + S + cells_len[j];   // FORMAT, tabs, '\n', cells
         }
         at[n] = pos;
     }
@@ -645,7 +724,7 @@ int format_cohort(bool ploidy, const svjg_vcf *v, uint32_t lo, uint32_t hi, uint
         }
     };
     const uint64_t body = at[n];
-    unsigned n_thr = std::max(1u, std::min(16u, std::thread::hardware_concurrency()));
+    unsigned n_thr = hw_thr;
     if (body < (4u << 20) || n < 64) n_thr = 1;
     if (n_thr == 1) {
         fill(0, n);
@@ -680,8 +759,8 @@ extern "C" int svjg_vcf_format_cohort_tags(const svjg_vcf *v, uint32_t lo, uint3
                                            uint64_t names_len, const uint8_t *gt, const uint8_t *flags, const uint32_t *ad2,
                                            const int64_t *pl, uint32_t tags, const uint32_t *gcount, const double *hwe,
                                            const double *exchet, char **out, uint64_t *out_len, uint64_t *n_genotyped) {
-    return format_cohort(false, v, lo, hi, n_samples, names, names_len, gt, flags, ad2, pl, tags, gcount, hwe, exchet, out,
-                         out_len, n_genotyped);
+    return svjg_vcf_format_cohort_post(v, lo, hi, n_samples, names, names_len, gt, flags, ad2, pl, 0, tags, gcount, hwe,
+                                       exchet, nullptr, nullptr, nullptr, out, out_len, n_genotyped);
 }
 
 extern "C" int svjg_vcf_format_cohort_ploidy(const svjg_vcf *v, uint32_t lo, uint32_t hi, uint32_t n_samples,
@@ -689,8 +768,19 @@ extern "C" int svjg_vcf_format_cohort_ploidy(const svjg_vcf *v, uint32_t lo, uin
                                              const uint32_t *ad2, const int64_t *pl, uint32_t tags, const uint32_t *gcount,
                                              const double *hwe, const double *exchet, char **out, uint64_t *out_len,
                                              uint64_t *n_genotyped) {
-    return format_cohort(true, v, lo, hi, n_samples, names, names_len, gt, flags, ad2, pl, tags, gcount, hwe, exchet, out,
-                         out_len, n_genotyped);
+    return svjg_vcf_format_cohort_post(v, lo, hi, n_samples, names, names_len, gt, flags, ad2, pl, 1, tags, gcount, hwe,
+                                       exchet, nullptr, nullptr, nullptr, out, out_len, n_genotyped);
+}
+
+extern "C" int svjg_vcf_format_cohort_post(const svjg_vcf *v, uint32_t lo, uint32_t hi, uint32_t n_samples,
+                                           const char *names, uint64_t names_len, const uint8_t *gt, const uint8_t *flags,
+                                           const uint32_t *ad2, const int64_t *pl, uint32_t ploidy, uint32_t tags,
+                                           const uint32_t *gcount, const double *hwe, const double *exchet, const double *af,
+                                           const double *gp, const uint8_t *gq, char **out, uint64_t *out_len,
+                                           uint64_t *n_genotyped) {
+    if (ploidy > 1) return set_error(SVJG_E_ARG, "svjg_vcf_format: ploidy must be 0 or 1");
+    return format_cohort(ploidy != 0, v, lo, hi, n_samples, names, names_len, gt, flags, ad2, pl, tags, gcount, hwe, exchet,
+                         af, gp, gq, out, out_len, n_genotyped);
 }
 
 extern "C" int svjg_vcf_format_cohort(const svjg_vcf *v, uint32_t lo, uint32_t hi, uint32_t n_samples, const char *names,

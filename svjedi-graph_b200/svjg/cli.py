@@ -279,6 +279,10 @@ def cohort_main(argv=None):
                          "A record's CHROM and POS decide its ploidy. Needs --sample-sex")
     ap.add_argument("--sample-sex", metavar="<file>", default=None,
                     help="NAME SEX per line, every sample once (other names are ignored). Needs --ploidy-file")
+    ap.add_argument("--posteriors", action="store_true",
+                    help="estimate each SV's allele frequency by EM over all samples' genotype likelihoods (INFO "
+                         "AF_EM) and write each cell's genotype posteriors under the Hardy-Weinberg prior at it "
+                         "(FORMAT GP) and the phred confidence of its GT call (FORMAT GQ, at most 99); GT is unchanged")
     args = ap.parse_args(argv)
     import os
     if not args.prefix:
@@ -350,7 +354,7 @@ def cohort_main(argv=None):
         fd, tmp = tempfile.mkstemp(prefix="." + os.path.basename(out_path) + ".", dir=os.path.dirname(out_path))
         with os.fdopen(fd, "wb") as out:
             _, n_gt = cohort.genotype_cohort_vcf(tables, co, vcf, names, args.minsupport, args.err, out=out,
-                                                 info_tags=info_tags, ploidy=ploidy)
+                                                 info_tags=info_tags, ploidy=ploidy, posteriors=args.posteriors)
         os.replace(tmp, out_path)
         tmp = None
         _lap("genotypes + VCF written")

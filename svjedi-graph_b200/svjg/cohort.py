@@ -14,6 +14,7 @@ import numpy as np
 from . import alnfilter, capi, genotype
 
 CELL_BYTES = 24 + 1 + 8 + 1          # pl, gt, ad2, flags of one cell
+POST_CELL_BYTES = 24 + 1             # gp, gq of one cell (genotype posteriors)
 BLOCK_BYTES = 256 << 20              # cell arrays of one block of records, at most
 # population INFO tags of --info-tags, in the order they are written: bit k of svjg_vcf_format_cohort_tags's mask
 INFO_TAGS = ("NS", "AN", "AC", "AF", "AC_Het", "AC_Hom", "F_MISSING", "HWE", "ExcHet")
@@ -47,6 +48,19 @@ def info_tags_mask(names):
             raise ValueError(f"unknown INFO tag {nm!r}")
         mask |= 1 << PLOIDY_INFO_TAGS.index(nm)
     return mask
+
+
+_phred_weights = None
+
+
+def phred_weights():
+    """T[k] = 10.0 ** (-k / 10) for k < capi.POST_PLW_N, the weight of a genotype whose PL is k above the cell's
+    smallest (svjg_cohort_posteriors).  Built by Python's own float power, so the device and the statement in the
+    tests use the same doubles; T underflows to 0.0 long before the last entry."""
+    global _phred_weights
+    if _phred_weights is None:
+        _phred_weights = np.array([10.0 ** (-k / 10) for k in range(capi.POST_PLW_N)], np.float64)
+    return _phred_weights
 
 
 def _table_lines(text):
@@ -204,9 +218,10 @@ class Cohort:
 class _Block:
     """Page-locked result arrays of one block of records: the copies from the device run at PCIe speed.  With
     ``n_records``, also the site statistics of that many records (svjg_cohort_site_stats, 32 B per record; with
-    ``ploidy``, svjg_cohort_site_stats_ploidy, 40 B)."""
+    ``ploidy``, svjg_cohort_site_stats_ploidy, 40 B).  With ``post_records``, the genotype posteriors of that many
+    records (svjg_cohort_posteriors: af, 8 B per record; gp and gq, 25 B per cell)."""
 
-    def __init__(self, n_cells, n_records=0, ploidy=False):
+    def __init__(self, n_cells, n_records=0, ploidy=False, post_records=0):
         n_cells = max(int(n_cells), 1)
         self._mem = [alnfilter.PinnedBytes(n_cells * b) for b in (24, 1, 8, 1)]
         self.pl = self._mem[0].array.view(np.int64).reshape(n_cells, 3)
@@ -220,6 +235,13 @@ class _Block:
             self.gcount = self._mem[4].array.view(np.uint32).reshape(n_records, g)
             self.hwe = self._mem[5].array.view(np.float64)
             self.exchet = self._mem[6].array.view(np.float64)
+        if post_records:
+            mem = [alnfilter.PinnedBytes(b) for b in (int(post_records) * 8, n_cells * 24, n_cells)]
+            self._mem += mem
+            self.af = mem[0].array.view(np.float64)
+            self.gp = mem[1].array.view(np.float64).reshape(n_cells, 3)
+            self.gq = mem[2].array
+        self.need = np.zeros(0, np.int64)           # the NEED_K cells the last _genotype_block patched
 
 
 def _genotype_block(cohort, idx, ty, min_support, e, blk, rclass=None):
@@ -250,6 +272,7 @@ def _genotype_block(cohort, idx, ty, min_support, e, blk, rclass=None):
                                                 ty[need // S], min_support, e)
         gt[need] = np.where(gt[need] >= capi.GT_HAP_REF, gt[need], g2)
         fl[need], ad[need], pl[need] = f2, a2, p2
+    blk.need = need
     return gt, fl, ad, pl
 
 
@@ -264,8 +287,25 @@ def _site_stats(cohort, n, blk, ploidy=False):
     return g, hw, ex
 
 
+def _posteriors(cohort, n, blk, iters=None):
+    """(af [n], gp [n * S][3], gq [n * S]) of the block _genotype_block genotyped last (svjg_cohort_posteriors), with
+    the PLs that block's NEED_K patch computed on the host sent to the device first.  ``iters``: a uint8 [n] array
+    that receives the EM steps per record."""
+    cells = n * cohort.n_samples
+    af, gp, gq = blk.af[:n], blk.gp[:cells], blk.gq[:cells]
+    need = blk.need
+    pcell = np.ascontiguousarray(need, np.uint32)
+    ppl = np.ascontiguousarray(blk.pl[need], np.int64)
+    T = phred_weights()
+    capi.check(capi.lib.svjg_cohort_posteriors(cohort._h, n, need.size, pcell.ctypes.data if need.size else None,
+                                               ppl.ctypes.data if need.size else None, T.ctypes.data, T.size,
+                                               af.ctypes.data, gp.ctypes.data, gq.ctypes.data,
+                                               None if iters is None else iters.ctypes.data))
+    return af, gp, gq
+
+
 def genotype_cohort_vcf(tables, cohort, vcf_bytes, names, min_support=genotype.MIN_SUPPORT, e=genotype.ERR, out=None,
-                        block_records=None, info_tags=(), ploidy=None):
+                        block_records=None, info_tags=(), ploidy=None, posteriors=False):
     """predict-genotype.py's decision_vcf for every sample of ``cohort``: the multi-sample VCF, whose column s is
     the SAMPLE column of sample s's single-sample VCF.  ``vcf_bytes``: the catalogue VCF's bytes (or lines, or a
     genotype.NativeVcf of them).
@@ -275,7 +315,9 @@ def genotype_cohort_vcf(tables, cohort, vcf_bytes, names, min_support=genotype.M
     names; their values are computed on the device from each block's genotypes (svjg_cohort_site_stats) and written
     into the INFO column, and their ##INFO lines in front of the ##FORMAT lines (svjg_vcf_format_cohort_tags).
     ``ploidy``: a PloidyRules for the samples of ``names``; the cells are called with their ploidy and the text is
-    that of svjg_vcf_format_cohort_ploidy (PL Number=G, AC_Hemi available)."""
+    that of svjg_vcf_format_cohort_ploidy (PL Number=G, AC_Hemi available).  ``posteriors``: the allele frequency of
+    every record by EM over its cells' likelihoods (INFO AF_EM), and each cell's GP and GQ under the Hardy-Weinberg
+    prior at it (svjg_cohort_posteriors, svjg_vcf_format_cohort_post); GT stays the likelihood call."""
     S = cohort.n_samples
     mask = info_tags_mask(info_tags)
     if len(names) != S:
@@ -294,8 +336,10 @@ def genotype_cohort_vcf(tables, cohort, vcf_bytes, names, min_support=genotype.M
         rclass, table = ploidy.record_classes(v)
         capi.check(capi.lib.svjg_cohort_set_ploidy(cohort._h, table.shape[0], table.shape[1], table.ctypes.data,
                                                    ploidy.sex_index.ctypes.data))
-    step = int(block_records) if block_records else max(1, BLOCK_BYTES // (CELL_BYTES * S))
-    blk = _Block(min(step, max(n, 1)) * S, min(step, max(n, 1)) if mask else 0, ploidy is not None)
+    cell_bytes = CELL_BYTES + (POST_CELL_BYTES if posteriors else 0)
+    step = int(block_records) if block_records else max(1, BLOCK_BYTES // (cell_bytes * S))
+    rows = min(step, max(n, 1))
+    blk = _Block(rows * S, rows if mask else 0, ploidy is not None, rows if posteriors else 0)
     if not 0 < e < 1:
         # math.log10 raises inside likelihood() only once a record passes the gate (predict-genotype.py:216), as in
         # genotype.genotype_host: a cohort in which no cell passes it is written with "./." everywhere.  A cell of
@@ -317,9 +361,15 @@ def genotype_cohort_vcf(tables, cohort, vcf_bytes, names, min_support=genotype.M
         if mask:
             site = [a.ctypes.data for a in _site_stats(cohort, hi - lo, blk, rclass is not None)]
         buf, n_out = C.c_void_p(), C.c_uint64()
-        fmt = capi.lib.svjg_vcf_format_cohort_ploidy if rclass is not None else capi.lib.svjg_vcf_format_cohort_tags
-        capi.check(fmt(v._h, lo, hi, S, joined, len(joined), gt.ctypes.data, fl.ctypes.data, ad.ctypes.data,
-                       pl.ctypes.data, mask, *site, C.byref(buf), C.byref(n_out), n_gt.ctypes.data))
+        if posteriors:
+            post = [a.ctypes.data for a in _posteriors(cohort, hi - lo, blk)]
+            capi.check(capi.lib.svjg_vcf_format_cohort_post(
+                v._h, lo, hi, S, joined, len(joined), gt.ctypes.data, fl.ctypes.data, ad.ctypes.data, pl.ctypes.data,
+                int(rclass is not None), mask, *site, *post, C.byref(buf), C.byref(n_out), n_gt.ctypes.data))
+        else:
+            fmt = capi.lib.svjg_vcf_format_cohort_ploidy if rclass is not None else capi.lib.svjg_vcf_format_cohort_tags
+            capi.check(fmt(v._h, lo, hi, S, joined, len(joined), gt.ctypes.data, fl.ctypes.data, ad.ctypes.data,
+                           pl.ctypes.data, mask, *site, C.byref(buf), C.byref(n_out), n_gt.ctypes.data))
         try:
             if out is not None:
                 if n_out.value:
