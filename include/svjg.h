@@ -319,6 +319,29 @@ int svjg_cohort_site_stats_ploidy(svjg_cohort *c, uint32_t n, uint32_t *gcount, 
 int svjg_cohort_posteriors(svjg_cohort *c, uint32_t n, uint32_t n_patch, const uint32_t *patch_cell, const int64_t *patch_pl,
                            const double *plw, uint32_t plw_n, double *af, double *gp, uint8_t *gq, uint8_t *iters);
 
+/* Sample QC and relatedness (DESIGN.md §8a): per-sample genotype counts and pairwise KING-robust counts over the final
+ * gt codes of every block, kept on the device for the whole run.
+ *   svjg_cohort_qc_begin    allocates and zeroes the histogram and, when want_pairs, the bit planes of n_words words
+ *                           (32 records each) per sample; a block of n records takes ceil(n / 32) words, starting a new
+ *                           word.  SVJG_E_ARG when want_pairs and n_samples > SVJG_QC_MAX_PAIR_SAMPLES.  Calling it again
+ *                           starts over.
+ *   svjg_cohort_qc_add      adds the block of the last svjg_cohort_genotype(_ploidy) call (n must be its record count,
+ *                           each block once, within n_words).  Asynchronous: its errors show at the next call.
+ *   svjg_cohort_qc_sample_counts  out [n_samples][5][8] u32: rows ALL, DEL, INS, INV, BND (svtype & 0x3F = 0..3; other
+ *                           types count in ALL only), columns the gt codes 0-7.  Synchronous.
+ *   svjg_cohort_qc_planes   out [3][n_samples][n_words] u32: planes C (codes 0-2), H (code 1), A (code 2); bit r of
+ *                           word w is record 32 w + r of the block that took word w; other bits 0.  Synchronous.
+ *   svjg_cohort_relatedness out [S (S - 1) / 2][5] u32, pair (i < j) at i (2 S - i - 1) / 2 + j - i - 1, i major:
+ *                           over the records where both cells are diploid and called (codes 0-2), NSV = such records,
+ *                           HET1 / HET2 = those where i / j is 0/1, HETHET = both 0/1, IBS0 = one 0/0 and the other
+ *                           1/1.  Needs want_pairs.  Synchronous. */
+#define SVJG_QC_MAX_PAIR_SAMPLES 16384
+int svjg_cohort_qc_begin(svjg_cohort *c, uint32_t n_words, int want_pairs);
+int svjg_cohort_qc_add(svjg_cohort *c, uint32_t n);
+int svjg_cohort_qc_sample_counts(svjg_cohort *c, uint32_t *out);
+int svjg_cohort_qc_planes(svjg_cohort *c, uint32_t *out);
+int svjg_cohort_relatedness(svjg_cohort *c, uint32_t *out);
+
 /* Page-locked host memory (cudaHostAlloc) for file buffers and results: copies to and from it run
  * at PCIe speed.  For callers that do not want a tensor library just to pin memory. */
 int svjg_host_alloc(uint64_t bytes, void **out);
@@ -476,6 +499,14 @@ int svjg_vcf_format_cohort_post(const svjg_vcf *v, uint32_t lo, uint32_t hi, uin
                                 const int64_t *pl, uint32_t ploidy, uint32_t tags, const uint32_t *gcount,
                                 const double *hwe, const double *exchet, const double *af, const double *gp,
                                 const uint8_t *gq, char **out, uint64_t *out_len, uint64_t *n_genotyped);
+/* svjg_format_relatedness: the lines of rows i in [i_lo, i_hi) of the relatedness table from svjg_cohort_relatedness's
+ * counts `pairs` (the whole array) and the names joined by '\t' (exactly n_samples of them), with the header line
+ * "#ID1 ID2 NSV HET1 HET2 HETHET IBS0 KINSHIP" (tab-separated) when i_lo == 0.  One line per pair i < j, i major:
+ * ID1 ID2 and the five counts, then KINSHIP = (HETHET - 2 IBS0) / (HET1 + HET2) as one double division of the exact
+ * integers, "%.6g", "." when HET1 + HET2 = 0.  use_min != 0: only pairs whose KINSHIP is >= min_kinship (finite) are
+ * written, "." ones never.  The pieces of consecutive row ranges joined are the whole table. */
+int svjg_format_relatedness(uint32_t n_samples, const char *names, uint64_t names_len, const uint32_t *pairs, uint32_t i_lo,
+                            uint32_t i_hi, int use_min, double min_kinship, char **out, uint64_t *out_len);
 void svjg_buffer_free(char *p);
 
 /* ---- output (host) ------------------------------------------------------------

@@ -382,6 +382,7 @@ extern "C" void svjg_cohort_free(svjg_cohort *c) {
     if (c->d_ploidy) cudaFree(c->d_ploidy);
     if (c->d_plw) cudaFree(c->d_plw);
     if (c->d_post) cudaFree(c->d_post);
+    if (c->d_qc) cudaFree(c->d_qc);
     if (c->stream) cudaStreamDestroy(c->stream);
     delete c;
 }

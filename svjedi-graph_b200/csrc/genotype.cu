@@ -607,6 +607,145 @@ __global__ void cohort_patch_kernel(const uint32_t *__restrict__ cell, const int
     flags[c] &= uint8_t(~SVJG_GT_NEED_K);
 }
 
+// ---- sample QC and relatedness (DESIGN.md §8a, "Sample QC and relatedness") ----
+// Pack: one thread per (sample, QC_PACK_WORDS words of 32 records) of the block the last cohort genotype call left on
+// the device.  Bit r of word w of a sample's planes is record 32 w + r of the block: C = diploid called (codes 0-2),
+// H = 0/1, A = 1/1; the block's words start at word w0 of the row.  The histogram cell (type row, code) of the thread's
+// cells is counted in shared memory (column threadIdx.x: no two threads share a bank) and added to hist [S][5][8]
+// with one atomic per non-zero partial; internal row 4 holds the records whose type is not DEL / INS / INV / BND,
+// which count in the ALL row only.
+constexpr int QC_PACK_THREADS = 128;
+constexpr uint32_t QC_PACK_WORDS = 8;
+__global__ void __launch_bounds__(QC_PACK_THREADS)
+cohort_qc_pack_kernel(const uint8_t *__restrict__ gt, const uint8_t *__restrict__ ty, uint32_t n, uint32_t S,
+                      uint32_t *__restrict__ hist, uint32_t *__restrict__ planes, size_t stride, uint32_t w0) {
+    __shared__ uint32_t cnt[5 * 8][QC_PACK_THREADS];
+    const uint32_t s = blockIdx.x * QC_PACK_THREADS + threadIdx.x;
+    if (s >= S) return;                                  // only the thread's own column is used: no barrier
+#pragma unroll
+    for (int k = 0; k < 5 * 8; ++k) cnt[k][threadIdx.x] = 0;
+    const uint32_t n_words = (n + 31) / 32;
+    for (uint32_t wlo = blockIdx.y * QC_PACK_WORDS; wlo < n_words; wlo += gridDim.y * QC_PACK_WORDS) {
+        const uint32_t whi = min(wlo + QC_PACK_WORDS, n_words);
+        for (uint32_t w = wlo; w < whi; ++w) {
+            uint32_t C = 0, H = 0, A = 0;
+            const uint32_t r0 = 32 * w, r1 = min(r0 + 32, n);
+            for (uint32_t r = r0; r < r1; ++r) {
+                const uint32_t g = gt[size_t(r) * S + s], t = ty[r] & 0x3F;
+                ++cnt[(t <= 3 ? t : 4) * 8 + g][threadIdx.x];
+                const uint32_t bit = 1u << (r - r0);
+                C |= g <= 2 ? bit : 0u;
+                H |= g == 1 ? bit : 0u;
+                A |= g == 2 ? bit : 0u;
+            }
+            if (planes) {
+                const size_t o = size_t(s) * stride + w0 + w, plane = size_t(S) * stride;
+                planes[o] = C;
+                planes[o + plane] = H;
+                planes[o + 2 * plane] = A;
+            }
+        }
+    }
+    uint32_t *h = hist + size_t(s) * 40;
+    for (int g = 0; g < 8; ++g) {
+        uint32_t all = 0;
+        for (int t = 0; t < 5; ++t) {
+            const uint32_t v = cnt[t * 8 + g][threadIdx.x];
+            all += v;
+            if (t < 4 && v) atomicAdd(h + (1 + t) * 8 + g, v);
+        }
+        if (all) atomicAdd(h + g, all);
+    }
+}
+
+// Pairs: the upper triangle of the S x S grid in tiles of PAIR_T x PAIR_T samples, tile (bi, bj) with bi <= bj at
+// linear index bj (bj + 1) / 2 + bi.  A K slab of PAIR_KW words of the three planes of both sample ranges is staged in
+// shared memory ([side][plane][word][sample]); each thread of a 16 x 16 grid owns the 4 x 4 pairs (i0 + 4 ty + a,
+// j0 + 4 tx + b) and keeps five counters per pair.  Per word, with R = C & ~H & ~A (= C ^ H ^ A: H and A are disjoint
+// subsets of C): NSV += popc(Ci & Cj), HET1 += popc(Hi & Cj), HET2 += popc(Hj & Ci), HETHET += popc(Hi & Hj),
+// IBS0 += popc((Ai & Rj) | (Ri & Aj)).  Pair (i < j) goes to out[5 p], p = i (2 S - i - 1) / 2 + j - i - 1.
+constexpr uint32_t PAIR_T = 64;
+constexpr uint32_t PAIR_KW = 16;
+constexpr int PAIR_THREADS = 256;
+__global__ void __launch_bounds__(PAIR_THREADS)
+cohort_pair_kernel(const uint32_t *__restrict__ planes, uint32_t S, size_t stride, uint32_t n_slabs,
+                   uint32_t *__restrict__ out) {
+    __shared__ __align__(16) uint32_t sm[2][3][PAIR_KW][PAIR_T];
+    const uint32_t t = blockIdx.x;
+    uint32_t bj = uint32_t((sqrt(8.0 * t + 1.0) - 1.0) / 2.0);
+    while (bj * (bj + 1) / 2 > t) --bj;
+    while ((bj + 1) * (bj + 2) / 2 <= t) ++bj;
+    const uint32_t bi = t - bj * (bj + 1) / 2;
+    const uint32_t i0 = bi * PAIR_T, j0 = bj * PAIR_T;
+    const uint32_t tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
+    const uint32_t lr = threadIdx.x >> 2, lq = threadIdx.x & 3;           // loader: sample lr, words 4 lq .. 4 lq + 3
+    const size_t plane = size_t(S) * stride;
+    uint32_t cnt[4][4][5];
+#pragma unroll
+    for (int a = 0; a < 4; ++a)
+#pragma unroll
+        for (int b = 0; b < 4; ++b)
+#pragma unroll
+            for (int q = 0; q < 5; ++q) cnt[a][b][q] = 0;
+    for (uint32_t slab = 0; slab < n_slabs; ++slab) {
+#pragma unroll
+        for (int side = 0; side < 2; ++side) {
+            const uint32_t row = (side ? j0 : i0) + lr;
+#pragma unroll
+            for (int p = 0; p < 3; ++p) {
+                uint4 v = make_uint4(0, 0, 0, 0);
+                if (row < S) v = __ldg(reinterpret_cast<const uint4 *>(planes + p * plane + size_t(row) * stride +
+                                                                       size_t(slab) * PAIR_KW + 4 * lq));
+                sm[side][p][4 * lq][lr] = v.x;
+                sm[side][p][4 * lq + 1][lr] = v.y;
+                sm[side][p][4 * lq + 2][lr] = v.z;
+                sm[side][p][4 * lq + 3][lr] = v.w;
+            }
+        }
+        __syncthreads();
+#pragma unroll 2
+        for (uint32_t k = 0; k < PAIR_KW; ++k) {
+            const uint4 ci = *reinterpret_cast<const uint4 *>(&sm[0][0][k][4 * ty]);
+            const uint4 hi = *reinterpret_cast<const uint4 *>(&sm[0][1][k][4 * ty]);
+            const uint4 ai = *reinterpret_cast<const uint4 *>(&sm[0][2][k][4 * ty]);
+            const uint4 cj = *reinterpret_cast<const uint4 *>(&sm[1][0][k][4 * tx]);
+            const uint4 hj = *reinterpret_cast<const uint4 *>(&sm[1][1][k][4 * tx]);
+            const uint4 aj = *reinterpret_cast<const uint4 *>(&sm[1][2][k][4 * tx]);
+            const uint32_t Ci[4] = {ci.x, ci.y, ci.z, ci.w}, Hi[4] = {hi.x, hi.y, hi.z, hi.w},
+                           Ai[4] = {ai.x, ai.y, ai.z, ai.w};
+            const uint32_t Cj[4] = {cj.x, cj.y, cj.z, cj.w}, Hj[4] = {hj.x, hj.y, hj.z, hj.w},
+                           Aj[4] = {aj.x, aj.y, aj.z, aj.w};
+#pragma unroll
+            for (int a = 0; a < 4; ++a) {
+                const uint32_t Ri = Ci[a] ^ Hi[a] ^ Ai[a];
+#pragma unroll
+                for (int b = 0; b < 4; ++b) {
+                    const uint32_t Rj = Cj[b] ^ Hj[b] ^ Aj[b];
+                    cnt[a][b][0] += __popc(Ci[a] & Cj[b]);
+                    cnt[a][b][1] += __popc(Hi[a] & Cj[b]);
+                    cnt[a][b][2] += __popc(Hj[b] & Ci[a]);
+                    cnt[a][b][3] += __popc(Hi[a] & Hj[b]);
+                    cnt[a][b][4] += __popc((Ai[a] & Rj) | (Ri & Aj[b]));
+                }
+            }
+        }
+        __syncthreads();
+    }
+#pragma unroll
+    for (int a = 0; a < 4; ++a) {
+        const uint32_t i = i0 + 4 * ty + a;
+#pragma unroll
+        for (int b = 0; b < 4; ++b) {
+            const uint32_t j = j0 + 4 * tx + b;
+            if (i < j && j < S) {
+                uint32_t *o = out + 5 * (uint64_t(i) * (2 * uint64_t(S) - i - 1) / 2 + (j - i - 1));
+#pragma unroll
+                for (int q = 0; q < 5; ++q) o[q] = cnt[a][b][q];
+            }
+        }
+    }
+}
+
 }  // namespace
 
 extern "C" int svjg_genotype_device(const uint32_t *d_counts, const uint32_t *d_sv_index, const uint8_t *d_svtype,
@@ -718,6 +857,7 @@ int cohort_genotype(const char *fn, svjg_cohort *c, const uint32_t *sv_index, co
     const std::string f = fn;
     if (!c) return svjg::set_error(SVJG_E_ARG, f + ": NULL cohort");
     c->blk_n = 0;                          // set again once this block's cells are complete
+    c->blk_qc = false;
     if (n == 0) return SVJG_OK;
     if (!sv_index || !svtype || !lut || !pl || !gt || !ad2 || !flags)
         return svjg::set_error(SVJG_E_ARG, f + ": NULL argument");
@@ -780,6 +920,7 @@ int cohort_genotype(const char *fn, svjg_cohort *c, const uint32_t *sv_index, co
     c->blk_gt = o_gt;
     c->blk_pl = o_pl;
     c->blk_fl = o_fl;
+    c->blk_ty = o_ty;
     return SVJG_OK;
 }
 
@@ -914,6 +1055,98 @@ extern "C" int svjg_cohort_posteriors(svjg_cohort *c, uint32_t n, uint32_t n_pat
     SVJG_CUDA(cudaMemcpyAsync(&bad, d_bad, 4, cudaMemcpyDeviceToHost, st));
     SVJG_CUDA(cudaStreamSynchronize(st));
     if (bad) return svjg::set_error(SVJG_E_ARG, f + ": a contributing cell still has SVJG_GT_NEED_K (no PL patched in)");
+    return SVJG_OK;
+}
+
+// Sample QC and relatedness: resident histogram and bit planes, filled block by block, read once at the end.
+extern "C" int svjg_cohort_qc_begin(svjg_cohort *c, uint32_t n_words, int want_pairs) {
+    const std::string f = "svjg_cohort_qc_begin";
+    if (!c) return svjg::set_error(SVJG_E_ARG, f + ": NULL cohort");
+    if (want_pairs && c->n_samples > SVJG_QC_MAX_PAIR_SAMPLES)
+        return svjg::set_error(SVJG_E_ARG, f + ": relatedness takes at most SVJG_QC_MAX_PAIR_SAMPLES samples");
+    SVJG_CUDA(cudaSetDevice(c->t->device));
+    if (c->d_qc) SVJG_CUDA(cudaFree(c->d_qc));
+    c->d_qc = nullptr;
+    c->qc_on = false;
+    const size_t S = c->n_samples, stride = (size_t(n_words) + PAIR_KW - 1) / PAIR_KW * PAIR_KW;
+    const size_t words = S * 40 + (want_pairs ? 3 * S * stride : 0);
+    SVJG_CUDA(cudaMalloc(&c->d_qc, words * 4));
+    SVJG_CUDA(cudaMemset(c->d_qc, 0, words * 4));
+    c->qc_words = n_words;
+    c->qc_used = 0;
+    c->qc_stride = stride;
+    c->qc_pairs = want_pairs != 0;
+    c->qc_on = true;
+    return SVJG_OK;
+}
+
+extern "C" int svjg_cohort_qc_add(svjg_cohort *c, uint32_t n) {
+    const std::string f = "svjg_cohort_qc_add";
+    if (!c) return svjg::set_error(SVJG_E_ARG, f + ": NULL cohort");
+    if (!c->qc_on) return svjg::set_error(SVJG_E_ARG, f + ": no svjg_cohort_qc_begin");
+    if (n != c->blk_n)
+        return svjg::set_error(SVJG_E_ARG, f + ": n is not the record count of the last svjg_cohort_genotype call");
+    if (n == 0) return SVJG_OK;
+    if (c->blk_qc) return svjg::set_error(SVJG_E_ARG, f + ": the block of the last genotype call was added already");
+    const uint32_t words = (n + 31) / 32;
+    if (uint64_t(c->qc_used) + words > c->qc_words)
+        return svjg::set_error(SVJG_E_ARG, f + ": more words than svjg_cohort_qc_begin's n_words");
+    SVJG_CUDA(cudaSetDevice(c->t->device));
+    const uint32_t S = c->n_samples;
+    const dim3 grid((S + QC_PACK_THREADS - 1) / QC_PACK_THREADS, std::min<uint32_t>((words + QC_PACK_WORDS - 1) / QC_PACK_WORDS, 65535));
+    cohort_qc_pack_kernel<<<grid, QC_PACK_THREADS, 0, c->stream>>>(c->d_blk + c->blk_gt, c->d_blk + c->blk_ty, n, S, c->d_qc,
+                                                                   c->qc_pairs ? c->d_qc + size_t(S) * 40 : nullptr,
+                                                                   c->qc_stride, c->qc_used);
+    SVJG_CUDA(cudaGetLastError());
+    c->qc_used += words;
+    c->blk_qc = true;
+    return SVJG_OK;
+}
+
+extern "C" int svjg_cohort_qc_sample_counts(svjg_cohort *c, uint32_t *out) {
+    if (!c || !out) return svjg::set_error(SVJG_E_ARG, "svjg_cohort_qc_sample_counts: NULL argument");
+    if (!c->qc_on) return svjg::set_error(SVJG_E_ARG, "svjg_cohort_qc_sample_counts: no svjg_cohort_qc_begin");
+    SVJG_CUDA(cudaSetDevice(c->t->device));
+    SVJG_CUDA(cudaMemcpyAsync(out, c->d_qc, size_t(c->n_samples) * 40 * 4, cudaMemcpyDeviceToHost, c->stream));
+    SVJG_CUDA(cudaStreamSynchronize(c->stream));
+    return SVJG_OK;
+}
+
+extern "C" int svjg_cohort_qc_planes(svjg_cohort *c, uint32_t *out) {
+    const std::string f = "svjg_cohort_qc_planes";
+    if (!c || !out) return svjg::set_error(SVJG_E_ARG, f + ": NULL argument");
+    if (!c->qc_on || !c->qc_pairs) return svjg::set_error(SVJG_E_ARG, f + ": no svjg_cohort_qc_begin with want_pairs");
+    if (c->qc_words == 0) return SVJG_OK;
+    SVJG_CUDA(cudaSetDevice(c->t->device));
+    SVJG_CUDA(cudaMemcpy2DAsync(out, size_t(c->qc_words) * 4, c->d_qc + size_t(c->n_samples) * 40, c->qc_stride * 4,
+                                size_t(c->qc_words) * 4, 3 * size_t(c->n_samples), cudaMemcpyDeviceToHost, c->stream));
+    SVJG_CUDA(cudaStreamSynchronize(c->stream));
+    return SVJG_OK;
+}
+
+extern "C" int svjg_cohort_relatedness(svjg_cohort *c, uint32_t *out) {
+    const std::string f = "svjg_cohort_relatedness";
+    if (!c) return svjg::set_error(SVJG_E_ARG, f + ": NULL cohort");
+    if (!c->qc_on || !c->qc_pairs) return svjg::set_error(SVJG_E_ARG, f + ": no svjg_cohort_qc_begin with want_pairs");
+    const uint64_t S = c->n_samples, n_pairs = S * (S - 1) / 2;
+    if (n_pairs == 0) return SVJG_OK;
+    if (!out) return svjg::set_error(SVJG_E_ARG, f + ": NULL argument");
+    SVJG_CUDA(cudaSetDevice(c->t->device));
+    cudaStream_t st = c->stream;
+    uint32_t *d_out = nullptr;
+    SVJG_CUDA(cudaMallocAsync(reinterpret_cast<void **>(&d_out), n_pairs * 20, st));
+    const uint64_t tiles = (S + PAIR_T - 1) / PAIR_T;
+    const uint32_t n_slabs = uint32_t((uint64_t(c->qc_used) + PAIR_KW - 1) / PAIR_KW);
+    cudaError_t e = cudaSuccess;
+    if (n_slabs == 0) e = cudaMemsetAsync(d_out, 0, n_pairs * 20, st);
+    else cohort_pair_kernel<<<uint32_t(tiles * (tiles + 1) / 2), PAIR_THREADS, 0, st>>>(c->d_qc + S * 40, uint32_t(S),
+                                                                                         c->qc_stride, n_slabs, d_out);
+    if (e == cudaSuccess) e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out, d_out, n_pairs * 20, cudaMemcpyDeviceToHost, st);
+    cudaFreeAsync(d_out, st);
+    const cudaError_t es = cudaStreamSynchronize(st);
+    if (e == cudaSuccess) e = es;
+    if (e != cudaSuccess) return svjg::cuda_fail(int(e), "svjg_cohort_relatedness");
     return SVJG_OK;
 }
 

@@ -46,6 +46,13 @@ struct svjg_cohort {
     uint32_t blk_n = 0;                       // records of the last block genotyped (0: none)
     size_t blk_gt = 0;                        // offset of its gt codes [blk_n][n_samples] in d_blk
     size_t blk_pl = 0, blk_fl = 0;            // offsets of its pl [blk_n][n_samples][3] and flags [blk_n][n_samples]
+    size_t blk_ty = 0;                        // offset of its svtype codes [blk_n]
+    bool blk_qc = false;                      // svjg_cohort_qc_add has packed the last block
+    uint32_t *d_qc = nullptr;                 // svjg_cohort_qc_begin: histogram [n_samples][5][8], then (qc_pairs) the
+                                              // bit planes C, H, A [3][n_samples][qc_stride]
+    uint32_t qc_words = 0, qc_used = 0;       // words of a plane row the caller announced, and packed so far
+    size_t qc_stride = 0;                     // qc_words rounded up to whole K slabs of the pair kernel
+    bool qc_on = false, qc_pairs = false;
     uint8_t *d_site = nullptr;                // site statistics of the last block (svjg_cohort_site_stats)
     size_t site_cap = 0;
     std::vector<double> plw;                  // host copy of what d_plw holds: T[k] = 10^(-k/10) (svjg_cohort_posteriors)

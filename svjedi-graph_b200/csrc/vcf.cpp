@@ -6,6 +6,7 @@
 // Only spellings whose Python meaning is reproduced exactly are accepted: a file with a non-ASCII
 // byte, or a POS/END of more than 18 digits, is answered with SVJG_E_UNSUPPORTED and the caller uses
 // the Python statement instead.
+#include <cmath>
 #include <cstdio>
 #include <algorithm>
 #include <cstring>
@@ -798,6 +799,77 @@ extern "C" int svjg_vcf_format(const svjg_vcf *v, const uint8_t *gt, const uint8
                                           &genotyped);
     if (rc == SVJG_OK && n_genotyped) *n_genotyped = genotyped;
     return rc;
+}
+
+extern "C" int svjg_format_relatedness(uint32_t n_samples, const char *names, uint64_t names_len, const uint32_t *pairs,
+                                       uint32_t i_lo, uint32_t i_hi, int use_min, double min_kinship, char **out,
+                                       uint64_t *out_len) {
+    const char *f = "svjg_format_relatedness";
+    if (!names || !out || !out_len) return set_error(SVJG_E_ARG, std::string(f) + ": NULL argument");
+    const size_t S = n_samples;
+    if (S == 0 || i_lo > i_hi || i_hi > S) return set_error(SVJG_E_ARG, std::string(f) + ": bad sample count or row range");
+    if (use_min && !std::isfinite(min_kinship)) return set_error(SVJG_E_ARG, std::string(f) + ": min_kinship must be finite");
+    std::vector<sv> name;
+    for (size_t a = 0;;) {
+        const size_t b = sv(names, names_len).find('\t', a);
+        name.emplace_back(names + a, (b == sv::npos ? names_len : b) - a);
+        if (b == sv::npos) break;
+        a = b + 1;
+    }
+    if (name.size() != S) return set_error(SVJG_E_ARG, std::string(f) + ": the names are not n_samples tab-separated names");
+    auto first_pair = [&](size_t i) { return i * (2 * S - i - 1) / 2; };   // pair (i, i + 1)
+    if (first_pair(i_hi) > first_pair(i_lo) && !pairs) return set_error(SVJG_E_ARG, std::string(f) + ": NULL argument");
+    // rows of about equal pair counts per thread, each rendered into its own piece
+    const uint64_t n_pairs = first_pair(i_hi) - first_pair(i_lo);
+    const unsigned n_thr = n_pairs < (1u << 16) ? 1 : std::max(1u, std::min(16u, std::thread::hardware_concurrency()));
+    std::vector<size_t> cut(n_thr + 1, i_lo);
+    for (unsigned p = 1; p < n_thr; ++p) {
+        size_t i = cut[p - 1];
+        while (i < i_hi && first_pair(i) - first_pair(i_lo) < n_pairs * p / n_thr) ++i;
+        cut[p] = i;
+    }
+    cut[n_thr] = i_hi;
+    std::vector<std::string> piece(n_thr);
+    auto render = [&](unsigned p) {
+        std::string &o = piece[p];
+        char num[96];
+        for (size_t i = cut[p]; i < cut[p + 1]; ++i) {
+            const uint32_t *c = pairs + 5 * first_pair(i);
+            for (size_t j = i + 1; j < S; ++j, c += 5) {
+                const uint64_t den = uint64_t(c[1]) + c[2];
+                const double kin = den ? double(int64_t(c[3]) - 2 * int64_t(c[4])) / double(den) : 0.0;
+                if (use_min && (!den || !(kin >= min_kinship))) continue;
+                o.append(name[i].data(), name[i].size());
+                o += '\t';
+                o.append(name[j].data(), name[j].size());
+                char *e = num;
+                for (int q = 0; q < 5; ++q) {
+                    *e++ = '\t';
+                    e = put_u64(e, c[q]);
+                }
+                *e++ = '\t';
+                if (den) e += snprintf(e, 32, "%.6g", kin);
+                else *e++ = '.';
+                *e++ = '\n';
+                o.append(num, size_t(e - num));
+            }
+        }
+    };
+    std::vector<std::thread> pool;
+    for (unsigned p = 1; p < n_thr; ++p) pool.emplace_back(render, p);
+    render(0);
+    for (auto &th : pool) th.join();
+    static const char HEADER[] = "#ID1\tID2\tNSV\tHET1\tHET2\tHETHET\tIBS0\tKINSHIP\n";
+    uint64_t total = i_lo == 0 ? sizeof HEADER - 1 : 0;
+    for (const auto &s : piece) total += s.size();
+    char *buf = (char *)malloc(total + 1);
+    if (!buf) return set_error(SVJG_E_NOMEM, std::string(f) + ": out of memory");
+    char *o = buf;
+    if (i_lo == 0) o = put_mem(o, HEADER, sizeof HEADER - 1);
+    for (const auto &s : piece) o = put_mem(o, s.data(), s.size());
+    *out = buf;
+    *out_len = total;
+    return SVJG_OK;
 }
 
 extern "C" void svjg_buffer_free(char *p) { free(p); }

@@ -14,6 +14,7 @@ GT_HAP_REF, GT_HAP_ALT, GT_HAP_MISSING, GT_NO_CALL = 4, 5, 6, 7        # gt code
 PLOIDY_MAX_CLASSES, PLOIDY_MAX_SEXES = 255, 64
 # svjg_cohort_posteriors: entries of the weight table, EM step cap and tolerance, GQ cap and "no GQ"
 POST_PLW_N, POST_MAX_ITERS, POST_TOL, POST_GQ_MAX, POST_GQ_NONE = 4096, 100, 1e-10, 99, 255
+QC_MAX_PAIR_SAMPLES = 16384                # svjg_cohort_qc_begin with want_pairs: at most this many samples
 NO_SV = 0xFFFFFFFF
 FLAG_EXACT_CHECKS, FLAG_FORCE_GENERAL = 1, 2
 TUNE_TILE_BYTES, TUNE_TILE_LINES, TUNE_SCAN_BLOCKS, TUNE_SCAN_ONLY, TUNE_POOL_UNITS = 1, 2, 3, 4, 5
@@ -104,6 +105,11 @@ def _load():
         "svjg_cohort_site_stats_ploidy": (C.c_int, [vp, C.c_uint32, u32p, f64p, f64p]),
         "svjg_cohort_posteriors": (C.c_int, [vp, C.c_uint32, C.c_uint32, u32p, i64p, f64p, C.c_uint32, f64p, f64p, u8p,
                                              u8p]),
+        "svjg_cohort_qc_begin": (C.c_int, [vp, C.c_uint32, C.c_int]),
+        "svjg_cohort_qc_add": (C.c_int, [vp, C.c_uint32]),
+        "svjg_cohort_qc_sample_counts": (C.c_int, [vp, u32p]),
+        "svjg_cohort_qc_planes": (C.c_int, [vp, u32p]),
+        "svjg_cohort_relatedness": (C.c_int, [vp, u32p]),
         "svjg_host_alloc": (C.c_int, [C.c_uint64, C.POINTER(C.c_void_p)]),
         "svjg_host_free": (C.c_int, [vp]),
         "svjg_host_register": (C.c_int, [vp, C.c_uint64]),
@@ -147,6 +153,8 @@ def _load():
         "svjg_vcf_format_cohort_post": (C.c_int, [vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_char_p, C.c_uint64, u8p,
                                                   u8p, u32p, i64p, C.c_uint32, C.c_uint32, u32p, f64p, f64p, f64p, f64p,
                                                   u8p, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64), u64p]),
+        "svjg_format_relatedness": (C.c_int, [C.c_uint32, C.c_char_p, C.c_uint64, u32p, C.c_uint32, C.c_uint32, C.c_int,
+                                              C.c_double, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]),
         "svjg_buffer_free": (None, [vp]),
         "svjg_emit_informative_json": (C.c_int, [vp, u8p, C.c_uint64, u32p, u64p, u32p, C.c_uint64, C.c_char_p]),
         "svjg_emit_informative_json_mem": (C.c_int, [vp, u8p, C.c_uint64, u32p, u64p, u32p, C.c_uint64,

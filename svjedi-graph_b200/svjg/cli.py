@@ -283,6 +283,15 @@ def cohort_main(argv=None):
                     help="estimate each SV's allele frequency by EM over all samples' genotype likelihoods (INFO "
                          "AF_EM) and write each cell's genotype posteriors under the Hardy-Weinberg prior at it "
                          "(FORMAT GP) and the phred confidence of its GT call (FORMAT GQ, at most 99); GT is unchanged")
+    ap.add_argument("--sample-qc", metavar="<file>", default=None,
+                    help="write a per-sample QC table: genotype counts, CALL_RATE and HET_HOM_RATIO for all records "
+                         "and per SVTYPE (DEL, INS, INV, BND); the VCF is unchanged")
+    ap.add_argument("--relatedness", metavar="<file>", default=None,
+                    help="write the KING-robust kinship of every pair of samples (NSV HET1 HET2 HETHET IBS0 KINSHIP) "
+                         "over the records where both are diploid and called; at most 16384 samples (the pair "
+                         "counts take S^2 x 10 bytes); the VCF is unchanged")
+    ap.add_argument("--min-kinship", metavar="<x>", default=None,
+                    help="with --relatedness: write only the pairs whose KINSHIP is at least x (a finite number)")
     args = ap.parse_args(argv)
     import os
     if not args.prefix:
@@ -296,9 +305,32 @@ def cohort_main(argv=None):
             info_tags = parse_info_tags(args.info_tags, ploidy=args.ploidy_file is not None)
         except ValueError as exc:
             _die(f"--info-tags: {exc}")
+    min_kinship = None
+    if args.min_kinship is not None:
+        if args.relatedness is None:
+            _die("--min-kinship needs --relatedness")
+        import math
+        try:
+            min_kinship = float(args.min_kinship)
+        except ValueError:
+            min_kinship = math.nan
+        if not math.isfinite(min_kinship):
+            _die(f"--min-kinship {args.min_kinship!r}: it must be a finite number")
+    out_path = os.path.abspath(args.output)
+    tables_out = {}                                   # path -> the table written there
+    for opt, path in (("--sample-qc", args.sample_qc), ("--relatedness", args.relatedness)):
+        if path is not None:
+            path = os.path.abspath(path)
+            if path == out_path or path in tables_out:
+                _die(f"{opt} names the same file as another output")
+            tables_out[path] = opt
     if os.environ.get("SVJG_GPUS", "1").strip() != "1":
         _die("genotype-cohort runs on one GPU: SVJG_GPUS must be 1")
     samples = [[f for f in a.split(",")] for a in args.gaf]
+    if args.relatedness is not None:
+        from .capi import QC_MAX_PAIR_SAMPLES
+        if len(samples) > QC_MAX_PAIR_SAMPLES:
+            _die(f"--relatedness takes at most {QC_MAX_PAIR_SAMPLES} samples, not {len(samples)}")
     if any(not f for files in samples for f in files):
         _die("empty file name in -a")
     names = args.names.split(",") if args.names is not None else [_sample_name(files[0]) for files in samples]
@@ -318,11 +350,10 @@ def cohort_main(argv=None):
         except (OSError, ValueError) as exc:
             _die(str(exc))
     d_over = 100 if args.min_overlap is None else args.min_overlap
-    out_path = os.path.abspath(args.output)
     from concurrent.futures import ThreadPoolExecutor
 
     from . import alnfilter, capi, cohort, genotype, gzio
-    tmp = None
+    tmps = {}                                          # output path -> its temporary name, renamed once all succeed
     try:
         _lap("")
         ready = _start_device()
@@ -351,15 +382,30 @@ def cohort_main(argv=None):
                 del bufs
                 _lap(f"sample {k} filtered")
         import tempfile
-        fd, tmp = tempfile.mkstemp(prefix="." + os.path.basename(out_path) + ".", dir=os.path.dirname(out_path))
-        with os.fdopen(fd, "wb") as out:
-            _, n_gt = cohort.genotype_cohort_vcf(tables, co, vcf, names, args.minsupport, args.err, out=out,
-                                                 info_tags=info_tags, ploidy=ploidy, posteriors=args.posteriors)
-        os.replace(tmp, out_path)
-        tmp = None
+
+        def temp_file(path, mode):
+            fd, tmps[path] = tempfile.mkstemp(prefix="." + os.path.basename(path) + ".", dir=os.path.dirname(path))
+            return os.fdopen(fd, mode)
+        with temp_file(out_path, "wb") as out:
+            res = cohort.genotype_cohort_vcf(tables, co, vcf, names, args.minsupport, args.err, out=out,
+                                             info_tags=info_tags, ploidy=ploidy, posteriors=args.posteriors,
+                                             sample_qc=args.sample_qc is not None,
+                                             relatedness=args.relatedness is not None)
+        n_gt = res[1]
         _lap("genotypes + VCF written")
+        if args.sample_qc is not None:
+            with temp_file(os.path.abspath(args.sample_qc), "wb") as fh:
+                fh.write(cohort.sample_qc_text(names, res[2]).encode())
+        if args.relatedness is not None:
+            with temp_file(os.path.abspath(args.relatedness), "wb") as fh:
+                cohort.write_relatedness(fh, names, res[3], min_kinship)
+        if tables_out:
+            _lap("QC tables written")
+        for path in list(tmps):
+            os.replace(tmps[path], path)
+            del tmps[path]
     except (alnfilter.InputError, genotype.VcfError, capi.SvjgError, OSError, ValueError) as exc:
-        if tmp is not None:
+        for tmp in tmps.values():
             os.unlink(tmp)
         _die(str(exc))
     for nm, n in zip(names, n_gt):

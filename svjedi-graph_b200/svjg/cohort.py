@@ -50,6 +50,59 @@ def info_tags_mask(names):
     return mask
 
 
+# rows of the sample QC table (svjg_cohort_qc_sample_counts): every record, then the records of each SVTYPE code
+QC_TYPES = ("ALL", "DEL", "INS", "INV", "BND")
+SAMPLE_QC_HEADER = "#SAMPLE\tSVTYPE\tHOM_REF\tHET\tHOM_ALT\tHAP_REF\tHAP_ALT\tMISSING\tNO_PLOIDY\tCALL_RATE\tHET_HOM_RATIO\n"
+RELATEDNESS_PIECE_PAIRS = 1 << 22          # pairs formatted per svjg_format_relatedness call
+
+
+def _ratio(a, b):
+    return "." if b == 0 else "%.6g" % (a / b)
+
+
+def sample_qc_text(names, hist):
+    """The sample QC table of the samples ``names`` from their histograms ``hist`` [S][5][8] (rows QC_TYPES, columns
+    the gt codes 0-7): per sample and row, HOM_REF HET HOM_ALT HAP_REF HAP_ALT (codes 0, 1, 2, 4, 5), MISSING (3 and
+    6), NO_PLOIDY (7), CALL_RATE = called / (called + MISSING) and HET_HOM_RATIO = HET / HOM_ALT ("." over 0)."""
+    lines = [SAMPLE_QC_HEADER]
+    for nm, h in zip(names, hist):
+        for ty, row in zip(QC_TYPES, h):
+            c = [int(x) for x in row]
+            called, missing = c[0] + c[1] + c[2] + c[4] + c[5], c[3] + c[6]
+            lines.append(f"{nm}\t{ty}\t{c[0]}\t{c[1]}\t{c[2]}\t{c[4]}\t{c[5]}\t{missing}\t{c[7]}\t"
+                         f"{_ratio(called, called + missing)}\t{_ratio(c[1], c[2])}\n")
+    return "".join(lines)
+
+
+def write_relatedness(out, names, pairs, min_kinship=None):
+    """Writes the relatedness table of the samples ``names`` from svjg_cohort_relatedness's counts ``pairs``
+    [S (S - 1) / 2][5] to the binary file object ``out`` (svjg_format_relatedness, a range of rows per call).  With
+    ``min_kinship``, only the pairs whose KINSHIP is at least that."""
+    S = len(names)
+    pairs = np.ascontiguousarray(pairs, np.uint32)
+    if pairs.shape != (S * (S - 1) // 2, 5):
+        raise ValueError(f"pair counts of shape {pairs.shape} for {S} samples")
+    joined = "\t".join(names).encode()
+    i = 0
+    while True:
+        lo, n_pairs = i, 0
+        while i < S and n_pairs < RELATEDNESS_PIECE_PAIRS:
+            n_pairs += S - 1 - i
+            i += 1
+        buf, n_out = C.c_void_p(), C.c_uint64()
+        capi.check(capi.lib.svjg_format_relatedness(S, joined, len(joined), pairs.ctypes.data if pairs.size else None,
+                                                    lo, i, int(min_kinship is not None),
+                                                    0.0 if min_kinship is None else float(min_kinship), C.byref(buf),
+                                                    C.byref(n_out)))
+        try:
+            if n_out.value:
+                out.write(memoryview((C.c_char * n_out.value).from_address(buf.value)))
+        finally:
+            capi.lib.svjg_buffer_free(buf)
+        if i >= S:
+            return
+
+
 _phred_weights = None
 
 
@@ -305,7 +358,8 @@ def _posteriors(cohort, n, blk, iters=None):
 
 
 def genotype_cohort_vcf(tables, cohort, vcf_bytes, names, min_support=genotype.MIN_SUPPORT, e=genotype.ERR, out=None,
-                        block_records=None, info_tags=(), ploidy=None, posteriors=False):
+                        block_records=None, info_tags=(), ploidy=None, posteriors=False, sample_qc=False,
+                        relatedness=False):
     """predict-genotype.py's decision_vcf for every sample of ``cohort``: the multi-sample VCF, whose column s is
     the SAMPLE column of sample s's single-sample VCF.  ``vcf_bytes``: the catalogue VCF's bytes (or lines, or a
     genotype.NativeVcf of them).
@@ -317,13 +371,18 @@ def genotype_cohort_vcf(tables, cohort, vcf_bytes, names, min_support=genotype.M
     ``ploidy``: a PloidyRules for the samples of ``names``; the cells are called with their ploidy and the text is
     that of svjg_vcf_format_cohort_ploidy (PL Number=G, AC_Hemi available).  ``posteriors``: the allele frequency of
     every record by EM over its cells' likelihoods (INFO AF_EM), and each cell's GP and GQ under the Hardy-Weinberg
-    prior at it (svjg_cohort_posteriors, svjg_vcf_format_cohort_post); GT stays the likelihood call."""
+    prior at it (svjg_cohort_posteriors, svjg_vcf_format_cohort_post); GT stays the likelihood call.
+    ``sample_qc`` / ``relatedness``: the genotype codes of every block are also counted on the device
+    (svjg_cohort_qc_add), and the result is (text, counts, hist, pairs): hist [S][5][8] (svjg_cohort_qc_sample_counts)
+    or None, pairs [S (S - 1) / 2][5] (svjg_cohort_relatedness) or None; the text is the same."""
     S = cohort.n_samples
     mask = info_tags_mask(info_tags)
     if len(names) != S:
         raise ValueError(f"{len(names)} names for {S} samples")
     if ploidy is None and "AC_Hemi" in info_tags:
         raise ValueError("AC_Hemi counts haploid calls: it needs ploidy rules")
+    if relatedness and S > capi.QC_MAX_PAIR_SAMPLES:
+        raise ValueError(f"relatedness takes at most {capi.QC_MAX_PAIR_SAMPLES} samples")
     v = vcf_bytes if isinstance(vcf_bytes, genotype.NativeVcf) else genotype.NativeVcf.from_input(vcf_bytes)
     if v is None:
         raise genotype.VcfError("the VCF has non-ASCII bytes or a POS/END of more than 18 digits: "
@@ -350,6 +409,11 @@ def genotype_cohort_vcf(tables, cohort, vcf_bytes, names, min_support=genotype.M
             if ((fl & capi.GT_GENOTYPED).astype(bool) & (gt != capi.GT_NO_CALL)).any():
                 raise genotype.VcfError("error rate must be in (0, 1)")
         e = genotype.ERR
+    qc = sample_qc or relatedness
+    if qc:
+        # every block starts a new word of the bit planes
+        n_words = n // step * -(-step // 32) + -(-(n % step) // 32)
+        capi.check(capi.lib.svjg_cohort_qc_begin(cohort._h, n_words, int(bool(relatedness))))
     joined = "\t".join(names).encode()
     n_gt = np.zeros(S, np.uint64)
     pieces = []
@@ -357,6 +421,8 @@ def genotype_cohort_vcf(tables, cohort, vcf_bytes, names, min_support=genotype.M
         hi = min(n, lo + step)
         gt, fl, ad, pl = _genotype_block(cohort, idx[lo:hi], ty[lo:hi], min_support, e, blk,
                                          None if rclass is None else rclass[lo:hi])
+        if qc:
+            capi.check(capi.lib.svjg_cohort_qc_add(cohort._h, hi - lo))
         site = [None] * 3
         if mask:
             site = [a.ctypes.data for a in _site_stats(cohort, hi - lo, blk, rclass is not None)]
@@ -379,4 +445,13 @@ def genotype_cohort_vcf(tables, cohort, vcf_bytes, names, min_support=genotype.M
         finally:
             capi.lib.svjg_buffer_free(buf)
     text = None if out is not None else b"".join(pieces).decode("ascii")
-    return text, [int(x) for x in n_gt]
+    if not qc:
+        return text, [int(x) for x in n_gt]
+    hist = pairs = None
+    if sample_qc:
+        hist = np.zeros((S, len(QC_TYPES), 8), np.uint32)
+        capi.check(capi.lib.svjg_cohort_qc_sample_counts(cohort._h, hist.ctypes.data))
+    if relatedness:
+        pairs = np.zeros((S * (S - 1) // 2, 5), np.uint32)
+        capi.check(capi.lib.svjg_cohort_relatedness(cohort._h, pairs.ctypes.data if pairs.size else None))
+    return text, [int(x) for x in n_gt], hist, pairs
