@@ -341,6 +341,15 @@ int svjg_cohort_qc_add(svjg_cohort *c, uint32_t n);
 int svjg_cohort_qc_sample_counts(svjg_cohort *c, uint32_t *out);
 int svjg_cohort_qc_planes(svjg_cohort *c, uint32_t *out);
 int svjg_cohort_relatedness(svjg_cohort *c, uint32_t *out);
+/* svjg_cohort_grm: the genetic relationship matrix over the same planes (DESIGN.md §8a, "Relationship matrix and
+ * PCA").  Per record, AN = 2 x (cells with codes 0-2) and AC = (code 1) + 2 x (code 2); it is used iff 0 < AC < AN and
+ * min(AC, AN - AC) / AN >= min_maf; then p = AC / AN, s = 2 p, w = 1 / (s (1 - p)), v_g = g - s, u_g = w v_g.  Per pair
+ * i <= j, over the used records where both cells are diploid and called, in record order: N = their count, acc = acc +
+ * u_{g_i} v_{g_j} from +0.0 (every step one double operation rounded to nearest), G = acc / N, 0 when N = 0.  Out
+ * grm [S (S + 1) / 2] f64 and n [S (S + 1) / 2] u32, pair (i <= j) at i (2 S - i + 1) / 2 + (j - i).  Needs
+ * want_pairs; SVJG_E_ARG for min_maf outside [0, 0.5] (or NaN) and a NULL output when S >= 1.  The planes are not
+ * changed (call it before or after svjg_cohort_relatedness).  Synchronous. */
+int svjg_cohort_grm(svjg_cohort *c, double min_maf, double *grm, uint32_t *n);
 
 /* Page-locked host memory (cudaHostAlloc) for file buffers and results: copies to and from it run
  * at PCIe speed.  For callers that do not want a tensor library just to pin memory. */

@@ -746,6 +746,154 @@ cohort_pair_kernel(const uint32_t *__restrict__ planes, uint32_t S, size_t strid
     }
 }
 
+// ---- relationship matrix (DESIGN.md §8a, "Relationship matrix and PCA") ----
+// Per record: one CTA per plane word w (records 32 w + lane).  Each warp counts the C, H and A bits of its lane's
+// record down a stride of the samples, the partials are summed in shared memory, and warp 0 writes the record's
+// (u0, u1, u2, v0, v1, v2) to tab [32 n_words][6] and the used-record mask to used[w].  AN = 2 nC, AC = nH + 2 nA; the
+// record is used iff 0 < AC < AN and min(AC, AN - AC) / AN >= min_maf; then p = AC / AN, s = 2 p, w = 1 / (s (1 - p)),
+// v_g = g - s, u_g = w v_g, each one double operation rounded to nearest.  An unused record's (and a padding bit's)
+// entries are 0.
+constexpr int GRM_PREP_THREADS = 256;
+__global__ void __launch_bounds__(GRM_PREP_THREADS)
+cohort_grm_prep_kernel(const uint32_t *__restrict__ planes, uint32_t S, size_t stride, double min_maf,
+                       double *__restrict__ tab, uint32_t *__restrict__ used) {
+    constexpr int WARPS = GRM_PREP_THREADS / 32;
+    __shared__ uint32_t part[3][WARPS][32];
+    const uint32_t w = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const size_t plane = size_t(S) * stride;
+    uint32_t nc = 0, nh = 0, na = 0;
+#pragma unroll 4
+    for (uint32_t s = warp; s < S; s += WARPS) {
+        const uint32_t *p = planes + size_t(s) * stride + w;
+        nc += (__ldg(p) >> lane) & 1;
+        nh += (__ldg(p + plane) >> lane) & 1;
+        na += (__ldg(p + 2 * plane) >> lane) & 1;
+    }
+    part[0][warp][lane] = nc;
+    part[1][warp][lane] = nh;
+    part[2][warp][lane] = na;
+    __syncthreads();
+    if (warp) return;
+    for (int k = 1; k < WARPS; ++k) {
+        nc += part[0][k][lane];
+        nh += part[1][k][lane];
+        na += part[2][k][lane];
+    }
+    const uint32_t an = 2 * nc, ac = nh + 2 * na;
+    const bool use = 0 < ac && ac < an && __ddiv_rn(double(min(ac, an - ac)), double(an)) >= min_maf;
+    double t[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    if (use) {
+        const double p = __ddiv_rn(double(ac), double(an));
+        const double s = __dmul_rn(2.0, p);
+        const double wt = __ddiv_rn(1.0, __dmul_rn(s, __dsub_rn(1.0, p)));
+#pragma unroll
+        for (int g = 0; g < 3; ++g) {
+            t[3 + g] = __dsub_rn(double(g), s);
+            t[g] = __dmul_rn(wt, t[3 + g]);
+        }
+    }
+    double *o = tab + (size_t(w) * 32 + lane) * 6;
+#pragma unroll
+    for (int q = 0; q < 6; ++q) o[q] = t[q];
+    const uint32_t m = __ballot_sync(0xFFFFFFFFu, use);
+    if (lane == 0) used[w] = m;
+}
+
+// Pairs: the upper triangle of the S x S grid in tiles of GRM_T x GRM_T samples, tile (bi, bj) with bi <= bj at linear
+// index bj (bj + 1) / 2 + bi, as in cohort_pair_kernel.  For each plane word w with a used record, the CTA decodes the
+// 32 records of its two sample ranges into shared memory ([side][record][sample]): u_{g_i} on the i side, v_{g_j} on
+// the j side, 0.0 for a cell that is not diploid called or a record that is not used (a +-0 term leaves a sum that
+// starts at +0.0 unchanged).  Each thread of a 16 x 16 grid owns the 4 x 4 pairs (i0 + 4 ty + a, j0 + tx + 16 b) and
+// adds acc = acc + u v record by record in ascending order (__dmul_rn / __dadd_rn: no contraction), with
+// N += popc(Ci & U & Cj) per word.  No split over records: every pair sums in record order, so the bits do not depend
+// on the tiling.  Pair (i <= j) goes to p = i (2 S - i + 1) / 2 + (j - i): g[p] = acc / N (0.0 when N = 0), n[p] = N.
+constexpr uint32_t GRM_T = 64;
+constexpr int GRM_THREADS = 256;
+__global__ void __launch_bounds__(GRM_THREADS, 2)
+cohort_grm_kernel(const uint32_t *__restrict__ planes, uint32_t S, size_t stride, uint32_t n_words,
+                  const double *__restrict__ tab, const uint32_t *__restrict__ used, double *__restrict__ g,
+                  uint32_t *__restrict__ nout) {
+    __shared__ __align__(16) double uv[2][32][GRM_T];
+    __shared__ uint32_t cw[2][GRM_T];                                 // C & U of the word, per side and sample
+    const uint32_t t = blockIdx.x;
+    uint32_t bj = uint32_t((sqrt(8.0 * t + 1.0) - 1.0) / 2.0);
+    while (bj * (bj + 1) / 2 > t) --bj;
+    while ((bj + 1) * (bj + 2) / 2 <= t) ++bj;
+    const uint32_t bi = t - bj * (bj + 1) / 2;
+    const uint32_t i0 = bi * GRM_T, j0 = bj * GRM_T;
+    const uint32_t tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
+    // decoder: sample lr of side `side`, records 16 half .. 16 half + 15 of the word
+    const uint32_t lr = threadIdx.x & 63, side = (threadIdx.x >> 6) & 1, half = threadIdx.x >> 7;
+    const uint32_t row = (side ? j0 : i0) + lr;
+    const size_t plane = size_t(S) * stride;
+    double acc[4][4];
+    uint32_t cnt[4][4];
+#pragma unroll
+    for (int a = 0; a < 4; ++a)
+#pragma unroll
+        for (int b = 0; b < 4; ++b) {
+            acc[a][b] = 0.0;
+            cnt[a][b] = 0;
+        }
+    for (uint32_t w = 0; w < n_words; ++w) {
+        const uint32_t U = __ldg(used + w);
+        if (U == 0) continue;                                           // the same for the whole CTA
+        uint32_t Cw = 0, Hw = 0, Aw = 0;
+        if (row < S) {
+            const uint32_t *p = planes + size_t(row) * stride + w;
+            Cw = __ldg(p) & U;
+            Hw = __ldg(p + plane);
+            Aw = __ldg(p + 2 * plane);
+        }
+        if (half == 0) cw[side][lr] = Cw;
+        const double *tw = tab + size_t(w) * 32 * 6 + 3 * side;
+#pragma unroll
+        for (int k = 0; k < 16; ++k) {
+            const uint32_t r = 16 * half + k, bit = 1u << r;
+            double x = 0.0;
+            if (Cw & bit) x = __ldg(tw + r * 6 + ((Hw & bit) ? 1 : (Aw & bit) ? 2 : 0));
+            uv[side][r][lr] = x;
+        }
+        __syncthreads();
+        uint32_t Ci[4], Cj[4];
+#pragma unroll
+        for (int a = 0; a < 4; ++a) Ci[a] = cw[0][4 * ty + a];
+#pragma unroll
+        for (int b = 0; b < 4; ++b) Cj[b] = cw[1][tx + 16 * b];
+#pragma unroll
+        for (int a = 0; a < 4; ++a)
+#pragma unroll
+            for (int b = 0; b < 4; ++b) cnt[a][b] += __popc(Ci[a] & Cj[b]);
+#pragma unroll 4
+        for (int k = 0; k < 32; ++k) {
+            const double2 u01 = *reinterpret_cast<const double2 *>(&uv[0][k][4 * ty]);
+            const double2 u23 = *reinterpret_cast<const double2 *>(&uv[0][k][4 * ty + 2]);
+            const double ui[4] = {u01.x, u01.y, u23.x, u23.y};
+            double vj[4];
+#pragma unroll
+            for (int b = 0; b < 4; ++b) vj[b] = uv[1][k][tx + 16 * b];
+#pragma unroll
+            for (int a = 0; a < 4; ++a)
+#pragma unroll
+                for (int b = 0; b < 4; ++b) acc[a][b] = __dadd_rn(acc[a][b], __dmul_rn(ui[a], vj[b]));
+        }
+        __syncthreads();
+    }
+#pragma unroll
+    for (int a = 0; a < 4; ++a) {
+        const uint32_t i = i0 + 4 * ty + a;
+#pragma unroll
+        for (int b = 0; b < 4; ++b) {
+            const uint32_t j = j0 + tx + 16 * b;
+            if (i <= j && j < S) {
+                const uint64_t p = uint64_t(i) * (2 * uint64_t(S) - i + 1) / 2 + (j - i);
+                nout[p] = cnt[a][b];
+                g[p] = cnt[a][b] ? __ddiv_rn(acc[a][b], double(cnt[a][b])) : 0.0;
+            }
+        }
+    }
+}
+
 }  // namespace
 
 extern "C" int svjg_genotype_device(const uint32_t *d_counts, const uint32_t *d_sv_index, const uint8_t *d_svtype,
@@ -1147,6 +1295,47 @@ extern "C" int svjg_cohort_relatedness(svjg_cohort *c, uint32_t *out) {
     const cudaError_t es = cudaStreamSynchronize(st);
     if (e == cudaSuccess) e = es;
     if (e != cudaSuccess) return svjg::cuda_fail(int(e), "svjg_cohort_relatedness");
+    return SVJG_OK;
+}
+
+// Relationship matrix over the resident planes: the per-record table, then the pair tiles; the planes are only read.
+extern "C" int svjg_cohort_grm(svjg_cohort *c, double min_maf, double *grm, uint32_t *n) {
+    const std::string f = "svjg_cohort_grm";
+    if (!c) return svjg::set_error(SVJG_E_ARG, f + ": NULL cohort");
+    if (!c->qc_on || !c->qc_pairs) return svjg::set_error(SVJG_E_ARG, f + ": no svjg_cohort_qc_begin with want_pairs");
+    if (!(min_maf >= 0.0 && min_maf <= 0.5)) return svjg::set_error(SVJG_E_ARG, f + ": min_maf must be in [0, 0.5]");
+    const uint64_t S = c->n_samples, n_pairs = S * (S + 1) / 2;
+    if (n_pairs == 0) return SVJG_OK;
+    if (!grm || !n) return svjg::set_error(SVJG_E_ARG, f + ": NULL argument");
+    SVJG_CUDA(cudaSetDevice(c->t->device));
+    cudaStream_t st = c->stream;
+    const uint64_t n_words = c->qc_used;
+    // one allocation: G [n_pairs] f64, the table [32 n_words][6] f64, N [n_pairs] u32, the mask [n_words] u32
+    const size_t o_tab = n_pairs * 8, o_n = o_tab + n_words * 32 * 6 * 8, o_used = o_n + n_pairs * 4;
+    char *d = nullptr;
+    SVJG_CUDA(cudaMallocAsync(reinterpret_cast<void **>(&d), o_used + n_words * 4, st));
+    double *d_g = reinterpret_cast<double *>(d), *d_tab = reinterpret_cast<double *>(d + o_tab);
+    uint32_t *d_n = reinterpret_cast<uint32_t *>(d + o_n), *d_used = reinterpret_cast<uint32_t *>(d + o_used);
+    const uint32_t *planes = c->d_qc + S * 40;
+    const uint64_t tiles = (S + GRM_T - 1) / GRM_T;
+    cudaError_t e = cudaSuccess;
+    if (n_words == 0) {
+        e = cudaMemsetAsync(d, 0, o_used, st);
+    } else {
+        cohort_grm_prep_kernel<<<uint32_t(n_words), GRM_PREP_THREADS, 0, st>>>(planes, uint32_t(S), c->qc_stride, min_maf,
+                                                                                d_tab, d_used);
+        e = cudaGetLastError();
+        if (e == cudaSuccess)
+            cohort_grm_kernel<<<uint32_t(tiles * (tiles + 1) / 2), GRM_THREADS, 0, st>>>(
+                planes, uint32_t(S), c->qc_stride, uint32_t(n_words), d_tab, d_used, d_g, d_n);
+    }
+    if (e == cudaSuccess) e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaMemcpyAsync(grm, d_g, n_pairs * 8, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(n, d_n, n_pairs * 4, cudaMemcpyDeviceToHost, st);
+    cudaFreeAsync(d, st);
+    const cudaError_t es = cudaStreamSynchronize(st);
+    if (e == cudaSuccess) e = es;
+    if (e != cudaSuccess) return svjg::cuda_fail(int(e), "svjg_cohort_grm");
     return SVJG_OK;
 }
 

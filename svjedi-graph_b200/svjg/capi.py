@@ -110,6 +110,7 @@ def _load():
         "svjg_cohort_qc_sample_counts": (C.c_int, [vp, u32p]),
         "svjg_cohort_qc_planes": (C.c_int, [vp, u32p]),
         "svjg_cohort_relatedness": (C.c_int, [vp, u32p]),
+        "svjg_cohort_grm": (C.c_int, [vp, C.c_double, f64p, u32p]),
         "svjg_host_alloc": (C.c_int, [C.c_uint64, C.POINTER(C.c_void_p)]),
         "svjg_host_free": (C.c_int, [vp]),
         "svjg_host_register": (C.c_int, [vp, C.c_uint64]),

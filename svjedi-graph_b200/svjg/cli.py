@@ -292,6 +292,18 @@ def cohort_main(argv=None):
                          "counts take S^2 x 10 bytes); the VCF is unchanged")
     ap.add_argument("--min-kinship", metavar="<x>", default=None,
                     help="with --relatedness: write only the pairs whose KINSHIP is at least x (a finite number)")
+    ap.add_argument("--grm", metavar="<prefix>", default=None,
+                    help="write the genetic relationship matrix of the samples in GCTA's binary layout: <prefix>.grm.bin "
+                         "and <prefix>.grm.N.bin (lower triangle, float32) and <prefix>.grm.id; at most 16384 samples; "
+                         "the VCF is unchanged")
+    ap.add_argument("--pca", metavar="<prefix>", default=None,
+                    help="write the leading principal components of that matrix: <prefix>.eigenvec and "
+                         "<prefix>.eigenval; at most 16384 samples; the VCF is unchanged")
+    ap.add_argument("--pca-components", metavar="<k>", default=None,
+                    help="with --pca: how many components, 1 to the number of samples (default 10)")
+    ap.add_argument("--grm-min-maf", metavar="<x>", default=None,
+                    help="with --grm or --pca: only records whose minor allele frequency over the diploid calls is "
+                         "at least x, in [0, 0.5], enter the matrix (default 0.01)")
     args = ap.parse_args(argv)
     import os
     if not args.prefix:
@@ -316,9 +328,34 @@ def cohort_main(argv=None):
             min_kinship = math.nan
         if not math.isfinite(min_kinship):
             _die(f"--min-kinship {args.min_kinship!r}: it must be a finite number")
+    from .cohort import GRM_MIN_MAF, PCA_COMPONENTS
+    n_pcs = PCA_COMPONENTS
+    if args.pca_components is not None:
+        if args.pca is None:
+            _die("--pca-components needs --pca")
+        try:
+            n_pcs = int(args.pca_components)
+        except ValueError:
+            _die(f"--pca-components {args.pca_components!r}: it must be an integer")
+    grm_min_maf = GRM_MIN_MAF
+    if args.grm_min_maf is not None:
+        if args.grm is None and args.pca is None:
+            _die("--grm-min-maf needs --grm or --pca")
+        import math
+        try:
+            grm_min_maf = float(args.grm_min_maf)
+        except ValueError:
+            grm_min_maf = math.nan
+        if not 0.0 <= grm_min_maf <= 0.5:
+            _die(f"--grm-min-maf {args.grm_min_maf!r}: it must be a number in [0, 0.5]")
     out_path = os.path.abspath(args.output)
     tables_out = {}                                   # path -> the table written there
-    for opt, path in (("--sample-qc", args.sample_qc), ("--relatedness", args.relatedness)):
+    derived = []
+    if args.grm is not None:
+        derived += [("--grm", args.grm + ext) for ext in (".grm.bin", ".grm.N.bin", ".grm.id")]
+    if args.pca is not None:
+        derived += [("--pca", args.pca + ext) for ext in (".eigenvec", ".eigenval")]
+    for opt, path in (("--sample-qc", args.sample_qc), ("--relatedness", args.relatedness), *derived):
         if path is not None:
             path = os.path.abspath(path)
             if path == out_path or path in tables_out:
@@ -331,6 +368,13 @@ def cohort_main(argv=None):
         from .capi import QC_MAX_PAIR_SAMPLES
         if len(samples) > QC_MAX_PAIR_SAMPLES:
             _die(f"--relatedness takes at most {QC_MAX_PAIR_SAMPLES} samples, not {len(samples)}")
+    for opt in ("--grm", "--pca"):
+        if getattr(args, opt[2:]) is not None:
+            from .capi import QC_MAX_PAIR_SAMPLES
+            if len(samples) > QC_MAX_PAIR_SAMPLES:
+                _die(f"{opt} takes at most {QC_MAX_PAIR_SAMPLES} samples, not {len(samples)}")
+    if args.pca is not None and not 1 <= n_pcs <= len(samples):
+        _die(f"--pca-components {n_pcs}: it must be between 1 and the number of samples ({len(samples)})")
     if any(not f for files in samples for f in files):
         _die("empty file name in -a")
     names = args.names.split(",") if args.names is not None else [_sample_name(files[0]) for files in samples]
@@ -350,6 +394,7 @@ def cohort_main(argv=None):
         except (OSError, ValueError) as exc:
             _die(str(exc))
     d_over = 100 if args.min_overlap is None else args.min_overlap
+    want_grm = args.grm is not None or args.pca is not None
     from concurrent.futures import ThreadPoolExecutor
 
     from . import alnfilter, capi, cohort, genotype, gzio
@@ -390,7 +435,8 @@ def cohort_main(argv=None):
             res = cohort.genotype_cohort_vcf(tables, co, vcf, names, args.minsupport, args.err, out=out,
                                              info_tags=info_tags, ploidy=ploidy, posteriors=args.posteriors,
                                              sample_qc=args.sample_qc is not None,
-                                             relatedness=args.relatedness is not None)
+                                             relatedness=args.relatedness is not None,
+                                             grm=want_grm, grm_min_maf=grm_min_maf)
         n_gt = res[1]
         _lap("genotypes + VCF written")
         if args.sample_qc is not None:
@@ -399,6 +445,18 @@ def cohort_main(argv=None):
         if args.relatedness is not None:
             with temp_file(os.path.abspath(args.relatedness), "wb") as fh:
                 cohort.write_relatedness(fh, names, res[3], min_kinship)
+        if args.grm is not None:
+            G, N = res[4]
+            with temp_file(os.path.abspath(args.grm + ".grm.bin"), "wb") as fb, \
+                    temp_file(os.path.abspath(args.grm + ".grm.N.bin"), "wb") as fn, \
+                    temp_file(os.path.abspath(args.grm + ".grm.id"), "wb") as fi:
+                cohort.write_grm(fb, fn, fi, names, G, N)
+        if args.pca is not None:
+            vals, vecs = cohort.pca(res[4][0], n_pcs)
+            _lap("PCA computed")
+            with temp_file(os.path.abspath(args.pca + ".eigenvec"), "wb") as fv, \
+                    temp_file(os.path.abspath(args.pca + ".eigenval"), "wb") as fe:
+                cohort.write_pca(fv, fe, names, vals, vecs)
         if tables_out:
             _lap("QC tables written")
         for path in list(tmps):

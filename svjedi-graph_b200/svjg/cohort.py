@@ -103,6 +103,64 @@ def write_relatedness(out, names, pairs, min_kinship=None):
             return
 
 
+GRM_MIN_MAF = 0.01                         # --grm-min-maf default
+PCA_COMPONENTS = 10                        # --pca-components default
+
+
+def grm_square(packed, S, dtype):
+    """The symmetric [S][S] matrix of svjg_cohort_grm's packed upper triangle (pair i <= j at i (2 S - i + 1) / 2 +
+    j - i), filled row by row so that no index arrays of S^2 entries are made."""
+    out = np.zeros((S, S), dtype)
+    o = 0
+    for i in range(S):
+        row = packed[o:o + S - i]
+        out[i, i:] = row
+        out[i:, i] = row
+        o += S - i
+    return out
+
+
+def pca(G, k):
+    """The k leading principal components of the symmetric relationship matrix G [S][S] (numpy.linalg.eigh): the k
+    largest eigenvalues in descending order and their unit eigenvectors [S][k], each eigenvector's sign flipped so that
+    its component of largest absolute value (the first such one on ties) is positive."""
+    G = np.asarray(G, np.float64)
+    if not 1 <= k <= G.shape[0]:
+        raise ValueError(f"{k} principal components of {G.shape[0]} samples")
+    vals, vecs = np.linalg.eigh(G)
+    vals, vecs = vals[::-1][:k].copy(), vecs[:, ::-1][:, :k].copy()
+    lead = vecs[np.argmax(np.abs(vecs), axis=0), np.arange(k)]
+    vecs[:, lead < 0] *= -1.0
+    return vals, vecs
+
+
+def write_grm(bin_out, n_out, id_out, names, G, N):
+    """GCTA's binary relationship matrix: the lower triangle with the diagonal, row by row (i from 0, j <= i), of G
+    (``bin_out``) and of N (``n_out``) as little-endian float32, and one "NAME\\tNAME" line per sample (``id_out``).
+    All three are binary file objects."""
+    S = len(names)
+    if np.shape(G) != (S, S) or np.shape(N) != (S, S):
+        raise ValueError(f"relationship matrices of shape {np.shape(G)} / {np.shape(N)} for {S} samples")
+    rows = max(1, (1 << 22) // max(S, 1))                      # about 4 M entries per write
+    for lo in range(0, S, rows):
+        hi = min(S, lo + rows)
+        for M, out in ((G, bin_out), (N, n_out)):
+            out.write(np.concatenate([M[i, :i + 1] for i in range(lo, hi)]).astype("<f4").tobytes())
+    id_out.write("".join(f"{nm}\t{nm}\n" for nm in names).encode())
+
+
+def write_pca(vec_out, val_out, names, vals, vecs):
+    """The eigenvectors [S][K] (header "#IID\\tPC1 ... PCK", then one line per sample) and the eigenvalues [K] (one per
+    line) of pca(), "%.6g", to the binary file objects ``vec_out`` and ``val_out``."""
+    K = len(vals)
+    if np.shape(vecs) != (len(names), K):
+        raise ValueError(f"eigenvectors of shape {np.shape(vecs)} for {len(names)} samples and {K} components")
+    lines = ["#IID" + "".join(f"\tPC{k + 1}" for k in range(K)) + "\n"]
+    lines += [nm + "".join("\t%.6g" % x for x in row) + "\n" for nm, row in zip(names, vecs.tolist())]
+    vec_out.write("".join(lines).encode())
+    val_out.write("".join("%.6g\n" % x for x in vals.tolist()).encode())
+
+
 _phred_weights = None
 
 
@@ -359,7 +417,7 @@ def _posteriors(cohort, n, blk, iters=None):
 
 def genotype_cohort_vcf(tables, cohort, vcf_bytes, names, min_support=genotype.MIN_SUPPORT, e=genotype.ERR, out=None,
                         block_records=None, info_tags=(), ploidy=None, posteriors=False, sample_qc=False,
-                        relatedness=False):
+                        relatedness=False, grm=False, grm_min_maf=GRM_MIN_MAF):
     """predict-genotype.py's decision_vcf for every sample of ``cohort``: the multi-sample VCF, whose column s is
     the SAMPLE column of sample s's single-sample VCF.  ``vcf_bytes``: the catalogue VCF's bytes (or lines, or a
     genotype.NativeVcf of them).
@@ -374,7 +432,10 @@ def genotype_cohort_vcf(tables, cohort, vcf_bytes, names, min_support=genotype.M
     prior at it (svjg_cohort_posteriors, svjg_vcf_format_cohort_post); GT stays the likelihood call.
     ``sample_qc`` / ``relatedness``: the genotype codes of every block are also counted on the device
     (svjg_cohort_qc_add), and the result is (text, counts, hist, pairs): hist [S][5][8] (svjg_cohort_qc_sample_counts)
-    or None, pairs [S (S - 1) / 2][5] (svjg_cohort_relatedness) or None; the text is the same."""
+    or None, pairs [S (S - 1) / 2][5] (svjg_cohort_relatedness) or None; the text is the same.
+    ``grm``: the bit planes are kept as for ``relatedness``, and the result is (text, counts, hist, pairs, (G, N)): the
+    relationship matrix over the records whose minor allele frequency is at least ``grm_min_maf`` (svjg_cohort_grm),
+    G [S][S] float64 and N [S][S] uint32, both symmetric."""
     S = cohort.n_samples
     mask = info_tags_mask(info_tags)
     if len(names) != S:
@@ -383,6 +444,10 @@ def genotype_cohort_vcf(tables, cohort, vcf_bytes, names, min_support=genotype.M
         raise ValueError("AC_Hemi counts haploid calls: it needs ploidy rules")
     if relatedness and S > capi.QC_MAX_PAIR_SAMPLES:
         raise ValueError(f"relatedness takes at most {capi.QC_MAX_PAIR_SAMPLES} samples")
+    if grm and S > capi.QC_MAX_PAIR_SAMPLES:
+        raise ValueError(f"the relationship matrix takes at most {capi.QC_MAX_PAIR_SAMPLES} samples")
+    if grm and not 0.0 <= grm_min_maf <= 0.5:
+        raise ValueError(f"grm_min_maf {grm_min_maf!r} is not in [0, 0.5]")
     v = vcf_bytes if isinstance(vcf_bytes, genotype.NativeVcf) else genotype.NativeVcf.from_input(vcf_bytes)
     if v is None:
         raise genotype.VcfError("the VCF has non-ASCII bytes or a POS/END of more than 18 digits: "
@@ -409,11 +474,11 @@ def genotype_cohort_vcf(tables, cohort, vcf_bytes, names, min_support=genotype.M
             if ((fl & capi.GT_GENOTYPED).astype(bool) & (gt != capi.GT_NO_CALL)).any():
                 raise genotype.VcfError("error rate must be in (0, 1)")
         e = genotype.ERR
-    qc = sample_qc or relatedness
+    qc = sample_qc or relatedness or grm
     if qc:
         # every block starts a new word of the bit planes
         n_words = n // step * -(-step // 32) + -(-(n % step) // 32)
-        capi.check(capi.lib.svjg_cohort_qc_begin(cohort._h, n_words, int(bool(relatedness))))
+        capi.check(capi.lib.svjg_cohort_qc_begin(cohort._h, n_words, int(bool(relatedness or grm))))
     joined = "\t".join(names).encode()
     n_gt = np.zeros(S, np.uint64)
     pieces = []
@@ -454,4 +519,10 @@ def genotype_cohort_vcf(tables, cohort, vcf_bytes, names, min_support=genotype.M
     if relatedness:
         pairs = np.zeros((S * (S - 1) // 2, 5), np.uint32)
         capi.check(capi.lib.svjg_cohort_relatedness(cohort._h, pairs.ctypes.data if pairs.size else None))
-    return text, [int(x) for x in n_gt], hist, pairs
+    if not grm:
+        return text, [int(x) for x in n_gt], hist, pairs
+    g = np.zeros(S * (S + 1) // 2, np.float64)
+    nn = np.zeros(S * (S + 1) // 2, np.uint32)
+    capi.check(capi.lib.svjg_cohort_grm(cohort._h, float(grm_min_maf), g.ctypes.data if S else None,
+                                        nn.ctypes.data if S else None))
+    return text, [int(x) for x in n_gt], hist, pairs, (grm_square(g, S, np.float64), grm_square(nn, S, np.uint32))
